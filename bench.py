@@ -16,12 +16,16 @@ whole contig.
 
 `--impl reference` times the oracle port (the reference is Python + samtools + TensorFlow,
 none of which can run on the GPU box) with all host cores on bounded samples.
+
+`--dump-outputs DIR` writes what the last timed end-to-end step returned to its caller as DIR/<name>.npy
+(see dump_outputs), so that two builds can be compared output for output on the same seeded inputs.
 """
 import argparse
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -34,6 +38,10 @@ FLOP_PER_SITE = {18: 47.786e6, 30: 48.597e6}       # SURVEY.md §8(d), BASELINE.
 
 
 E2E_DEPTH = int(os.environ.get("C3R_E2E_DEPTH", "2"))        # submits queued ahead of the one being waited for in the end-to-end leg (three tickets in flight)
+# Generated inputs are cached between runs outside the source tree, which may be read-only.  One directory per user:
+# a directory that another account left in a shared /tmp can be neither written to nor trusted.
+CACHE_DIR = os.path.join(tempfile.gettempdir(), "c3r_bench_cache_%d" % os.getuid())
+DUMP_LIMIT = 64 * 10 ** 6                                      # bytes written by --dump-outputs at most
 
 def peaks():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
@@ -54,7 +62,7 @@ def measured_traffic(workload_name):
     return {}, None
 
 
-def dataset(cfg_idx, scale, contig_slot, cache_dir="/tmp/c3r_bench_cache"):
+def dataset(cfg_idx, scale, contig_slot, cache_dir=CACHE_DIR):
     """reads + reference of one contig; `contig_slot` varies the seed per rank."""
     import dataclasses
     from clair3_rna_b200 import synth
@@ -222,7 +230,7 @@ def _cfg5_make_contig(args):
     return ci
 
 
-def cfg5_dataset(scale, rank, world, cores, barrier, cache_dir="/tmp/c3r_bench_cache"):
+def cfg5_dataset(scale, rank, world, cores, barrier, cache_dir=CACHE_DIR):
     """reads.bam (+ .bai), genome.fa (+ .fai), weights.npz of the config-5 genome at `scale`, made once per box:
     the ranks generate the contigs between them (process pools), rank 0 then writes the BAM, the last rank the FASTA"""
     import multiprocessing as mp
@@ -363,6 +371,34 @@ def shard_cfg5_leg(scale, rank, world, local_rank, cores, barrier, gloo, eng):
     }
 
 
+# ------------------------------------------------------------------ outputs of the timed path
+def dump_outputs(out_dir, r, seed=0):
+    """Writes the arrays of a ChunkResult as the caller of Engine.wait receives them, one .npy each: pos, depth,
+    alt_off, alt_n (int, stored as float64, which holds them exactly), probs (float32) and alt_<field> for the fields
+    of the allele table.  The allele table holds each candidate's alt_n entries in candidate order (the slots between
+    two candidates' entries are never written, so they are left out).  When all of it would exceed DUMP_LIMIT bytes,
+    a fixed, seeded sample of the candidates is written, in ascending order.  -> (candidates written, candidates)"""
+    n = r.n_cand
+    alt_n = r.alt_n.astype(np.int64)
+    cost = 4 * 8 + 24 * 4 + 8 * len(r.alt.dtype.names) * alt_n          # bytes written per candidate
+    budget = DUMP_LIMIT - 4096                                           # less the .npy headers
+    keep = np.arange(n)
+    if cost.sum() > budget:
+        order = np.random.default_rng(seed).permutation(n)
+        keep = np.sort(order[np.cumsum(cost[order]) <= budget])
+    k_n = alt_n[keep]
+    first = np.repeat(r.alt_off[keep], k_n)
+    within = np.arange(int(k_n.sum())) - np.repeat(np.cumsum(k_n) - k_n, k_n)
+    alt = r.alt[first + within]
+    arrays = {"pos": r.pos[keep], "depth": r.depth[keep], "probs": r.probs[keep], "alt_off": r.alt_off[keep],
+              "alt_n": r.alt_n[keep]}
+    arrays.update(("alt_" + f, alt[f]) for f in alt.dtype.names)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32 if a.dtype == np.float32 else np.float64))
+    return keep.size, n
+
+
 # ------------------------------------------------------------------ main
 def main():
     ap = argparse.ArgumentParser()
@@ -376,7 +412,14 @@ def main():
     ap.add_argument("--no_cpu_baseline", action="store_true")
     ap.add_argument("--cfg5_scale", type=float, default=1.0,
                     help="genome scale of the sharded config-5 leg (1.0 = GRCh38 lengths, 631 chunks; 0 = skip the leg)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed end-to-end step returned (rank 0) as DIR/<name>.npy, "
+                         "float32 / float64, at most 64 MB")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -515,6 +558,9 @@ def main():
     # the last timed step's results against the first (sequential) call of this run: same inputs, same outputs
     # (the alt table is not compared as a block: the slots between two candidates' entries are never written)
     assert np.array_equal(r.pos, res0.pos) and np.array_equal(r.probs, res0.probs) and np.array_equal(r.alt_n, res0.alt_n)
+    if args.dump_outputs and rank == 0:
+        print("--dump-outputs: %d of %d candidates written to %s" % (dump_outputs(args.dump_outputs, r) + (args.dump_outputs,)),
+              file=sys.stderr)
     eng.release(tk)
     while inflight:
         eng.wait(inflight.popleft())                   # drain (untimed)
