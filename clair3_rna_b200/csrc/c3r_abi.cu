@@ -99,7 +99,7 @@ struct c3r_ctx {
     int prio_hi = 0;
     const c3r_site_filter* filter = nullptr;   // of the submit in progress
     bool tc_dirty = false;    // a tensor-core forward ran since the last device error check
-    cudaEvent_t nn_done = nullptr;   // end of the last network pass: the scratch (h1, zx2, h2 ...) is shared by all tickets
+    cudaEvent_t nn_done = nullptr;   // end of the last network pass: the scratch (h1, h2, l4 ...) is shared by all tickets
     Buf thr;                  // allele-frequency threshold tables (k_thr_table)
     Buf ref_res;              // resident reference window (c3r_set_reference)
     Buf refnib_res;           // its one-hot nibble form (k_refnib)
@@ -715,12 +715,8 @@ static int submit_once(c3r_ctx* ctx, const c3r_reads* rd, const uint8_t* ref, in
         ++s.launches;
     }
     // The copies above overlap the network pass of the ticket before this one, and so do the position / row stages:
-    // the network's partly filled rounds and its tail leave SMs idle that these ~20 short kernels take (measured with
-    // the fused LSTM2: 9.66 M sites/s end to end against 8.73 M when they wait for the pass to end).  With the
-    // hoisted LSTM2 (C3R_LSTM2=hoisted) every SM is busy and interleaving delays both (2.62 against 2.35 ms per
-    // pass): there, and with C3R_NO_INTERLEAVE, the stages wait.
-    if (ctx->prm.nn_impl == 1 && (!lstm2_fused() || getenv("C3R_NO_INTERLEAVE") != nullptr))
-        if (cudaEvent_t done = tc_pass_done(ctx->tc)) CK(cudaStreamWaitEvent(st, done, 0));
+    // the network's partly filled rounds and its tail leave SMs idle that these ~20 short kernels take (9.66 M sites/s
+    // end to end against 8.73 M when they wait for the pass to end).
     s.in_use = true;                                 // from here on every error path releases the slot (below)
     lap(1);
     int rc = run_stage_a(ctx, s);
@@ -921,13 +917,10 @@ int c3r_debug_fetch(c3r_ctx* ctx, int which, void* dst, int64_t max_bytes, int64
     const void* src = nullptr;
     size_t bytes = 0;
     switch (which) {
-        case 0: src = t.h1_cur ? t.h1_cur : t.h1; bytes = tiles * NT * 4 * TC_IMG * 2; break;
-        case 1:
-            if (lstm2_fused()) return fail(ctx, C3R_ERR_STATE, "zx2 does not exist: LSTM2 runs fused (C3R_LSTM2=hoisted keeps it)");
-            src = t.zx2; bytes = tiles * NT * 10 * ZX_CHUNK_WORDS * 4; break;
+        case 0: src = t.h1_cur ? t.h1_cur : t.h1[0]; bytes = tiles * NT * 4 * TC_IMG * 2; break;
         case 2: src = t.h2; bytes = tiles * NT * 5 * TC_IMG * 2; break;
         case 3: src = t.l4; bytes = tiles * 128 * DENSE * 4; break;
-        case 4: src = t.trace; bytes = t.trace ? (2 * 2 * NT * 8 * 8 + 64 * 32) * sizeof(long long) : 0; break;
+        case 4: src = t.trace; bytes = t.trace ? 2 * 2 * NT * 8 * 8 * sizeof(long long) : 0; break;
         default: return fail(ctx, C3R_ERR_ARG, "unknown buffer");
     }
     if ((int64_t)bytes > max_bytes) bytes = (size_t)max_bytes;

@@ -1,8 +1,7 @@
 // LSTM2 with its input projection fused into the recurrent step ("fused LSTM2").
 //
-// The hoisted form (k_gemm_zx + k_lstm_tc<5,0>) writes the projection zx2 = h1 . W2 + b to HBM (127 KB per site)
-// and reads it back: 4.5 of the 5.4 GB a pass moves.  Here the projection never leaves the SM: every step's
-// accumulator is  z_t = h1_t . W2_hi + h1_t . W2_lo + h2_{t-1} . U2 + [1 1 0..] . [b_hi ; b_lo ; 0..]  (K = 688) in TMEM,
+// The projection never leaves the SM: every step's accumulator is
+//   z_t = h1_t . W2_hi + h1_t . W2_lo + h2_{t-1} . U2 + [1 1 0..] . [b_hi ; b_lo ; 0..]  (K = 688) in TMEM,
 // issued as tcgen05 cta_group::2 MMAs (M = 256 sites, N = 128 gate columns per chunk) by the pair's leader.
 // W2 (hi + lo fp16 terms) and U2 do not fit next to the operands in 227 KB, so the weights are not resident: they
 // stream from L2 through a ring of 16 KB stages in exactly the order the MMAs consume them - the same 430 KB
@@ -19,7 +18,10 @@
 // chosen by elect.sync (straight-line UTCHMMA, ~40 cycles each).
 //
 // The projection part of a chunk has no dependency on h_{t-1}, so it is issued while the gate warps still work on
-// the previous chunk: the tensor pipe, idle 83 % of the time in the hoisted recurrence, carries the projection.
+// the previous chunk, in the tensor pipe's idle time of the recurrence.
+// This kernel replaced a hoisted form (k_gemm_zx + k_lstm_tc<5,0>) that wrote the projection zx2 = h1 . W2 + b to HBM
+// (127 KB per site) and read it back - 4.5 of the 5.4 GB a pass moved - while its recurrence left the tensor pipe
+// idle 83 % of the time.
 // Math restated from /root/reference/clair3_rna/model.py:132-136,181 (Bidirectional LSTM, 160 units, Keras gate
 // order i,f,c,o); gate stage identical to k_lstm_tc.
 #pragma once
@@ -358,10 +360,9 @@ __global__ void __launch_bounds__(L2F_THREADS, 1) k_lstm2_fused(Lstm2fArgs a) {
 // c*32 + (hr*64+j)%32; i, f, o columns carry 0.5 * z like every other packed LSTM weight.
 inline void lstm2f_pack(std::vector<uint8_t>& out, const float* h, size_t o_w2, size_t o_b2, size_t o_u2) {
     out.assign((size_t)4 * L2F_STREAM_BYTES, 0);
-    const bool no_lo = getenv("C3R_L2F_NOLO") != nullptr;     // experiment: W2 rounded to one fp16 (the low-order images are zero)
-    auto split = [no_lo](float w, __half& hi, __half& lo) {
+    auto split = [](float w, __half& hi, __half& lo) {
         hi = __float2half(w);
-        lo = __float2half(no_lo ? 0.0f : w - __half2float(hi));
+        lo = __float2half(w - __half2float(hi));
     };
     for (int dir = 0; dir < 2; ++dir)
         for (int hr = 0; hr < 2; ++hr) {

@@ -6,12 +6,12 @@
 //
 // Kernels
 //   k_gemm_tc   tcgen05 GEMM, cta_group::1, 128x128 tiles, bulk-async-copy (TMA unit) operand
-//               pipeline.  Used for LSTM2's hoisted input projection (K=256, N=1280) and L4
-//               (K=10560, N=128, +SELU).
-//   k_lstm_tc   persistent recurrent layer, cta_group::2: a CTA pair owns 256 sites of one
-//               direction; the recurrent (and, for LSTM1, input) weights stay resident in
-//               shared memory split across the pair; per step tcgen05.mma -> TMEM -> gates in
-//               registers -> h back to shared memory as the next step's A operand.
+//               pipeline.  Used for L4 (K=10560, N=128) and L5 (K=128, N=256, +SELU).
+//   k_lstm_tc   LSTM1 as a persistent recurrent layer, cta_group::2: a CTA pair owns 256 sites of
+//               one direction; the input and recurrent weights stay resident in shared memory
+//               split across the pair; per step tcgen05.mma -> TMEM -> gates in registers -> h
+//               back to shared memory as the next step's A operand.
+//   LSTM2 is k_lstm2_fused (nn_lstm2f.cuh).
 //
 // Operand layout everywhere: K-major, no swizzle, 8x(16 B) core matrices; element (r, k) of a
 // tile with R rows sits at  (k/8)*R*8 + r*8 + k%8  halfs  (LBO = R*16 B, SBO = 128 B).
@@ -31,34 +31,12 @@
 
 namespace c3r {
 
-// The hoisted LSTM2 input projection zx2 is the largest array of the network (41 KB per site and direction) and
-// both its producer (k_gemm_zx) and its consumer (k_lstm_tc<5,0>) are bound by moving it through HBM, so it is
-// stored as 24-bit floats (fp32 rounded to 15 mantissa bits, relative error 2^-17, far below the fp16 operand
-// rounding of the recurrent MMA): 4 values in 3 words, planar so that every store and load stays coalesced:
-//   [tile][t][dir*CH + chunk][32 col-groups][3 planes][128 rows] uint32
-constexpr int ZX_CHUNK_WORDS = 32 * 3 * 128;
-__device__ __forceinline__ uint32_t f24_bits(float v) { return (__float_as_uint(v) + 0x80u) >> 8; }
-// words: w0 = hi16(a) | hi16(b) << 16, w1 = hi16(c) | hi16(d) << 16, w2 = the four low bytes; one byte permute per
-// value on the way back (its lowest byte repeats the low byte instead of being zero: 2^-16 relative, immaterial)
-__device__ __forceinline__ void pack24(float a, float b, float c, float d, uint32_t& w0, uint32_t& w1, uint32_t& w2) {
-    const uint32_t ua = f24_bits(a), ub = f24_bits(b), uc = f24_bits(c), ud = f24_bits(d);
-    w0 = __byte_perm(ua, ub, 0x6521);
-    w1 = __byte_perm(uc, ud, 0x6521);
-    w2 = __byte_perm(__byte_perm(ua, ub, 0x0040), __byte_perm(uc, ud, 0x0040), 0x5410);
-}
-__device__ __forceinline__ void unpack24(uint32_t w0, uint32_t w1, uint32_t w2, float& a, float& b, float& c, float& d) {
-    a = __uint_as_float(__byte_perm(w0, w2, 0x1044));
-    b = __uint_as_float(__byte_perm(w0, w2, 0x3255));
-    c = __uint_as_float(__byte_perm(w1, w2, 0x1066));
-    d = __uint_as_float(__byte_perm(w1, w2, 0x3277));
-}
-
 constexpr int TC_TILE = 128;                 // sites per CTA tile
 constexpr int TC_KB = 64;                    // K per pipeline stage
 constexpr int TC_IMG = TC_TILE * TC_KB;      // halfs in one 128x64 operand image (16 KB)
 
 // ================================================================== GEMM
-// Both GEMMs run the split-precision product  A_hi*B_hi + A_lo*B_hi + A_hi*B_lo  (A = A_hi + A_lo and
+// The GEMM runs the split-precision product  A_hi*B_hi + A_lo*B_hi + A_hi*B_lo  (A = A_hi + A_lo and
 // B = B_hi + B_lo as two fp16 terms each), which removes the fp16 rounding of both operands.
 struct GemmArgs {
     const __half* A;      // [m_tiles][n_kb][TC_IMG]
@@ -67,13 +45,10 @@ struct GemmArgs {
     const __half* B_lo;
     int terms;            // split-precision products as a bit mask: 1 = A_hi*B_hi, 2 = A_lo*B_hi, 4 = A_hi*B_lo
     const float* bias;    // [n_tiles*128], GEMM column order
-    float* out;
+    float* out;           // row-major [m*128+r][n_tiles*128], + bias + SELU
     int m_tiles, n_tiles, n_kb;
-    int mode;             // 0: 24-bit ZX layout [m][n][32 col-groups][3][128 rows]   1: row-major [m*128+r][n_tiles*128] + SELU
-    int ksplit;           // mode 1: K cut into ksplit ranges, one work item each; > 1: raw partial sums (no bias, no SELU)
-    size_t split_stride;  //         go to out + range * split_stride and the consumer adds them up (k_heads)
-    int dbg;              // experiments: 1 = skip the output stores, 2 = hi*hi term only
-    long long* trace;     // optional [64 tiles][32 events] SM-clock stamps of CTA 0
+    int ksplit;           // K cut into ksplit ranges, one work item each; > 1: raw partial sums (no bias, no SELU)
+    size_t split_stride;  // go to out + range * split_stride and the consumer adds them up (k_l4_finish)
     int* err;
 };
 
@@ -183,28 +158,15 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) k_gemm_tc(GemmArgs g) {
                 uint32_t v[16];
                 ptx::tmem_ld16(taddr + j * 16, v);
                 ptx::tmem_wait_ld();
-                if (g.mode == 0) {
-                    float4* o = (float4*)g.out + (((size_t)m * g.n_tiles + n) * 32 + j * 4) * 128 + row;
+                float* o = g.out + ((size_t)m * 128 + row) * ((size_t)g.n_tiles * 128) + (size_t)n * 128 + j * 16;
+                if (ksplit > 1) {
+                    float4* o4 = (float4*)(o + (size_t)ks * g.split_stride);
 #pragma unroll
-                    for (int c4 = 0; c4 < 4; ++c4) {
-                        float4 f;
-                        f.x = __uint_as_float(v[c4 * 4 + 0]) + bias[j * 16 + c4 * 4 + 0];
-                        f.y = __uint_as_float(v[c4 * 4 + 1]) + bias[j * 16 + c4 * 4 + 1];
-                        f.z = __uint_as_float(v[c4 * 4 + 2]) + bias[j * 16 + c4 * 4 + 2];
-                        f.w = __uint_as_float(v[c4 * 4 + 3]) + bias[j * 16 + c4 * 4 + 3];
-                        o[(size_t)c4 * 128] = f;
-                    }
+                    for (int c = 0; c < 4; ++c)
+                        o4[c] = make_float4(__uint_as_float(v[4 * c]), __uint_as_float(v[4 * c + 1]), __uint_as_float(v[4 * c + 2]), __uint_as_float(v[4 * c + 3]));
                 } else {
-                    float* o = g.out + ((size_t)m * 128 + row) * ((size_t)g.n_tiles * 128) + (size_t)n * 128 + j * 16;
-                    if (ksplit > 1) {
-                        float4* o4 = (float4*)(o + (size_t)ks * g.split_stride);
 #pragma unroll
-                        for (int c = 0; c < 4; ++c)
-                            o4[c] = make_float4(__uint_as_float(v[4 * c]), __uint_as_float(v[4 * c + 1]), __uint_as_float(v[4 * c + 2]), __uint_as_float(v[4 * c + 3]));
-                    } else {
-#pragma unroll
-                        for (int c = 0; c < 16; ++c) o[c] = seluf_(__uint_as_float(v[c]) + bias[j * 16 + c]);
-                    }
+                    for (int c = 0; c < 16; ++c) o[c] = seluf_(__uint_as_float(v[c]) + bias[j * 16 + c]);
                 }
             }
             ptx::tc_fence_before();
@@ -217,233 +179,11 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) k_gemm_tc(GemmArgs g) {
     if (warp == 1) ptx::tmem_dealloc<1>(tmem, 256);
 }
 
-// ------------------------------------------------------------------ A-stationary 2-CTA variant
-// LSTM2's hoisted input projection (K = 256, N = 1280) as tcgen05 cta_group::2 MMAs (M = 256, N = 256).
-// A CTA pair owns two 128-site m-tiles: each CTA keeps ITS tile's activation images resident (hi and
-// lo fp16 terms, 4 x 32 KB, one per 64-wide k block) and streams ITS half (128 of 256 columns) of the
-// weight images through a 3-stage ring of 32 KB stages (hi and lo image of one k block).
-// Per stage 12 MMAs:  A_hi*B_hi + A_lo*B_hi + A_hi*B_lo  for the four k16 steps of the block.
-// The activation images are re-loaded per k block as soon as the last n-tile has consumed that block
-// (a_free[kb] -> a_full[kb]), so switching m-tiles overlaps with the tail of the previous one.
-// Only the leader CTA issues MMAs; the peer relays "my stage / my A block has landed" with one
-// cluster-scope arrival each, commits are multicast to both CTAs.  CTA pair p walks the n-tiles starting at
-// p mod n_tiles, so that the 74 pairs do not all pull the same weight block out of L2 at the same moment.
-constexpr int ZXG_KB = 4;                                   // K = 256 = 4 k blocks of 64
-constexpr int ZXG_STAGES = 3;
-constexpr int ZXG_EPI_WARPS = 8;                            // two per TMEM lane quarter, 128 of the 256 columns each
-constexpr int ZXG_THREADS = 64 + 32 * ZXG_EPI_WARPS + 32;   // warp 0: weight ring, 1: MMA / relay, 2-9: epilogue, 10: activation loader
-constexpr int ZXG_SMEM = (2 * ZXG_KB + 2 * ZXG_STAGES) * TC_IMG * 2 + 1024 + 512;
-
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(ZXG_THREADS, 1) k_gemm_zx(GemmArgs g) {
-    extern __shared__ __align__(1024) uint8_t smem[];
-    constexpr uint32_t IMG_B = TC_IMG * 2;                  // 16 KB: a 128x64 image
-    uint8_t* tail = smem + (2 * ZXG_KB + 2 * ZXG_STAGES) * IMG_B;
-    float* bias_s = (float*)tail;                           // this n-tile's 256 bias values
-    uint64_t* bars = (uint64_t*)(tail + 1024);
-    // bars: 0-2 full | 3-5 empty | 6,7 acc_full | 8,9 acc_empty | 10-13 a_full | 14-17 a_free |
-    //       18-20 peer_full (leader) | 21-24 peer_a_full (leader) ; tmem ptr
-    uint32_t* tmem_ptr_s = (uint32_t*)(bars + 26);
-    const int n_tiles = g.n_tiles;                          // 256-column tiles
-    const uint32_t s_base = ptx::smem_u32(smem);
-    const uint32_t s_a = s_base, s_b = s_base + 2 * ZXG_KB * IMG_B;     // A: [kb][hi | lo], B ring: [stage][hi | lo]
-    const uint32_t b0 = ptx::smem_u32(bars);
-    const uint32_t b_full = b0, b_empty = b0 + 24, b_accf = b0 + 48, b_acce = b0 + 64, b_afull = b0 + 80,
-                   b_afree = b0 + 112, b_pfull = b0 + 144, b_pafull = b0 + 168;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t rank = ptx::cluster_ctarank();
-    const int pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
-    const int m_pairs = g.m_tiles / 2;                      // m_tiles is even (tiles come in pairs)
-    if (threadIdx.x == 0) {
-        for (int i = 0; i < ZXG_STAGES; ++i) {
-            ptx::mbar_init(b_full + 8 * i, 1); ptx::mbar_init(b_empty + 8 * i, 1); ptx::mbar_init(b_pfull + 8 * i, 1);
-        }
-        for (int i = 0; i < 2; ++i) { ptx::mbar_init(b_accf + 8 * i, 1); ptx::mbar_init(b_acce + 8 * i, 2 * ZXG_EPI_WARPS); }
-        for (int i = 0; i < ZXG_KB; ++i) {
-            ptx::mbar_init(b_afull + 8 * i, 1); ptx::mbar_init(b_afree + 8 * i, 1); ptx::mbar_init(b_pafull + 8 * i, 1);
-        }
-        ptx::fence_barrier_init();
-    }
-    if (warp == 1) {
-        ptx::tmem_alloc<2>(ptx::smem_u32(tmem_ptr_s), 512);
-        ptx::tmem_relinquish<2>();
-    }
-    ptx::tc_fence_before();
-    __syncthreads();
-    ptx::cluster_sync();
-    ptx::tc_fence_after();
-    const uint32_t tmem = *tmem_ptr_s;
-    const uint32_t idesc = ptx::make_idesc_f16(256, 256);
-
-    if (warp == 0) {
-        if (lane == 0) {
-            // ---------------------------------------------------- weight ring producer (both CTAs, own half)
-            uint32_t it = 0;
-            for (int mp = pair; mp < m_pairs; mp += n_pairs)
-                for (int n = 0; n < n_tiles; ++n)
-                    for (int kb = 0; kb < ZXG_KB; ++kb, ++it) {
-                        const uint32_t s = it % ZXG_STAGES, ph = (it / ZXG_STAGES) & 1;
-                        ptx::mbar_wait(b_empty + 8 * s, ph ^ 1, g.err, 112);
-                        if (g.dbg == 2 && it >= ZXG_STAGES) { ptx::mbar_arrive(b_full + 8 * s); continue; }   // experiment: no weight traffic
-                        ptx::mbar_arrive_expect_tx(b_full + 8 * s, 2 * IMG_B);
-                        // weight images are [n256][rank half][kb64][128 x 64]
-                        const size_t off = ((((size_t)((n + pair) % n_tiles) * 2 + rank) * ZXG_KB) + kb) * TC_IMG;
-                        ptx::bulk_g2s(s_b + s * 2 * IMG_B, g.B + off, IMG_B, b_full + 8 * s);
-                        ptx::bulk_g2s(s_b + s * 2 * IMG_B + IMG_B, g.B_lo + off, IMG_B, b_full + 8 * s);
-                    }
-        }
-    } else if (warp == 2 + ZXG_EPI_WARPS) {
-        if (lane == 0) {
-            // ---------------------------------------------------- activation loader (both CTAs, own tile)
-            uint32_t mi = 0;
-            for (int mp = pair; mp < m_pairs; mp += n_pairs, ++mi) {
-                const int m = 2 * mp + (int)rank;
-                for (int kb = 0; kb < ZXG_KB; ++kb) {
-                    ptx::mbar_wait(b_afree + 8 * kb, (mi & 1) ^ 1, g.err, 111);    // last n-tile of the previous pair used it
-                    const bool lo = g.terms & 2;                    // the low-order activation image is only read by term 2
-                    ptx::mbar_arrive_expect_tx(b_afull + 8 * kb, lo ? 2 * IMG_B : IMG_B);
-                    ptx::bulk_g2s(s_a + kb * 2 * IMG_B, g.A + ((size_t)m * ZXG_KB + kb) * TC_IMG, IMG_B, b_afull + 8 * kb);
-                    if (lo) ptx::bulk_g2s(s_a + kb * 2 * IMG_B + IMG_B, g.A_lo + ((size_t)m * ZXG_KB + kb) * TC_IMG, IMG_B, b_afull + 8 * kb);
-                }
-                if (rank == 1)
-                    for (int kb = 0; kb < ZXG_KB; ++kb) {
-                        ptx::mbar_wait(b_afull + 8 * kb, mi & 1, g.err, 121);
-                        ptx::mbar_arrive_cluster(b_pafull + 8 * kb, 0);
-                    }
-            }
-        }
-    } else if (warp == 1) {
-        if (lane == 0 && rank == 1) {
-            // ---------------------------------------------------- peer relay: stage landed -> leader
-            uint32_t it = 0;
-            for (int mp = pair; mp < m_pairs; mp += n_pairs)
-                for (int n = 0; n < n_tiles; ++n)
-                    for (int kb = 0; kb < ZXG_KB; ++kb, ++it) {
-                        const uint32_t s = it % ZXG_STAGES, ph = (it / ZXG_STAGES) & 1;
-                        ptx::mbar_wait(b_full + 8 * s, ph, g.err, 122);
-                        ptx::mbar_arrive_cluster(b_pfull + 8 * s, 0);
-                    }
-        }
-        if (lane == 0 && rank == 0) {
-            // ---------------------------------------------------- MMA issue (leader)
-            uint32_t it = 0, tc = 0, mi = 0;
-            for (int mp = pair; mp < m_pairs; mp += n_pairs, ++mi) {
-                for (int n = 0; n < n_tiles; ++n, ++tc) {
-                    const uint32_t slot = tc & 1, aph = (tc >> 1) & 1;
-                    ptx::mbar_wait_cluster(b_acce + 8 * slot, aph ^ 1, g.err, 114);
-                    ptx::tc_fence_after();
-                    const bool trm = g.trace && blockIdx.x == 0 && tc < 64;
-                    if (trm) g.trace[tc * 32 + 16] = clock64();
-                    for (int kb = 0; kb < ZXG_KB; ++kb, ++it) {
-                        const uint32_t s = it % ZXG_STAGES, ph = (it / ZXG_STAGES) & 1;
-                        if (n == 0) {                                   // this pair-tile's activation block
-                            ptx::mbar_wait(b_afull + 8 * kb, mi & 1, g.err, 113);
-                            ptx::mbar_wait_cluster(b_pafull + 8 * kb, mi & 1, g.err, 123);
-                        }
-                        ptx::mbar_wait(b_full + 8 * s, ph, g.err, 115);
-                        ptx::mbar_wait_cluster(b_pfull + 8 * s, ph, g.err, 125);
-                        ptx::tc_fence_after();
-                        if (trm) g.trace[tc * 32 + 8 + kb] = clock64();
-                        // descriptors once per stage, then constant adds (the address field counts 16-byte units)
-                        const uint64_t dA0 = ptx::make_smem_desc(s_a + kb * 2 * IMG_B, TC_TILE * 16, 128);
-                        const uint64_t dB0 = ptx::make_smem_desc(s_b + s * 2 * IMG_B, TC_TILE * 16, 128);
-#pragma unroll
-                        for (int term = 0; term < 3; ++term) {          // A_hi*B_hi, A_lo*B_hi, A_hi*B_lo
-                            if (!((g.terms >> term) & 1)) continue;
-#pragma unroll
-                            for (int k4 = 0; k4 < TC_KB / 16; ++k4) {
-                                const uint64_t da = dA0 + (uint64_t)(((term == 1 ? IMG_B : 0) + k4 * 2 * (TC_TILE * 16)) >> 4);
-                                const uint64_t db = dB0 + (uint64_t)(((term == 2 ? IMG_B : 0) + k4 * 2 * (TC_TILE * 16)) >> 4);
-                                ptx::mma_f16<2>(tmem + slot * 256, da, db, idesc, (kb > 0 || term > 0 || k4 > 0) ? 1u : 0u);
-                            }
-                        }
-                        ptx::mma_commit_2_mcast(b_empty + 8 * s, 3);
-                        if (n == n_tiles - 1) ptx::mma_commit_2_mcast(b_afree + 8 * kb, 3);   // block kb may be re-loaded
-                    }
-                    ptx::mma_commit_2_mcast(b_accf + 8 * slot, 3);
-                    if (trm) g.trace[tc * 32 + 17] = clock64();
-                }
-            }
-        }
-    } else {
-        // -------------------------------------------------------- epilogue (both CTAs, own rows)
-        // warp -> TMEM lane quarter (warp & 3) and one of the two 128-column chunks of the tile
-        constexpr int EPI_T = 32 * ZXG_EPI_WARPS;
-        const int et = threadIdx.x - 64;                        // 0 .. EPI_T-1
-        const int q = warp & 3;
-        const int half = (warp - 2) >> 2;
-        const int row = q * 32 + lane;
-        uint32_t tc = 0;
-        for (int mp = pair; mp < m_pairs; mp += n_pairs) {
-            const int m = 2 * mp + (int)rank;
-            {
-                // pull the NEXT pair-tile's activation images (2 x 64 KB, read once from HBM) towards L2 now,
-                // one 128-byte line per prefetch over the epilogue threads: the bulk copies that re-load
-                // them later are then L2 hits and do not stall the (in-order) copy queue of the weight ring
-                const int mn = m + 2 * n_pairs;
-                if (mn < g.m_tiles) {
-                    const uint8_t* ph = (const uint8_t*)(g.A + (size_t)mn * ZXG_KB * TC_IMG);
-                    const uint8_t* pl = (const uint8_t*)(g.A_lo + (size_t)mn * ZXG_KB * TC_IMG);
-                    for (uint32_t o = et * 128; o < ZXG_KB * IMG_B; o += EPI_T * 128) {
-                        ptx::prefetch_l2(ph + o);
-                        if (g.terms & 2) ptx::prefetch_l2(pl + o);
-                    }
-                }
-            }
-            for (int n = 0; n < n_tiles; ++n, ++tc) {
-                const uint32_t slot = tc & 1, aph = (tc >> 1) & 1;
-                asm volatile("bar.sync 1, %0;" :: "n"(EPI_T) : "memory");      // previous tile's bias readers are done
-                const int nn = (n + pair) % n_tiles;            // same rotation as the weight loader
-                bias_s[et] = g.bias[(size_t)nn * 256 + et];
-                asm volatile("bar.sync 1, %0;" :: "n"(EPI_T) : "memory");
-                const float* bias = bias_s + half * 128;
-                ptx::mbar_wait(b_accf + 8 * slot, aph, g.err, 116);
-                ptx::tc_fence_after();
-                const bool tre = g.trace && blockIdx.x == 0 && tc < 64 && warp == 2 && lane == 0;
-                if (tre) g.trace[tc * 32 + 18] = clock64();
-                const uint32_t taddr = tmem + ((uint32_t)(q * 32) << 16) + slot * 256 + half * 128;
-                // ZX layout is per 128-column chunk: [m][n128][32 col-groups][3 planes][128 rows], 24-bit floats
-                uint32_t* o0 = (uint32_t*)g.out + (((size_t)m * (2 * n_tiles) + 2 * nn + half) * 32 * 3) * 128 + row;
-                // the TMEM load of the next 16 columns is in flight while the current 16 are packed and stored
-                uint32_t va[16], vb[16];
-                ptx::tmem_ld16(taddr, va);
-#pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    uint32_t (&v)[16] = (j & 1) ? vb : va;
-                    uint32_t (&vn)[16] = (j & 1) ? va : vb;
-                    ptx::tmem_wait_ld(v);
-                    if (j + 1 < 8) ptx::tmem_ld16(taddr + (j + 1) * 16, vn);
-                    uint32_t* o = o0 + (size_t)(j * 4 * 3) * 128;
-#pragma unroll
-                    for (int c4 = 0; c4 < 4; ++c4) {
-                        uint32_t w0, w1, w2;
-                        pack24(__uint_as_float(v[c4 * 4 + 0]) + bias[j * 16 + c4 * 4 + 0],
-                               __uint_as_float(v[c4 * 4 + 1]) + bias[j * 16 + c4 * 4 + 1],
-                               __uint_as_float(v[c4 * 4 + 2]) + bias[j * 16 + c4 * 4 + 2],
-                               __uint_as_float(v[c4 * 4 + 3]) + bias[j * 16 + c4 * 4 + 3], w0, w1, w2);
-                        if (g.dbg == 1 && w0 != 0x12345u) continue;    // experiment: no output traffic
-                        o[(size_t)(c4 * 3 + 0) * 128] = w0;
-                        o[(size_t)(c4 * 3 + 1) * 128] = w1;
-                        o[(size_t)(c4 * 3 + 2) * 128] = w2;
-                    }
-                }
-                ptx::tc_fence_before();
-                __syncwarp();
-                if (lane == 0) ptx::mbar_arrive_cluster(b_acce + 8 * slot, 0);
-                if (tre) g.trace[tc * 32 + 19] = clock64();
-            }
-        }
-    }
-    ptx::tc_fence_before();
-    __syncthreads();
-    ptx::cluster_sync();
-    if (warp == 1) ptx::tmem_dealloc<2>(tmem, 512);
-}
-
-// ================================================================== LSTM layer
+// ================================================================== LSTM1
 // One CTA pair (cluster of 2, tcgen05 cta_group::2) = 256 sites x one direction.
 //   CH      gate-column chunks per step; a chunk = 32 units x 4 gates = 128 accumulator columns
-//   KX      K of the input part fused into the step MMA (LSTM1: [x | x | 1 | 1 | 0..] against
-//           [W_hi ; W_lo ; b_hi ; b_lo ; 0]); 0 for LSTM2 whose input projection is hoisted
+//   KX      K of the input part fused into the step MMA ([x | x | 1 | 1 | 0..] against
+//           [W_hi ; W_lo ; b_hi ; b_lo ; 0])
 //   U       units (K of the recurrent part) = CH*32
 template <int CH, int KX>
 struct LstmCfg {
@@ -460,12 +200,8 @@ struct LstmCfg {
 
 struct LstmArgs {
     const __half* Wimg;     // [2 dirs][2 ranks][B_BYTES/2] operand images
-    const __half* xop;      // LSTM1: x operand images [tile][33][KX/8][128][8] (k_xop)
-    int C;
-    const float* zx;        // LSTM2: hoisted projection, 24-bit ZX layout [tile][33][2*CH][32][3][128] (words)
-    __half* hout;           // packed output [tile][33][KB_OUT][TC_IMG], high-order fp16 term
-    __half* hout_lo;        // low-order term: h - fp16(h), same layout; nullptr: the consumer does not use it
-    int kb_out;             // 64-column blocks per time step in hout (LSTM1: 4, LSTM2: 5)
+    const __half* xop;      // x operand images [tile][33][KX/8][128][8] (k_xop)
+    __half* hout;           // packed fp16 output [tile][33][4][TC_IMG]
     int64_t n_sites;        // valid sites (tensor rows); tiles beyond are zero
     int n_tiles;            // 128-site tiles (even)
     int* err;
@@ -501,8 +237,8 @@ __device__ __forceinline__ float sig_times_tanh(float zs, float zt) {
 }
 __device__ __forceinline__ float sigmoid_fast(float x) { return rcp_approx(1.0f + ex2_approx(-LOG2E * x)); }
 __device__ __forceinline__ float tanh_approx(float x) { float y; asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
-// sigmoid(z) from the pre-halved pre-activation x = 0.5 z (the i, f, o columns of every LSTM weight, bias and of the
-// hoisted projection are packed times 0.5 - an exact scaling - so the gate stage saves three multiplies per unit)
+// sigmoid(z) from the pre-halved pre-activation x = 0.5 z (the i, f, o columns of every LSTM weight and bias are
+// packed times 0.5 - an exact scaling - so the gate stage saves three multiplies per unit)
 __device__ __forceinline__ float sigmoid_tanh(float x) { return fmaf(tanh_approx(x), 0.5f, 0.5f); }
 
 // One LSTM cell update from the pre-activations (zi, zf, zo pre-halved, see above).
@@ -528,6 +264,7 @@ __device__ __forceinline__ void lstm_cell(float zi, float zf, float zg, float zo
 
 template <int CH, int KX>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(LSTM_THREADS, 1) k_lstm_tc(LstmArgs a) {
+    static_assert(KX > 0, "the input part is fused into the step MMA");
     typedef LstmCfg<CH, KX> Cfg;
     constexpr int U = Cfg::U, KT = Cfg::KT;
     extern __shared__ __align__(1024) uint8_t smem[];
@@ -601,10 +338,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(LSTM_THREADS, 1) k_l
                 for (int step = 0; step < NT; ++step) {
                     const uint32_t gstep = base_step + step;
                     const uint32_t buf = gstep & 1;
-                    if (KX > 0) {
-                        ptx::mbar_wait(b_xl + 8 * buf, (gstep >> 1) & 1, a.err, 202);
-                        ptx::mbar_wait(b_xr + 8 * buf, (gstep >> 1) & 1, a.err, 212);
-                    }
+                    ptx::mbar_wait(b_xl + 8 * buf, (gstep >> 1) & 1, a.err, 202);
+                    ptx::mbar_wait(b_xr + 8 * buf, (gstep >> 1) & 1, a.err, 212);
                     for (int c = 0; c < CH; ++c) {
                         const uint32_t use = base_use + step * CH + c;
                         const uint32_t slot = use & 1;
@@ -617,16 +352,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(LSTM_THREADS, 1) k_l
                         // of the whole CTA pair: descriptors are built once per chunk and advanced by constant adds
                         // (the start-address field counts 16-byte units and cannot carry out of its 14 bits here).
                         const uint64_t dB0 = ptx::make_smem_desc(s_B + c * (64 * KT * 2), 64 * 16, 128);
-                        bool first = true;
-                        if (KX > 0) {                              // the input part does not need h_{t-1}: it goes first
-                            const uint64_t dX0 = ptx::make_smem_desc(s_AX + buf * Cfg::AX_BYTES, TC_TILE * 16, 128);
+                        // the input part does not need h_{t-1}: it goes first
+                        const uint64_t dX0 = ptx::make_smem_desc(s_AX + buf * Cfg::AX_BYTES, TC_TILE * 16, 128);
 #pragma unroll
-                            for (int k = 0; k < KX / 16; ++k) {
-                                ptx::mma_f16<2>(tmem + slot * 128, dX0 + (uint64_t)(k * ((2 * TC_TILE * 16) >> 4)),
-                                                dB0 + (uint64_t)(k * ((2 * 64 * 16) >> 4)), IDESC, first ? 0u : 1u);
-                                first = false;
-                            }
-                        }
+                        for (int k = 0; k < KX / 16; ++k)
+                            ptx::mma_f16<2>(tmem + slot * 128, dX0 + (uint64_t)(k * ((2 * TC_TILE * 16) >> 4)),
+                                            dB0 + (uint64_t)(k * ((2 * 64 * 16) >> 4)), IDESC, k > 0 ? 1u : 0u);
                         // at the start of a step, h of the previous step must be complete in both CTAs
                         if (c == 0 && step > 0) {
                             ptx::mbar_wait(b_hrdy, (gstep - 1) & 1, a.err, 204);
@@ -636,13 +367,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(LSTM_THREADS, 1) k_l
                         if (step > 0) {
                             const uint64_t dH0 = ptx::make_smem_desc(s_AH + buf * Cfg::AH_BYTES, TC_TILE * 16, 128);
 #pragma unroll
-                            for (int k = 0; k < U / 16; ++k) {
+                            for (int k = 0; k < U / 16; ++k)
                                 ptx::mma_f16<2>(tmem + slot * 128, dH0 + (uint64_t)(k * ((2 * TC_TILE * 16) >> 4)),
-                                                dB0 + (uint64_t)(((KX / 8 + k * 2) * (64 * 16)) >> 4), IDESC, first ? 0u : 1u);
-                                first = false;
-                            }
+                                                dB0 + (uint64_t)(((KX / 8 + k * 2) * (64 * 16)) >> 4), IDESC, 1u);
                         }
-                        // (LSTM2, step 0: no MMA at all; the commit below still fires the barrier)
                         ptx::mma_commit_2_mcast(b_accf + 8 * slot, 3);
                         lstm_trace(a, tr, 0, step, c, 1);
                     }
@@ -668,25 +396,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(LSTM_THREADS, 1) k_l
                 }
             }
         } else if (warp == 1) {
-            // ------------------------------------------------ LSTM2: keep the hoisted projection two chunks ahead in L2
-            if (KX == 0 && lane == 0) {
-                // one (tile, t, dir, chunk) block of zx2 is 48 KB contiguous
-                for (int u = 0; u < NT * CH; ++u) {
-                    const int step = u / CH, c = u % CH;
-                    const int t = dir == 0 ? step : NT - 1 - step;
-                    ptx::bulk_prefetch_l2((const uint32_t*)a.zx + (((size_t)tile * NT + t) * (2 * CH) + dir * CH + c) * ZX_CHUNK_WORDS, ZX_CHUNK_WORDS * 4);
-                    if (u >= 2) {                            // pace on the MMA commits: use u-2 is complete
-                        const uint32_t use = base_use + u - 2;
-                        // best-effort pacing only: if this thread has fallen two uses behind the MMA thread the
-                        // parity test cannot tell (it would see "not yet" until the slot's next use), so give up
-                        // after a short spin instead of treating it as a protocol failure
-                        for (int spin = 0; spin < 2048; ++spin)
-                            if (ptx::mbar_try_wait(b_accf + 8 * (use & 1), (use >> 1) & 1)) break;
-                    }
-                }
-            }
-            // ------------------------------------------------ LSTM1: x_t operand tile, one bulk copy per step
-            if (KX > 0 && lane == 0) {
+            // ------------------------------------------------ x_t operand tile, one bulk copy per step
+            if (lane == 0) {
                 for (int step = 0; step < NT; ++step) {
                     const uint32_t gstep = base_step + step;
                     const uint32_t buf = gstep & 1;
@@ -711,154 +422,24 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(LSTM_THREADS, 1) k_l
             const int sub = gw >> 2;                         // which 8 units of the chunk's 32
             const int row = q * 32 + lane;
             const uint32_t lane_addr = (uint32_t)(q * 32) << 16;
-            if (KX == 0) {
-                // ---- LSTM2: the hoisted projection comes from HBM.  A chunk is processed as two groups of 4 units and the
-                // packed values of the NEXT group (which may belong to the next chunk or step) are requested before the
-                // current group's gate math, so their latency hides behind it instead of sitting in front of every chunk.
-                auto zsrc = [&](int hstep) -> const uint32_t* {                  // hstep = (step * CH + c) * 2 + ug
-                    const int ug = hstep & 1, cc = (hstep >> 1) % CH, st = (hstep >> 1) / CH;
-                    const int tt = dir == 0 ? st : NT - 1 - st;
-                    return (const uint32_t*)a.zx + (((size_t)tile * NT + tt) * (2 * CH) + dir * CH + cc) * ZX_CHUNK_WORDS +
-                           (size_t)((sub * 2 + ug) * 3) * 128 + row;
-                };
-                uint32_t zz[2][4][3];                            // group ug uses zz[ug] while zz[ug ^ 1] is being filled
-                {
-                    const uint32_t* zp = zsrc(0);
-#pragma unroll
-                    for (int gte = 0; gte < 4; ++gte)
-#pragma unroll
-                        for (int pl = 0; pl < 3; ++pl) zz[0][gte][pl] = zp[(size_t)(gte * 8 * 3 + pl) * 128];
-                }
-                for (int step = 0; step < NT; ++step) {
-                    const uint32_t gstep = base_step + step;
-                    const uint32_t nbuf = (gstep + 1) & 1;       // h_t goes to the buffer step+1 reads
-                    const int t = dir == 0 ? step : NT - 1 - step;
-                    uint8_t* ah = smem + Cfg::B_BYTES + nbuf * Cfg::AH_BYTES;
-                    __half* hout_t = a.hout + ((size_t)tile * NT + t) * a.kb_out * TC_IMG;
-                    __half* hout_lo_t = a.hout_lo + ((size_t)tile * NT + t) * a.kb_out * TC_IMG;
-                    const bool has_acc = step > 0;
-#pragma unroll
-                    for (int c = 0; c < CH; ++c) {
-                        const uint32_t use = base_use + step * CH + c;
-                        const uint32_t slot = use & 1;
-#pragma unroll
-                        for (int ug = 0; ug < 2; ++ug) {
-                            const int hnext = (step * CH + c) * 2 + ug + 1;
-                            if (hnext < NT * CH * 2) {
-                                const uint32_t* zp = zsrc(hnext);
-#pragma unroll
-                                for (int gte = 0; gte < 4; ++gte)
-#pragma unroll
-                                    for (int pl = 0; pl < 3; ++pl) zz[ug ^ 1][gte][pl] = zp[(size_t)(gte * 8 * 3 + pl) * 128];
-                            }
-                            if (ug == 0) {
-                                ptx::mbar_wait(b_accf + 8 * slot, (use >> 1) & 1, a.err, 208);
-                                ptx::tc_fence_after();
-                                lstm_trace(a, tr && gw == 0, rank, step, c, 2);
-                            }
-                            uint32_t cprev[4];
-                            uint32_t v[4][4];
-                            if (has_acc) {
-#pragma unroll
-                                for (int gte = 0; gte < 4; ++gte)
-                                    ptx::tmem_ld4(tmem + lane_addr + slot * 128 + gte * 32 + sub * 8 + ug * 4, v[gte]);
-                                ptx::tmem_ld4(tmem + lane_addr + Cfg::C_COL + c * 32 + sub * 8 + ug * 4, cprev);
-                                ptx::tmem_wait_ld();
-                            }
-                            if (ug == 0) lstm_trace(a, tr && gw == 0, rank, step, c, 3);
-                            if (ug == 1) {                       // the accumulator slot is in registers: hand it back
-                                ptx::tc_fence_before();
-                                __syncwarp();
-                                if (lane == 0) ptx::mbar_arrive(b_acce + 8 * slot);
-                                lstm_trace(a, tr && gw == 0, rank, step, c, 4);
-                            }
-                            float z[4][4];
-#pragma unroll
-                            for (int gte = 0; gte < 4; ++gte) {
-                                unpack24(zz[ug][gte][0], zz[ug][gte][1], zz[ug][gte][2], z[gte][0], z[gte][1], z[gte][2], z[gte][3]);
-                                if (has_acc) {
-#pragma unroll
-                                    for (int u = 0; u < 4; ++u) z[gte][u] += __uint_as_float(v[gte][u]);
-                                }
-                            }
-                            uint32_t cnew[4];
-                            float hv4[4];
-#pragma unroll
-                            for (int u = 0; u < 4; ++u) {
-                                const float cp = has_acc ? __uint_as_float(cprev[u]) : 0.0f;
-                                float cn;
-                                lstm_cell(z[0][u], z[1][u], z[2][u], z[3][u], cp, cn, hv4[u]);
-                                cnew[u] = __float_as_uint(cn);
-                            }
-                            // h as fp16 hi + lo terms, two values per conversion
-                            __half2 hh2[2], hl2[2];
-#pragma unroll
-                            for (int u = 0; u < 2; ++u) {
-                                hh2[u] = __floats2half2_rn(hv4[2 * u], hv4[2 * u + 1]);
-                                const float2 back = __half22float2(hh2[u]);
-                                hl2[u] = __floats2half2_rn(hv4[2 * u] - back.x, hv4[2 * u + 1] - back.y);
-                            }
-                            const __half2* hh = hh2;
-                            const __half2* hl = hl2;
-                            ptx::tmem_st4(tmem + lane_addr + Cfg::C_COL + c * 32 + sub * 8 + ug * 4, cnew);
-                            // h_t: next step's A operand (k index = unit): this group's 4 halfs of the row's 16-byte k8 cell
-                            const uint2 pk = *(const uint2*)hh;
-                            const int k8 = c * 4 + sub;
-                            *(uint2*)(ah + (size_t)k8 * (TC_TILE * 16) + row * 16 + ug * 8) = pk;
-                            if (ug == 1) {
-                                ptx::tmem_wait_st();
-                                if (c == CH - 1) {               // this warp's part of h_t is in shared memory: one
-                                    ptx::tc_fence_before();      // generic->async proxy fence covers all of its writes
-                                    ptx::fence_proxy_async();
-                                    __syncwarp();
-                                    if (lane == 0) ptx::mbar_arrive(b_hrdy);
-                                }
-                            }
-                            {
-                                const int col8 = (dir * U) / 8 + k8;             // 8-column group in the concat [fwd | bwd]
-                                const size_t oo = (size_t)(col8 / 8) * TC_IMG + (size_t)(col8 % 8) * (TC_TILE * 8) + row * 8 + ug * 4;
-                                *(uint2*)(hout_t + oo) = pk;
-                                if (a.hout_lo) *(uint2*)(hout_lo_t + oo) = *(const uint2*)hl;
-                            }
-                        }
-                    }
-                }
-            } else {
             for (int step = 0; step < NT; ++step) {
                 const uint32_t gstep = base_step + step;
                 const uint32_t nbuf = (gstep + 1) & 1;       // h_t goes to the buffer step+1 reads
                 const int t = dir == 0 ? step : NT - 1 - step;
                 uint8_t* ah = smem + Cfg::B_BYTES + nbuf * Cfg::AH_BYTES;
-                __half* hout_t = a.hout + ((size_t)tile * NT + t) * a.kb_out * TC_IMG;
-                __half* hout_lo_t = a.hout_lo + ((size_t)tile * NT + t) * a.kb_out * TC_IMG;
-                const bool has_acc = (KX > 0) || step > 0;
+                __half* hout_t = a.hout + ((size_t)tile * NT + t) * 4 * TC_IMG;
 #pragma unroll
                 for (int c = 0; c < CH; ++c) {
                     const uint32_t use = base_use + step * CH + c;
                     const uint32_t slot = use & 1;
-                    uint32_t zw[4][2][3];                        // LSTM2: this thread's 32 hoisted values, 24-bit packed
-                    if (KX == 0) {
-                        // hoisted projection: [tile][t][dir*CH + c][gate*8 + ug][plane][row]; requested before the wait
-                        const uint32_t* zp = (const uint32_t*)a.zx +
-                            (((size_t)tile * NT + t) * (2 * CH) + dir * CH + c) * ZX_CHUNK_WORDS + row;
-#pragma unroll
-                        for (int gte = 0; gte < 4; ++gte)
-#pragma unroll
-                            for (int ug = 0; ug < 2; ++ug)
-#pragma unroll
-                                for (int pl = 0; pl < 3; ++pl)
-                                    zw[gte][ug][pl] = zp[(size_t)((gte * 8 + sub * 2 + ug) * 3 + pl) * 128];
-                    }
                     ptx::mbar_wait(b_accf + 8 * slot, (use >> 1) & 1, a.err, 208);
                     ptx::tc_fence_after();
                     lstm_trace(a, tr && gw == 0, rank, step, c, 2);
                     uint32_t cprev[8];
                     uint32_t v[4][8];
-                    if (has_acc) {
 #pragma unroll
-                        for (int gte = 0; gte < 4; ++gte)
-                            ptx::tmem_ld8(tmem + lane_addr + slot * 128 + gte * 32 + sub * 8, v[gte]);
-                    }
+                    for (int gte = 0; gte < 4; ++gte)
+                        ptx::tmem_ld8(tmem + lane_addr + slot * 128 + gte * 32 + sub * 8, v[gte]);
                     if (step > 0) ptx::tmem_ld8(tmem + lane_addr + Cfg::C_COL + c * 32 + sub * 8, cprev);
                     ptx::tmem_wait_ld();
                     lstm_trace(a, tr && gw == 0, rank, step, c, 3);
@@ -866,34 +447,16 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(LSTM_THREADS, 1) k_l
                     __syncwarp();
                     if (lane == 0) ptx::mbar_arrive(b_acce + 8 * slot);
                     lstm_trace(a, tr && gw == 0, rank, step, c, 4);
-                    float z[4][8];
-#pragma unroll
-                    for (int gte = 0; gte < 4; ++gte) {
-                        if (KX == 0) {
-#pragma unroll
-                            for (int ug = 0; ug < 2; ++ug)
-                                unpack24(zw[gte][ug][0], zw[gte][ug][1], zw[gte][ug][2], z[gte][ug * 4 + 0], z[gte][ug * 4 + 1],
-                                         z[gte][ug * 4 + 2], z[gte][ug * 4 + 3]);
-                        } else {
-#pragma unroll
-                            for (int u = 0; u < 8; ++u) z[gte][u] = 0.0f;
-                        }
-                        if (has_acc) {
-#pragma unroll
-                            for (int u = 0; u < 8; ++u) z[gte][u] += __uint_as_float(v[gte][u]);
-                        }
-                    }
                     uint32_t cnew[8];
                     __align__(16) __half hh[8];
-                    __align__(16) __half hl[8];
 #pragma unroll
                     for (int u = 0; u < 8; ++u) {
                         const float cp = step > 0 ? __uint_as_float(cprev[u]) : 0.0f;
                         float cn, hv;
-                        lstm_cell(z[0][u], z[1][u], z[2][u], z[3][u], cp, cn, hv);
+                        lstm_cell(__uint_as_float(v[0][u]), __uint_as_float(v[1][u]), __uint_as_float(v[2][u]),
+                                  __uint_as_float(v[3][u]), cp, cn, hv);
                         cnew[u] = __float_as_uint(cn);
                         hh[u] = __float2half(hv);
-                        hl[u] = __float2half(hv - __half2float(hh[u]));
                     }
                     ptx::tmem_st8(tmem + lane_addr + Cfg::C_COL + c * 32 + sub * 8, cnew);
                     // h_t: next step's A operand (k index = unit)
@@ -907,16 +470,14 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(LSTM_THREADS, 1) k_l
                         __syncwarp();
                         if (lane == 0) ptx::mbar_arrive(b_hrdy);
                     }
-                    // layer output (hi + lo fp16 terms) goes out AFTER the arrival: the release fence of
-                    // the arrival would otherwise wait for these HBM stores on the recurrence's critical path
+                    // layer output goes out AFTER the arrival: the release fence of the arrival would
+                    // otherwise wait for these HBM stores on the recurrence's critical path
                     {
                         const int col8 = (dir * U) / 8 + k8;                 // 8-column group in the concat [fwd | bwd]
                         const size_t oo = (size_t)(col8 / 8) * TC_IMG + (size_t)(col8 % 8) * (TC_TILE * 8) + row * 8;
                         *(uint4*)(hout_t + oo) = pk;
-                        if (a.hout_lo) *(uint4*)(hout_lo_t + oo) = *(const uint4*)hl;
                     }
                 }
-            }
             }
             // the step_done commits multicast to this CTA have landed before it may exit
             if (gw == 0) {
@@ -1035,24 +596,13 @@ __global__ void __launch_bounds__(HOUT_WARPS * 32) k_heads_out(NetF32 w, const f
 // ================================================================== host side
 constexpr int L4_KSPLIT = 3;                 // L4's K = 165 k blocks goes in 3 ranges of 55 (see tc_l4_heads)
 
-// LSTM2 as one fused kernel (projection inside the recurrent step, nn_lstm2f.cuh) or, with C3R_LSTM2=hoisted, as the
-// projection GEMM + recurrent kernel pair that moves zx2 through HBM.
-inline bool lstm2_fused() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("C3R_LSTM2");
-        v = (e && std::string(e) == "hoisted") ? 0 : 1;
-    }
-    return v != 0;
-}
-
 struct TcNet {
     int ready = 0;
     int C = 18, KX = 48, sm_count = 148;
     void* wbuf = nullptr;          // all fp16 images + fp32 biases
     size_t wbytes = 0;
-    const __half *img1 = nullptr, *img2 = nullptr, *w2p = nullptr, *k4p = nullptr, *w2p_lo = nullptr, *k4p_lo = nullptr;
-    const float *b2p = nullptr, *b4 = nullptr;
+    const __half *img1 = nullptr, *k4p = nullptr, *k4p_lo = nullptr;
+    const float* b4 = nullptr;
     const uint8_t* wstream2 = nullptr;   // fused LSTM2: weight stream [2 dirs][2 halves][L2F_STREAM_BYTES]
     const __half *k5p = nullptr, *k5p_lo = nullptr;   // [L5_1 | L5_2] as one N = 256 GEMM: [2 n tiles][2 kb][TC_IMG]
     const float* b5p = nullptr;                        // [256]
@@ -1060,14 +610,15 @@ struct TcNet {
     void* abuf = nullptr;
     size_t abytes = 0;
     int cap_tiles = 0;
-    __half *h1 = nullptr, *h2 = nullptr, *h1_lo = nullptr, *h2_lo = nullptr, *xop = nullptr;
-    __half* h1_cur = nullptr;      // the h1 buffer of the pass queued last (fused LSTM2 alternates between h1 and h1_lo)
-    float *zx2 = nullptr, *l4 = nullptr, *l4p = nullptr;   // l4p: L4's partial sums [L4_KSPLIT][tiles*128][128]
+    __half* h1[2] = {};            // LSTM1 output, one buffer per pass parity (tc_forward)
+    __half *h2 = nullptr, *h2_lo = nullptr, *xop = nullptr;
+    __half* h1_cur = nullptr;      // the h1 buffer of the pass queued last
+    float *l4 = nullptr, *l4p = nullptr;                   // l4p: L4's partial sums [L4_KSPLIT][tiles*128][128]
     size_t l4_stride = 0;
     __half *l4h = nullptr, *l4h_lo = nullptr;              // l4 as fp16 operand images [tile][2 kb][TC_IMG] (hi, lo)
     float* a5 = nullptr;                                   // selu(L5_1) | selu(L5_2): [tiles*128][256]
     int* err = nullptr;
-    long long* trace = nullptr;    // [2 layers][2][33][8][8], filled when C3R_TRACE is set
+    long long* trace = nullptr;    // [LSTM1: 2 ranks][33][8][8] then the fused LSTM2 profile, filled when C3R_TRACE is set
     bool attr_set = false;
     struct TcPipe* pipe = nullptr; // second stream + events of the A/B tail overlap (tc_forward)
 };
@@ -1094,20 +645,15 @@ inline int tc_build(TcNet& t, const NetF32& net, const float* h, size_t o_w1, si
     t.KX = C == 18 ? 48 : 64;
     t.sm_count = sm_count;
     const int KX = t.KX;
-    const int KT1 = KX + U1, KT2 = U2;
+    const int KT1 = KX + U1;
     const size_t n_img1 = (size_t)2 * 2 * 4 * 64 * KT1;          // [dir][rank][chunk][64 x KT1]
-    const size_t n_img2 = (size_t)2 * 2 * 5 * 64 * KT2;
-    const size_t n_w2p = (size_t)10 * 4 * TC_IMG;                 // [n_tile][kb][128x64]
     const size_t n_k4p = (size_t)(L4_IN / TC_KB) * TC_IMG;
     const size_t n_k5p = (size_t)2 * 2 * TC_IMG;
-    std::vector<__half> hb(n_img1 + n_img2 + 2 * n_w2p + 2 * n_k4p + 2 * n_k5p);
-    std::vector<float> fb(2 * G2 + DENSE + 2 * DENSE);
+    std::vector<__half> hb(n_img1 + 2 * n_k4p + 2 * n_k5p);
+    std::vector<float> fb(DENSE + 2 * DENSE);
     __half* img1 = hb.data();
-    __half* img2 = img1 + n_img1;
-    __half* w2p = img2 + n_img2;
-    __half* k4p = w2p + n_w2p;
-    __half* w2p_lo = k4p + n_k4p;
-    __half* k4p_lo = w2p_lo + n_w2p;
+    __half* k4p = img1 + n_img1;
+    __half* k4p_lo = k4p + n_k4p;
     __half* k5p = k4p_lo + n_k4p;
     __half* k5p_lo = k5p + n_k5p;
     auto split = [](float w, __half& hi, __half& lo) {
@@ -1116,8 +662,7 @@ inline int tc_build(TcNet& t, const NetF32& net, const float* h, size_t o_w1, si
     };
     // Keras gate column of chunk column j (gate-major inside a chunk: j = gate*32 + unit_local)
     for (int dir = 0; dir < 2; ++dir)
-        for (int rank = 0; rank < 2; ++rank) {
-            // LSTM1
+        for (int rank = 0; rank < 2; ++rank)
             for (int c = 0; c < 4; ++c) {
                 __half* im = img1 + ((((size_t)dir * 2 + rank) * 4 + c) * 64) * KT1;
                 for (int j = 0; j < 64; ++j) {
@@ -1142,43 +687,13 @@ inline int tc_build(TcNet& t, const NetF32& net, const float* h, size_t o_w1, si
                     }
                 }
             }
-            // LSTM2 (recurrent part only)
-            for (int c = 0; c < 5; ++c) {
-                __half* im = img2 + ((((size_t)dir * 2 + rank) * 5 + c) * 64) * KT2;
-                for (int j = 0; j < 64; ++j) {
-                    const int col = rank * 64 + j, gate = col / 32, ul = col % 32;
-                    const int kc = gate * U2 + c * 32 + ul;
-                    const float gs = gate == 2 ? 1.0f : 0.5f;
-                    for (int k = 0; k < KT2; ++k)
-                        im[img_index(64, j, k)] = __float2half(gs * h[o_u2 + (size_t)dir * U2 * G2 + (size_t)k * G2 + kc]);
-                }
-            }
-        }
-    // hoisted LSTM2 input projection.  GEMM column = (dir*5 + chunk)*128 + gate*32 + unit_local; the weight
-    // images are [n256 = column/256][half = CTA rank][kb64][128 rows x 64 k], bias in the same column order
-    for (int dir = 0; dir < 2; ++dir)
-        for (int c = 0; c < 5; ++c) {
-            const int nt = dir * 5 + c;
-            for (int j = 0; j < 128; ++j) {
-                const int gate = j / 32, ul = j % 32;
-                const int kc = gate * U2 + c * 32 + ul;
-                const int col = nt * 128 + j;
-                const float gs = gate == 2 ? 1.0f : 0.5f;
-                fb[col] = gs * h[o_b2 + dir * G2 + kc];
-                for (int k = 0; k < H1W; ++k) {
-                    const int n256 = col / 256, half = (col % 256) / 128, r = col % 128;
-                    const size_t ix = (((size_t)n256 * 2 + half) * 4 + k / TC_KB) * TC_IMG + img_index(128, r, k % TC_KB);
-                    split(gs * h[o_w2 + (size_t)k * 2 * G2 + dir * G2 + kc], w2p[ix], w2p_lo[ix]);
-                }
-            }
-        }
     for (int k = 0; k < L4_IN; ++k)
         for (int j = 0; j < DENSE; ++j)
         {
             const size_t ix = (size_t)(k / TC_KB) * TC_IMG + img_index(128, j, k % TC_KB);
             split(h[o_k4 + (size_t)k * DENSE + j], k4p[ix], k4p_lo[ix]);
         }
-    for (int j = 0; j < DENSE; ++j) fb[2 * G2 + j] = h[o_b4 + j];
+    for (int j = 0; j < DENSE; ++j) fb[j] = h[o_b4 + j];
     // L5_1 and L5_2 side by side: GEMM column n*128 + j = unit j of layer n; B image row = output unit, k = input
     for (int n = 0; n < 2; ++n)
         for (int k = 0; k < DENSE; ++k)
@@ -1186,7 +701,7 @@ inline int tc_build(TcNet& t, const NetF32& net, const float* h, size_t o_w1, si
                 const size_t ix = ((size_t)n * 2 + k / TC_KB) * TC_IMG + img_index(128, j, k % TC_KB);
                 split(h[(n == 0 ? o_k51 : o_k52) + (size_t)k * DENSE + j], k5p[ix], k5p_lo[ix]);
             }
-    for (int j = 0; j < DENSE; ++j) { fb[2 * G2 + DENSE + j] = h[o_b51 + j]; fb[2 * G2 + 2 * DENSE + j] = h[o_b52 + j]; }
+    for (int j = 0; j < DENSE; ++j) { fb[DENSE + j] = h[o_b51 + j]; fb[2 * DENSE + j] = h[o_b52 + j]; }
 
     std::vector<uint8_t> ws;
     lstm2f_pack(ws, h, o_w2, o_b2, o_u2);
@@ -1202,22 +717,18 @@ inline int tc_build(TcNet& t, const NetF32& net, const float* h, size_t o_w1, si
     e = cudaMemcpy(d + foff, fb.data(), fb.size() * 4, cudaMemcpyHostToDevice);
     if (e != cudaSuccess) { *err = cudaGetErrorString(e); return -1; }
     t.img1 = (const __half*)d;
-    t.img2 = t.img1 + n_img1;
-    t.w2p = t.img2 + n_img2;
-    t.k4p = t.w2p + n_w2p;
-    t.w2p_lo = t.k4p + n_k4p;
-    t.k4p_lo = t.w2p_lo + n_w2p;
+    t.k4p = t.img1 + n_img1;
+    t.k4p_lo = t.k4p + n_k4p;
     t.k5p = t.k4p_lo + n_k4p;
     t.k5p_lo = t.k5p + n_k5p;
-    t.b2p = (const float*)(d + foff);
-    t.b4 = t.b2p + 2 * G2;
+    t.b4 = (const float*)(d + foff);
     t.b5p = t.b4 + DENSE;
     e = cudaMalloc((void**)&t.err, 64);
     if (e != cudaSuccess) { *err = cudaGetErrorString(e); return -1; }
     cudaMemset(t.err, 0, 64);
     if (getenv("C3R_TRACE")) {
-        cudaMalloc((void**)&t.trace, (2 * 2 * NT * 8 * 8 + 64 * 32) * sizeof(long long));
-        cudaMemset(t.trace, 0, (2 * 2 * NT * 8 * 8 + 64 * 32) * sizeof(long long));
+        cudaMalloc((void**)&t.trace, 2 * 2 * NT * 8 * 8 * sizeof(long long));
+        cudaMemset(t.trace, 0, 2 * 2 * NT * 8 * 8 * sizeof(long long));
     }
     t.ready = 1;
     return 0;
@@ -1228,21 +739,20 @@ inline int tc_ensure(TcNet& t, int tiles, std::string* err) {
     if (t.abuf) cudaFree(t.abuf);
     t.abuf = nullptr;
     const size_t n_h1 = (size_t)tiles * NT * 4 * TC_IMG, n_h2 = (size_t)tiles * NT * 5 * TC_IMG;
-    const size_t n_zx = lstm2_fused() ? 64 : (size_t)tiles * NT * 10 * ZX_CHUNK_WORDS, n_l4 = (size_t)tiles * 128 * DENSE;
+    const size_t n_l4 = (size_t)tiles * 128 * DENSE;
     const size_t n_xop = (size_t)tiles * NT * 64 * TC_TILE;
-    t.abytes = (n_h1 + n_h2) * 2 * 2 + n_xop * 2 + (n_zx + n_l4 * (1 + L4_KSPLIT)) * 4 + n_l4 * 2 * 2 + n_l4 * 2 * 4 + 1024;
+    t.abytes = (n_h1 + n_h2) * 2 * 2 + n_xop * 2 + n_l4 * (1 + L4_KSPLIT) * 4 + n_l4 * 2 * 2 + n_l4 * 2 * 4 + 1024;
     cudaError_t e = cudaMalloc(&t.abuf, t.abytes);
     if (e != cudaSuccess) { *err = std::string("activation scratch: ") + cudaGetErrorString(e); t.cap_tiles = 0; return -1; }
     uint8_t* p = (uint8_t*)t.abuf;
-    t.zx2 = (float*)p; p += n_zx * 4;
     t.l4 = (float*)p; p += n_l4 * 4;
     t.l4p = (float*)p; p += n_l4 * 4 * L4_KSPLIT;
     t.l4_stride = n_l4;
     t.a5 = (float*)p; p += n_l4 * 2 * 4;
     t.l4h = (__half*)p; p += n_l4 * 2;
     t.l4h_lo = (__half*)p; p += n_l4 * 2;
-    t.h1 = (__half*)p; p += n_h1 * 2;
-    t.h1_lo = (__half*)p; p += n_h1 * 2;
+    t.h1[0] = (__half*)p; p += n_h1 * 2;
+    t.h1[1] = (__half*)p; p += n_h1 * 2;
     t.h2 = (__half*)p; p += n_h2 * 2;
     t.h2_lo = (__half*)p; p += n_h2 * 2;
     t.xop = (__half*)p;
@@ -1250,7 +760,9 @@ inline int tc_ensure(TcNet& t, int tiles, std::string* err) {
     return 0;
 }
 
-constexpr int TC_SUB_TILES = 320;            // at most 40960 sites per sub-pass: bounds the hoisted-projection scratch (7 GB)
+// at most 40960 sites per sub-pass (tc_forward rounds it down to whole rounds of the recurrent kernels): bounds the
+// activation scratch (3.4 GB) and sets how a large batch is cut into sub-passes
+constexpr int TC_SUB_TILES = 320;
 
 template <int CH, int KX>
 inline cudaError_t launch_lstm(const LstmArgs& a, int sm_count, cudaStream_t st) {
@@ -1268,29 +780,9 @@ inline cudaError_t launch_lstm(const LstmArgs& a, int sm_count, cudaStream_t st)
     return cudaGetLastError();
 }
 
-// split-precision products of the hoisted LSTM2 projection as a bit mask: 1 = A_hi*B_hi, 2 = A_lo*B_hi,
-// 4 = A_hi*B_lo.  C3R_ZX_TERMS overrides for experiments (tools/zx_terms_probe.sh).
-inline int zx_terms() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("C3R_ZX_TERMS");
-        v = e ? atoi(e) : 5;
-        if (v < 1 || v > 7 || !(v & 1)) v = 5;
-    }
-    return v;
-}
-
-inline int zx_overlap_tiles() {              // projection tile pairs per idle SM pair under LSTM1's remainder round
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("C3R_ZX_OVERLAP");
-        v = e ? atoi(e) : 7;
-        if (v < 0 || v > 64) v = 7;
-    }
-    return v;
-}
-
-inline int l4_terms() {                      // same mask for the L4 GEMM (C3R_L4_TERMS)
+// split-precision products of the L4 GEMM as a bit mask: 1 = A_hi*B_hi, 2 = A_lo*B_hi, 4 = A_hi*B_lo.
+// C3R_L4_TERMS overrides for experiments (tools/l4_terms_probe.sh).
+inline int l4_terms() {
     static int v = -1;
     if (v < 0) {
         const char* e = getenv("C3R_L4_TERMS");
@@ -1298,20 +790,6 @@ inline int l4_terms() {                      // same mask for the L4 GEMM (C3R_L
         if (v < 1 || v > 7 || !(v & 1)) v = 7;
     }
     return v;
-}
-
-inline cudaError_t launch_gemm_zx(const GemmArgs& g, int sm_count, cudaStream_t st, int max_pairs = 1 << 30) {
-    static bool attr = false;
-    if (!attr) {
-        cudaError_t e = cudaFuncSetAttribute(k_gemm_zx, cudaFuncAttributeMaxDynamicSharedMemorySize, ZXG_SMEM);
-        if (e != cudaSuccess) return e;
-        attr = true;
-    }
-    int pairs = g.m_tiles / 2 < sm_count / 2 ? g.m_tiles / 2 : sm_count / 2;
-    if (pairs > max_pairs) pairs = max_pairs;
-    if (pairs < 1) pairs = 1;
-    k_gemm_zx<<<pairs * 2, ZXG_THREADS, ZXG_SMEM, st>>>(g);
-    return cudaGetLastError();
 }
 
 inline cudaError_t launch_gemm(const GemmArgs& g, int sm_count, cudaStream_t st) {
@@ -1333,19 +811,16 @@ inline cudaError_t launch_gemm(const GemmArgs& g, int sm_count, cudaStream_t st)
 // item count is not a multiple of the 74 CTA pairs leaves SMs idle in its last round (116 items at 14.6 k sites:
 // the second round is 57 % full).  LSTM2 is therefore launched as A (the full rounds) and B (the rest), and the
 // L4 GEMM + heads of A run on a second stream while B is in flight: they are one-tile-per-CTA kernels, so they
-// simply take the SMs B leaves idle (measured: 2.205 -> 2.174 ms per forward at 14.6 k sites).  Doing the same
-// between LSTM1 and the zx GEMM was measured slower (2.26 -> 2.45 ms): that GEMM's CTA pairs stride statically
-// over the tiles, so the pairs that start late set its finish time.
+// simply take the SMs B leaves idle (measured: 2.205 -> 2.174 ms per forward at 14.6 k sites).
 struct TcPipe {
     cudaStream_t s2 = nullptr;
     cudaEvent_t ev[2] = {};
-    // Passes of different tickets run on different streams but share the scratch buffers.  A pass may start
-    // (xop, LSTM1: they write xop and h1) once the previous pass's projection GEMM has read h1; it may write zx2 /
-    // h2 / l4 once the previous pass has ended.  (An event that was never recorded does not block.)
-    cudaEvent_t h1_free = nullptr, pass_done = nullptr;
-    // Fused LSTM2: h1 is double-buffered (the second buffer is the unused low-order image), so LSTM1 of the NEXT pass
-    // can run on the SMs the last LSTM2 launch of this pass leaves idle (its remainder round: 84 of 148 SMs at config
-    // 2).  h1_free2[b]: LSTM2 has read buffer b;  xop_free: LSTM1 has read the shared operand image;
+    // Passes of different tickets run on different streams but share the scratch buffers.  A pass may write h2 / l4
+    // once the previous pass has ended (pass_done).  (An event that was never recorded does not block.)
+    cudaEvent_t pass_done = nullptr;
+    // h1 is double-buffered (TcNet::h1[2]), so LSTM1 of the NEXT pass can run on the SMs the last LSTM2 launch of
+    // this pass leaves idle (its remainder round: 84 of 148 SMs at config 2).
+    // h1_free2[b]: LSTM2 has read buffer b;  xop_free: LSTM1 has read the shared operand image;
     // last_ready / last_done: the last LSTM2 launch of the previous pass may start / has ended;  last_pairs: its tile pairs.
     cudaEvent_t h1_free2[2] = {}, xop_free = nullptr, last_ready = nullptr, last_done = nullptr;
     int last_pairs = 0, parity = 0;
@@ -1356,13 +831,9 @@ inline int tc_pipe_init(TcPipe& p, std::string* err) {
     if (p.ok) return 0;
     int prio_lo = 0, prio_hi = 0;                    // the network's streams are high priority (c3r_create)
     cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);
-    // the second stream (L4 + heads of the full rounds, beside LSTM2's remainder round) sits between the network's main
-    // stream and the integer stages: C3R_S2_PRIO = steps below the highest priority (default 0)
-    int s2p = prio_hi + (getenv("C3R_S2_PRIO") ? atoi(getenv("C3R_S2_PRIO")) : 0);
-    if (s2p > prio_lo) s2p = prio_lo;
-    cudaError_t e = cudaStreamCreateWithPriority(&p.s2, cudaStreamNonBlocking, getenv("C3R_FLAT_PRIORITY") ? prio_lo : s2p);
+    // the second stream (L4 + heads of the full rounds, beside LSTM2's remainder round) is high priority as well
+    cudaError_t e = cudaStreamCreateWithPriority(&p.s2, cudaStreamNonBlocking, getenv("C3R_FLAT_PRIORITY") ? prio_lo : prio_hi);
     for (int i = 0; i < 2 && e == cudaSuccess; ++i) e = cudaEventCreateWithFlags(&p.ev[i], cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&p.h1_free, cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&p.pass_done, cudaEventDisableTiming);
     for (cudaEvent_t* ev : {&p.h1_free2[0], &p.h1_free2[1], &p.xop_free, &p.last_ready, &p.last_done})
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(ev, cudaEventDisableTiming);
@@ -1373,33 +844,22 @@ inline int tc_pipe_init(TcPipe& p, std::string* err) {
 inline void tc_pipe_release(TcPipe* p) {
     if (p->s2) cudaStreamDestroy(p->s2);
     for (cudaEvent_t e : p->ev) if (e) cudaEventDestroy(e);
-    if (p->h1_free) cudaEventDestroy(p->h1_free);
     if (p->pass_done) cudaEventDestroy(p->pass_done);
     for (cudaEvent_t ev : {p->h1_free2[0], p->h1_free2[1], p->xop_free, p->last_ready, p->last_done}) if (ev) cudaEventDestroy(ev);
     delete p;
 }
 
-// end of the last network pass (nullptr before the first one)
-inline cudaEvent_t tc_pass_done(const TcNet& t) { return t.pipe && t.pipe->ok ? t.pipe->pass_done : nullptr; }
-
 // tiles [t0, t0 + nt) of the pass, sites [s0, s0 + ns)
 struct TcSub { int t0, nt; int64_t s0, ns; };
 
 inline cudaError_t tc_lstm2(TcNet& t, const TcSub& b, cudaStream_t st, const __half* h1buf) {
-    if (lstm2_fused()) {
-        Lstm2fArgs f;
-        f.wstream = t.wstream2; f.h1 = h1buf + (size_t)b.t0 * NT * 4 * TC_IMG;
-        f.hout = t.h2 + (size_t)b.t0 * NT * 5 * TC_IMG;
-        f.hout_lo = (l4_terms() & 2) ? t.h2_lo + (size_t)b.t0 * NT * 5 * TC_IMG : nullptr;
-        f.n_tiles = b.nt; f.err = t.err;
-        f.prof = (t.trace && b.t0 == 0) ? t.trace + 2 * NT * 8 * 8 : nullptr;   // C3R_TRACE: wait-time totals of cluster 0 (LSTM2's part of the trace buffer)
-        return launch_lstm2f(f, t.sm_count, st);
-    }
-    LstmArgs a2;
-    a2.Wimg = t.img2; a2.xop = nullptr; a2.C = t.C; a2.zx = t.zx2 + (size_t)b.t0 * NT * 10 * ZX_CHUNK_WORDS;
-    a2.hout = t.h2 + (size_t)b.t0 * NT * 5 * TC_IMG; a2.hout_lo = (l4_terms() & 2) ? t.h2_lo + (size_t)b.t0 * NT * 5 * TC_IMG : nullptr; a2.kb_out = 5;
-    a2.n_sites = b.ns; a2.n_tiles = b.nt; a2.err = t.err; a2.trace = (t.trace && b.t0 == 0) ? t.trace + 2 * NT * 8 * 8 : nullptr;
-    return launch_lstm<5, 0>(a2, t.sm_count, st);
+    Lstm2fArgs f;
+    f.wstream = t.wstream2; f.h1 = h1buf + (size_t)b.t0 * NT * 4 * TC_IMG;
+    f.hout = t.h2 + (size_t)b.t0 * NT * 5 * TC_IMG;
+    f.hout_lo = (l4_terms() & 2) ? t.h2_lo + (size_t)b.t0 * NT * 5 * TC_IMG : nullptr;
+    f.n_tiles = b.nt; f.err = t.err;
+    f.prof = (t.trace && b.t0 == 0) ? t.trace + 2 * NT * 8 * 8 : nullptr;   // C3R_TRACE: wait-time totals of cluster 0 (LSTM2's part of the trace buffer)
+    return launch_lstm2f(f, t.sm_count, st);
 }
 inline cudaError_t tc_l4_heads(TcNet& t, const NetF32& net, const TcSub& b, float* probs, cudaStream_t st) {
     GemmArgs g4;
@@ -1407,7 +867,7 @@ inline cudaError_t tc_l4_heads(TcNet& t, const NetF32& net, const TcSub& b, floa
     // K = 10560 always goes in L4_KSPLIT ranges (partial sums added up by k_l4_finish): a remainder launch of a few dozen
     // tiles still fills the SMs, and the summation order is the same whatever the batch size
     g4.terms = l4_terms(); g4.bias = t.b4; g4.out = t.l4p + (size_t)b.t0 * 128 * DENSE; g4.m_tiles = b.nt; g4.n_tiles = 1; g4.n_kb = L4_IN / TC_KB;
-    g4.mode = 1; g4.ksplit = L4_KSPLIT; g4.split_stride = t.l4_stride; g4.err = t.err; g4.dbg = 0; g4.trace = nullptr;
+    g4.ksplit = L4_KSPLIT; g4.split_stride = t.l4_stride; g4.err = t.err;
     cudaError_t e = launch_gemm(g4, t.sm_count, st);
     if (e != cudaSuccess) return e;
     // l4 = selu(sum of the partial sums + bias) as fp16 operand images; [L5_1 | L5_2] as one tensor-core GEMM
@@ -1417,7 +877,7 @@ inline cudaError_t tc_l4_heads(TcNet& t, const NetF32& net, const TcSub& b, floa
     GemmArgs g5;
     g5.A = t.l4h + (size_t)b.t0 * 2 * TC_IMG; g5.A_lo = t.l4h_lo + (size_t)b.t0 * 2 * TC_IMG; g5.B = t.k5p; g5.B_lo = t.k5p_lo;
     g5.terms = 7; g5.bias = t.b5p; g5.out = t.a5 + (size_t)b.t0 * 128 * 256; g5.m_tiles = b.nt; g5.n_tiles = 2; g5.n_kb = 2;
-    g5.mode = 1; g5.ksplit = 1; g5.split_stride = 0; g5.err = t.err; g5.dbg = 0; g5.trace = nullptr;
+    g5.ksplit = 1; g5.split_stride = 0; g5.err = t.err;
     e = launch_gemm(g5, t.sm_count, st);
     if (e != cudaSuccess) return e;
     {
@@ -1446,15 +906,12 @@ inline int tc_forward(TcNet& t, const NetF32& net, const int32_t* tensor, int64_
         int tiles = (int)((m + TC_TILE - 1) / TC_TILE);
         tiles += tiles & 1;                  // CTA pairs
         if (tc_ensure(t, tiles, err)) return -1;
-        const bool fused = lstm2_fused();
-        const int hb = fused ? P.parity : 0;                        // h1 buffer of this pass
-        if (fused) P.parity ^= 1;
-        __half* const h1buf = hb ? t.h1_lo : t.h1;
+        const int hb = P.parity;                                    // h1 buffer of this pass
+        P.parity ^= 1;
+        __half* const h1buf = t.h1[hb];
         t.h1_cur = h1buf;
-        if (fused) {
-            TCK(cudaStreamWaitEvent(st, P.h1_free2[hb], 0), "wait");   // LSTM2 of the pass before the previous one has read this buffer
-            if (!xop_ready) TCK(cudaStreamWaitEvent(st, P.xop_free, 0), "wait");   // LSTM1 of the previous pass has read the shared image
-        } else TCK(cudaStreamWaitEvent(st, P.h1_free, 0), "wait");  // the previous pass no longer reads xop / h1
+        TCK(cudaStreamWaitEvent(st, P.h1_free2[hb], 0), "wait");   // LSTM2 of the pass before the previous one has read this buffer
+        if (!xop_ready) TCK(cudaStreamWaitEvent(st, P.xop_free, 0), "wait");   // LSTM1 of the previous pass has read the shared image
         const int kx_ = t.C == 18 ? 48 : 64;
         const __half* xop_in = t.xop;
         if (xop_ready) xop_in = xop_ready + (size_t)(o / TC_TILE) * NT * (size_t)(kx_ * TC_TILE);
@@ -1464,9 +921,9 @@ inline int tc_forward(TcNet& t, const NetF32& net, const int32_t* tensor, int64_
             ++launches;
         }
         // A = the tile pairs that fill whole rounds of the recurrent kernels, B = the rest
-        // tile pairs one round of the LSTM2 kernel takes (fused: clusters of 2*NP CTAs, half of them per direction)
+        // tile pairs one round of the LSTM2 kernel takes (clusters of 2*NP CTAs, half of them per direction)
         const int pairs = tiles / 2;
-        const int per_round = lstm2_fused() ? (t.sm_count / (2 * lstm2f_np()) / 2) * lstm2f_np() : t.sm_count / 4;
+        const int per_round = (t.sm_count / (2 * lstm2f_np()) / 2) * lstm2f_np();
         int pa = pairs;
         if (pairs > per_round && pairs % per_round != 0) pa = (pairs / per_round) * per_round;
         TcSub A, B;
@@ -1475,112 +932,69 @@ inline int tc_forward(TcNet& t, const NetF32& net, const int32_t* tensor, int64_
         auto lstm1 = [&](const TcSub& b, cudaStream_t s) -> cudaError_t {
             LstmArgs a1;
             const int kx = t.C == 18 ? 48 : 64;
-            a1.Wimg = t.img1; a1.xop = xop_in + (size_t)b.t0 * NT * kx * TC_TILE; a1.C = t.C; a1.zx = nullptr;
+            a1.Wimg = t.img1; a1.xop = xop_in + (size_t)b.t0 * NT * kx * TC_TILE;
             a1.hout = h1buf + (size_t)b.t0 * NT * 4 * TC_IMG;
-            a1.hout_lo = (!fused && (zx_terms() & 2)) ? t.h1_lo + (size_t)b.t0 * NT * 4 * TC_IMG : nullptr; a1.kb_out = 4;
             a1.n_sites = b.ns; a1.n_tiles = b.nt; a1.err = t.err; a1.trace = b.t0 == 0 ? t.trace : nullptr;
             return t.C == 18 ? launch_lstm<4, 48>(a1, t.sm_count, s) : launch_lstm<4, 64>(a1, t.sm_count, s);
         };
-        // hoisted LSTM2 projection of the 128-row tiles [m0, m0 + mt) (tile = site tile * 33 + time step)
-        auto zx = [&](int m0, int mt, int max_pairs, cudaStream_t s) -> cudaError_t {
-            GemmArgs g2;
-            g2.A = t.h1 + (size_t)m0 * ZXG_KB * TC_IMG; g2.A_lo = t.h1_lo + (size_t)m0 * ZXG_KB * TC_IMG;
-            g2.B = t.w2p; g2.B_lo = t.w2p_lo; g2.terms = zx_terms(); g2.bias = t.b2p;
-            g2.out = t.zx2 + (size_t)m0 * 10 * ZX_CHUNK_WORDS;
-            g2.m_tiles = mt; g2.n_tiles = 5; g2.n_kb = 4;
-            g2.mode = 0; g2.ksplit = 1; g2.split_stride = 0; g2.err = t.err; g2.dbg = getenv("C3R_ZX_DBG") ? atoi(getenv("C3R_ZX_DBG")) : 0;
-            g2.trace = (t.trace && m0 == 0) ? t.trace + 2 * 2 * NT * 8 * 8 : nullptr;
-            return launch_gemm_zx(g2, t.sm_count, s, max_pairs);
+        // The last LSTM2 launch of the pass before this one (its remainder round, or its only round) leaves
+        // sm_count - 4 x pairs SMs idle: while it is still ahead of us, LSTM1 of THIS pass goes in pieces that fit
+        // beside it - two pieces (an LSTM1 round takes less than half an LSTM2 round), then the rest once it has
+        // ended.  At config 2 (37 + 21 tile pairs): 16 + 16 pairs of LSTM1 run under the previous pass's
+        // remainder round and the remaining 26 are ONE round instead of two; a 5 Mb chunk of config 5 (20 pairs,
+        // one partly filled round) puts all of its LSTM1 beside the previous chunk's LSTM2.
+        const int ip = (t.sm_count - 4 * P.last_pairs) / 4;         // tile pairs (both directions) that fit beside it
+        bool overlap = o == 0 && P.last_pairs > 0 && ip >= 8 && getenv("C3R_NO_LSTM1_OVERLAP") == nullptr;
+        if (overlap) {
+            overlap = cudaEventQuery(P.last_done) == cudaErrorNotReady;
+            (void)cudaGetLastError();
+        }
+        auto piece = [&](int p0, int np) {
+            TcSub b; b.t0 = 2 * p0; b.nt = 2 * np; b.s0 = (int64_t)b.t0 * TC_TILE;
+            const int64_t left = m - b.s0;
+            b.ns = left < 0 ? 0 : left < (int64_t)b.nt * TC_TILE ? left : (int64_t)b.nt * TC_TILE;
+            return b;
         };
-        // While LSTM1's remainder round leaves SMs idle, the projection of the first tiles of A runs on them
-        // (second stream); each idle SM pair gets as many tile pairs as fit in the remainder round's ~190 us.
-        const int busy_b = 4 * (B.nt / 2 < per_round ? B.nt / 2 : per_round);
-        const int idle_pairs = (t.sm_count - busy_b) / 2;
-        int m_early = 2 * idle_pairs * zx_overlap_tiles();
-        if (m_early > A.nt * NT) m_early = A.nt * NT;
-        if (fused) {                                                // no projection GEMM: LSTM2 reads h1 itself
-            // The last LSTM2 launch of the pass before this one (its remainder round, or its only round) leaves
-            // sm_count - 4 x pairs SMs idle: while it is still ahead of us, LSTM1 of THIS pass goes in pieces that fit
-            // beside it - two pieces (an LSTM1 round takes less than half an LSTM2 round), then the rest once it has
-            // ended.  At config 2 (37 + 21 tile pairs): 16 + 16 pairs of LSTM1 run under the previous pass's
-            // remainder round and the remaining 26 are ONE round instead of two; a 5 Mb chunk of config 5 (20 pairs,
-            // one partly filled round) puts all of its LSTM1 beside the previous chunk's LSTM2.
-            const int ip = (t.sm_count - 4 * P.last_pairs) / 4;     // tile pairs (both directions) that fit beside it
-            bool overlap = o == 0 && P.last_pairs > 0 && ip >= 8 && getenv("C3R_NO_LSTM1_OVERLAP") == nullptr;
-            if (overlap) {
-                overlap = cudaEventQuery(P.last_done) == cudaErrorNotReady;
-                (void)cudaGetLastError();
+        ++P.n_pass;
+        if (overlap) {
+            ++P.n_overlap;
+            TCK(cudaStreamWaitEvent(st, P.last_ready, 0), "wait");
+            int done = 0;
+            for (int c = 0; c < 2 && done < pairs; ++c) {
+                const int np = pairs - done < ip ? pairs - done : ip;
+                TCK(lstm1(piece(done, np), st), "lstm1");
+                done += np; ++launches;
             }
-            auto piece = [&](int p0, int np) {
-                TcSub b; b.t0 = 2 * p0; b.nt = 2 * np; b.s0 = (int64_t)b.t0 * TC_TILE;
-                const int64_t left = m - b.s0;
-                b.ns = left < 0 ? 0 : left < (int64_t)b.nt * TC_TILE ? left : (int64_t)b.nt * TC_TILE;
-                return b;
-            };
-            ++P.n_pass;
-            if (overlap) {
-                ++P.n_overlap;
-                TCK(cudaStreamWaitEvent(st, P.last_ready, 0), "wait");
-                int done = 0;
-                for (int c = 0; c < 2 && done < pairs; ++c) {
-                    const int np = pairs - done < ip ? pairs - done : ip;
-                    TCK(lstm1(piece(done, np), st), "lstm1");
-                    done += np; ++launches;
-                }
-                if (done < pairs) {
-                    TCK(cudaStreamWaitEvent(st, P.last_done, 0), "wait");
-                    TCK(lstm1(piece(done, pairs - done), st), "lstm1");
-                } else --launches;                                      // (the common count below adds one)
-            } else {
-                TcSub all; all.t0 = 0; all.nt = tiles; all.s0 = 0; all.ns = m;
-                TCK(lstm1(all, st), "lstm1");
-            }
-            TCK(cudaEventRecord(P.xop_free, st), "event");
-            TCK(cudaStreamWaitEvent(st, P.pass_done, 0), "wait");   // the previous pass no longer reads h2 / l4
-            ++launches;
-        } else if (B.nt == 0 || A.nt == 0 || idle_pairs < 8 || m_early <= 0) {
+            if (done < pairs) {
+                TCK(cudaStreamWaitEvent(st, P.last_done, 0), "wait");
+                TCK(lstm1(piece(done, pairs - done), st), "lstm1");
+            } else --launches;                                          // (the common count below adds one)
+        } else {
             TcSub all; all.t0 = 0; all.nt = tiles; all.s0 = 0; all.ns = m;
             TCK(lstm1(all, st), "lstm1");
-            TCK(cudaStreamWaitEvent(st, P.pass_done, 0), "wait");   // the previous pass no longer reads zx2 / h2 / l4
-            TCK(zx(0, tiles * NT, 1 << 30, st), "zx2 gemm");
-            launches += 2;
-        } else {
-            TCK(lstm1(A, st), "lstm1");
-            TCK(cudaEventRecord(P.ev[0], st), "event");
-            TCK(lstm1(B, st), "lstm1");
-            TCK(cudaStreamWaitEvent(P.s2, P.ev[0], 0), "wait");
-            TCK(cudaStreamWaitEvent(P.s2, P.pass_done, 0), "wait");
-            TCK(zx(0, m_early, idle_pairs, P.s2), "zx2 gemm");
-            TCK(cudaEventRecord(P.ev[1], P.s2), "event");
-            TCK(cudaStreamWaitEvent(st, P.ev[1], 0), "wait");
-            TCK(cudaStreamWaitEvent(st, P.pass_done, 0), "wait");
-            TCK(zx(m_early, tiles * NT - m_early, 1 << 30, st), "zx2 gemm");
-            launches += 4;
         }
-        if (!fused) { TCK(cudaEventRecord(P.h1_free, st), "event"); P.last_pairs = 0; }
+        TCK(cudaEventRecord(P.xop_free, st), "event");
+        TCK(cudaStreamWaitEvent(st, P.pass_done, 0), "wait");       // the previous pass no longer reads h2 / l4
+        ++launches;
         float* pr = probs + o * 24;
-        if (fused && B.nt == 0) TCK(cudaEventRecord(P.last_ready, st), "event");
+        if (B.nt == 0) TCK(cudaEventRecord(P.last_ready, st), "event");
         TCK(tc_lstm2(t, A, st, h1buf), "lstm2");
         ++launches;
         if (B.nt == 0) {
-            if (fused) {
-                TCK(cudaEventRecord(P.last_done, st), "event");
-                TCK(cudaEventRecord(P.h1_free2[hb], st), "event");
-                P.last_pairs = pa;
-            }
+            TCK(cudaEventRecord(P.last_done, st), "event");
+            TCK(cudaEventRecord(P.h1_free2[hb], st), "event");
+            P.last_pairs = pa;
             TCK(tc_l4_heads(t, net, A, pr, st), "l4/heads");
             launches += 4;
             TCK(cudaEventRecord(P.pass_done, st), "event");
             continue;
         }
         TCK(cudaEventRecord(P.ev[0], st), "event");
-        if (fused) TCK(cudaEventRecord(P.last_ready, st), "event");
+        TCK(cudaEventRecord(P.last_ready, st), "event");
         TCK(tc_lstm2(t, B, st, h1buf), "lstm2");
-        if (fused) {
-            TCK(cudaEventRecord(P.last_done, st), "event");
-            TCK(cudaEventRecord(P.h1_free2[hb], st), "event");
-            P.last_pairs = B.nt / 2;
-        }
+        TCK(cudaEventRecord(P.last_done, st), "event");
+        TCK(cudaEventRecord(P.h1_free2[hb], st), "event");
+        P.last_pairs = B.nt / 2;
         TCK(cudaStreamWaitEvent(P.s2, P.ev[0], 0), "wait");
         TCK(tc_l4_heads(t, net, A, pr, P.s2), "l4/heads");
         TCK(cudaEventRecord(P.ev[1], P.s2), "event");

@@ -213,12 +213,11 @@ class Engine:
 
     def debug_fetch(self, which: int, n_sites: int):
         """intermediate activations of the last tensor-core forward, unpacked to plain arrays:
-        0 -> h1 [n,33,256], 1 -> zx2 [n,33,2,640] (Keras gate columns), 2 -> h2 [n,33,320], 3 -> l4 [n,128]"""
+        0 -> h1 [n,33,256], 2 -> h2 [n,33,320], 3 -> l4 [n,128]"""
         tiles = (n_sites + 127) // 128
         tiles += tiles & 1
-        sizes = {0: tiles * 33 * 4 * 8192 * 2, 1: tiles * 33 * 10 * 32 * 3 * 128 * 4, 2: tiles * 33 * 5 * 8192 * 2,
-                 3: tiles * 128 * 128 * 4}
-        buf = np.empty(sizes[which], np.uint8)
+        sizes = {0: tiles * 33 * 4 * 8192 * 2, 2: tiles * 33 * 5 * 8192 * 2, 3: tiles * 128 * 128 * 4}
+        buf = np.empty(sizes.get(which, 0), np.uint8)              # other numbers: the library refuses them (C3RError)
         nb = C.c_int64(0)
         self._check(self.lib.c3r_debug_fetch(self.ctx, which, buf.ctypes.data, buf.size, C.byref(nb)), "c3r_debug_fetch")
         if which in (0, 2):
@@ -226,16 +225,6 @@ class Engine:
             a = buf.view(np.float16).reshape(tiles, 33, kb, 8, 128, 8)        # [tile][t][kb][k8][row][8]
             a = a.transpose(0, 4, 1, 2, 3, 5).reshape(tiles * 128, 33, kb * 64)
             return a[:n_sites].astype(np.float32)
-        if which == 1:
-            w = buf.view(np.uint32).reshape(tiles, 33, 2, 5, 4, 8, 3, 128)    # [tile][t][dir][chunk][gate][ug][plane][row]
-            w0, w1, w2 = w[..., 0, :], w[..., 1, :], w[..., 2, :]
-            # 24-bit floats: w0 = hi16(a) | hi16(b) << 16, w1 = hi16(c) | hi16(d) << 16, w2 = the four low bytes
-            vals = [((w0 & 0xffff) << 16) | ((w2 & 0xff) << 8), (w0 & 0xffff0000) | (((w2 >> 8) & 0xff) << 8),
-                    ((w1 & 0xffff) << 16) | (((w2 >> 16) & 0xff) << 8), (w1 & 0xffff0000) | (((w2 >> 24) & 0xff) << 8)]
-            a = np.stack(vals, axis=-1).astype(np.uint32).view(np.float32).copy()
-            a[:, :, :, :, [0, 1, 3]] *= 2.0                                   # i, f, o columns are stored as 0.5 * z
-            a = a.transpose(0, 6, 1, 2, 4, 3, 5, 7).reshape(tiles * 128, 33, 2, 4 * 160)   # gate, chunk*32 + ug*4 + i
-            return a[:n_sites]
         return buf.view(np.float32).reshape(tiles * 128, 128)[:n_sites]
 
 

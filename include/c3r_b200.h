@@ -186,8 +186,8 @@ int c3r_rerun_resident(c3r_ctx* ctx, c3r_ticket ticket, float* total_ms, float* 
 int c3r_forward(c3r_ctx* ctx, const int32_t* tensor, int64_t n, float* probs, float* device_ms);
 
 /* Diagnostics: copy an intermediate activation buffer of the last tensor-core forward to the
- * host (which: 0 = LSTM1 output, packed fp16; 1 = LSTM2 input projection, fp32 ZX layout;
- * 2 = LSTM2 output, packed fp16; 3 = L4 output, fp32 [sites,128]).  Layouts in csrc/nn_tc.cuh. */
+ * host (which: 0 = LSTM1 output, packed fp16; 2 = LSTM2 output, packed fp16; 3 = L4 output,
+ * fp32 [sites,128]).  Layouts in csrc/nn_tc.cuh. */
 int c3r_debug_fetch(c3r_ctx* ctx, int which, void* dst, int64_t max_bytes, int64_t* n_bytes);
 
 /* Page-locked host memory for the arrays handed to c3r_submit_chunk (read by DMA while the call has long returned;

@@ -1,12 +1,12 @@
 """Fused-LSTM2 probe: numerics against the oracle (h2 and probabilities) and forward time at a bench-sized batch.
-Usage: [C3R_LSTM2=hoisted] [C3R_LSTM2F_NP=1|2|4] python tools/lstm2f_probe.py [n_sites] [out.npy]"""
+Usage: [C3R_LSTM2F_NP=1|2|4] python tools/lstm2f_probe.py [n_sites] [out.npy]"""
 import os, sys, time, numpy as np
 sys.path.insert(0, os.getcwd())
 from clair3_rna_b200 import weights
 from clair3_rna_b200.engine import Engine
 from oracle import model
 n_big = int(sys.argv[1]) if len(sys.argv) > 1 else 14617
-tag = "LSTM2=%s NP=%s" % (os.environ.get("C3R_LSTM2", "fused"), os.environ.get("C3R_LSTM2F_NP", "-"))
+tag = "NP=%s" % os.environ.get("C3R_LSTM2F_NP", "-")
 g = np.load("tests/golden/cfg1_ont_drna.npz")
 x = g["tensor"][:300]
 w = weights.synthetic(18, sharpen=8.0)
@@ -25,7 +25,7 @@ k = len(g["tensor"])
 print(tag, "batch-position invariance:", bool(np.array_equal(pb[:k], pb[k:2 * k])) if n_big >= 2 * k else "n/a", flush=True)
 if os.environ.get("C3R_TRACE"):
     import ctypes as C
-    buf = np.zeros(2 * 2 * 33 * 8 * 8 + 64 * 32, np.int64); nb = C.c_int64(0)
+    buf = np.zeros(2 * 2 * 33 * 8 * 8, np.int64); nb = C.c_int64(0)
     eng.lib.c3r_debug_fetch(eng.ctx, 4, buf.ctypes.data, buf.nbytes, C.byref(nb))
     buf = buf[2 * 33 * 8 * 8:]
     names = ["acc_empty", "acc_empty_peer", "x", "h_ready", "w_full", "w_peer_full", "total", "steps", "producer_wait_empty", "gate0_wait_acc"]
