@@ -247,7 +247,7 @@ int ensure_stage_b(c3r_ctx* ctx, Slot& s) {
     s.fused_window = ctx->prm.nn_impl == 1 && !ctx->prm.keep_tensor && !d.padding && getenv("C3R_NO_FUSED_WINDOW") == nullptr;
     if (s.fused_window) {
         const size_t tiles = (size_t)((n + 255) / 256) * 2;
-        if (ensure(ctx, s.xop, tiles * WIN * (size_t)((d.C == 18 ? 48 : 64) * 128) * 2)) return C3R_ERR_CUDA;
+        if (ensure(ctx, s.xop, tiles * WIN * (size_t)(lstm1_kx(d.C) * 128) * 2)) return C3R_ERR_CUDA;
     } else if (ensure(ctx, s.tensor, (size_t)n * per * 4)) return C3R_ERR_CUDA;
     if (ensure(ctx, s.alt_off, (size_t)(n + 1) * 8)) return C3R_ERR_CUDA;
     if (ensure(ctx, s.alt_n, (size_t)n * 4)) return C3R_ERR_CUDA;
@@ -275,8 +275,8 @@ int run_stage_b(c3r_ctx* ctx, Slot& s) {
         if (s.fused_window) {
             const int64_t wb = ((n + 255) / 256) * 2 * WIN;                // (tile, window row) blocks
             const unsigned gx = (unsigned)(wb < (int64_t)ctx->sm_count * 32 ? wb : (int64_t)ctx->sm_count * 32);
-            if (d.C == 18) k_window_xop<18, 48><<<gx, 128, 0, st>>>(d, P<__half>(s.xop));
-            else k_window_xop<30, 64><<<gx, 128, 0, st>>>(d, P<__half>(s.xop));
+            if (d.C == 18) k_window_xop<18, lstm1_kx(18)><<<gx, 128, 0, st>>>(d, P<__half>(s.xop));
+            else k_window_xop<30, lstm1_kx(30)><<<gx, 128, 0, st>>>(d, P<__half>(s.xop));
         } else k_window<<<grid, 128, 0, st>>>(d, d.padding ? 0 : 1);
         ++L;
         if (d.padding) {

@@ -1,8 +1,8 @@
 // Pileup network forward on the 5th-gen tensor cores ("nn_impl = 1").
 //
 //   fp16 operands, fp32 accumulation in TMEM, fp32 gate math and cell state.
-//   LSTM1's input kernel is split W = W_hi + W_lo (two fp16 terms) because its operand is
-//   raw read counts (|x| up to hundreds), everything else is single fp16.
+//   LSTM1's input kernel is split W = W_hi + W_lo (two fp16 terms) and so is its operand, raw read counts
+//   x = x_hi + x_lo (|x| up to 8000; fp16 holds integers exactly only up to 2048); everything else is single fp16.
 //
 // Kernels
 //   k_gemm_tc   tcgen05 GEMM, cta_group::1, 128x128 tiles, bulk-async-copy (TMA unit) operand
@@ -34,6 +34,10 @@ namespace c3r {
 constexpr int TC_TILE = 128;                 // sites per CTA tile
 constexpr int TC_KB = 64;                    // K per pipeline stage
 constexpr int TC_IMG = TC_TILE * TC_KB;      // halfs in one 128x64 operand image (16 KB)
+// K of LSTM1's input part for C channels: [x_hi | x_hi | x_lo | 1 | 1] rounded up to whole k16 MMA steps
+// (C = 18: 56 -> 64, C = 30: 92 -> 96)
+constexpr int lstm1_kx(int C) { return (3 * C + 2 + 15) / 16 * 16; }
+constexpr int LSTM1_KX_MAX = lstm1_kx(30);
 
 // ================================================================== GEMM
 // The GEMM runs the split-precision product  A_hi*B_hi + A_lo*B_hi + A_hi*B_lo  (A = A_hi + A_lo and
@@ -182,8 +186,8 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) k_gemm_tc(GemmArgs g) {
 // ================================================================== LSTM1
 // One CTA pair (cluster of 2, tcgen05 cta_group::2) = 256 sites x one direction.
 //   CH      gate-column chunks per step; a chunk = 32 units x 4 gates = 128 accumulator columns
-//   KX      K of the input part fused into the step MMA ([x | x | 1 | 1 | 0..] against
-//           [W_hi ; W_lo ; b_hi ; b_lo ; 0])
+//   KX      K of the input part fused into the step MMA ([x_hi | x_hi | x_lo | 1 | 1 | 0..] against
+//           [W_hi ; W_lo ; W_hi ; b_hi ; b_lo ; 0], lstm1_kx)
 //   U       units (K of the recurrent part) = CH*32
 template <int CH, int KX>
 struct LstmCfg {
@@ -194,6 +198,7 @@ struct LstmCfg {
     static constexpr int AX_BYTES = TC_TILE * KX * 2;       // x operand, one buffer
     static constexpr int BAR_OFF = B_BYTES + 2 * AH_BYTES + 2 * AX_BYTES;
     static constexpr int SMEM = BAR_OFF + 256;
+    static_assert(SMEM <= 232448, "LSTM1 operands exceed the shared memory of a CTA");
     static constexpr int TMEM_COLS = 512;                   // 2 accumulator slots (256) + cell state (U <= 160)
     static constexpr int C_COL = 256;
 };
@@ -494,10 +499,17 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(LSTM_THREADS, 1) k_l
 }
 
 // int32 windows [n][33][C] -> LSTM1 x operand images [tile][33][KX/8][128 rows][8 halfs]:
-//   k < C: x, C <= k < 2C: x again (meets W_lo), k = 2C, 2C+1: 1 (meets b_hi, b_lo), rest 0.
+//   k < C: x_hi, C <= k < 2C: x_hi again (meets W_lo), 2C <= k < 3C: x_lo (meets W_hi), k = 3C, 3C+1: 1 (meets
+//   b_hi, b_lo), rest 0.  x_hi = fp16(x), x_lo = x - x_hi: exact for |x| <= 8000 (|x_lo| <= 2), so counts above 2048,
+//   which fp16 cannot hold, reach the MMA unrounded (x_pack_hi_lo).
 // Block = one (tile, t), thread = one site; each k-group is one coalesced 2 KB store.
+__device__ __forceinline__ void x_pack_hi_lo(int32_t v, __half& hi, __half& lo) {
+    hi = __float2half((float)v);
+    lo = __float2half((float)v - __half2float(hi));
+}
 template <int C, int KX>
 __global__ void __launch_bounds__(TC_TILE) k_xop(const int32_t* __restrict__ tensor, __half* __restrict__ xop, int64_t n_sites) {
+    static_assert(KX >= 3 * C + 2 && KX % 16 == 0, "x_hi | x_hi | x_lo | 1 | 1 must fit the input part");
     const int tile = blockIdx.x / NT, t = blockIdx.x % NT, r = threadIdx.x;
     const int64_t site = (int64_t)tile * TC_TILE + r;
     __align__(16) __half hv[KX];
@@ -508,12 +520,14 @@ __global__ void __launch_bounds__(TC_TILE) k_xop(const int32_t* __restrict__ ten
 #pragma unroll
         for (int j = 0; j < C / 2; ++j) {
             const int2 v = src[j];
-            hv[2 * j] = hv[C + 2 * j] = __float2half((float)v.x);
-            hv[2 * j + 1] = hv[C + 2 * j + 1] = __float2half((float)v.y);
+            x_pack_hi_lo(v.x, hv[2 * j], hv[2 * C + 2 * j]);
+            x_pack_hi_lo(v.y, hv[2 * j + 1], hv[2 * C + 2 * j + 1]);
+            hv[C + 2 * j] = hv[2 * j];
+            hv[C + 2 * j + 1] = hv[2 * j + 1];
         }
     }
-    hv[2 * C] = __float2half(1.0f);
-    hv[2 * C + 1] = __float2half(1.0f);
+    hv[3 * C] = __float2half(1.0f);
+    hv[3 * C + 1] = __float2half(1.0f);
     __half* dst = xop + ((size_t)tile * NT + t) * (size_t)(KX * TC_TILE) + r * 8;
 #pragma unroll
     for (int k8 = 0; k8 < KX / 8; ++k8) *(uint4*)(dst + (size_t)k8 * (TC_TILE * 8)) = *(const uint4*)(&hv[k8 * 8]);
@@ -598,7 +612,7 @@ constexpr int L4_KSPLIT = 3;                 // L4's K = 165 k blocks goes in 3 
 
 struct TcNet {
     int ready = 0;
-    int C = 18, KX = 48, sm_count = 148;
+    int C = 18, KX = lstm1_kx(18), sm_count = 148;
     void* wbuf = nullptr;          // all fp16 images + fp32 biases
     size_t wbytes = 0;
     const __half *img1 = nullptr, *k4p = nullptr, *k4p_lo = nullptr;
@@ -642,7 +656,7 @@ inline int tc_build(TcNet& t, const NetF32& net, const float* h, size_t o_w1, si
     tc_release(t);
     const int C = net.C;
     t.C = C;
-    t.KX = C == 18 ? 48 : 64;
+    t.KX = lstm1_kx(C);
     t.sm_count = sm_count;
     const int KX = t.KX;
     const int KT1 = KX + U1;
@@ -671,15 +685,15 @@ inline int tc_build(TcNet& t, const NetF32& net, const float* h, size_t o_w1, si
                     const float gs = gate == 2 ? 1.0f : 0.5f;                   // i, f, o columns hold 0.5 * z (see the gate math)
                     for (int k = 0; k < KT1; ++k) {
                         __half v = __float2half(0.0f);
-                        if (k < C || (k >= C && k < 2 * C)) {
-                            const int ch = k < C ? k : k - C;
+                        if (k < 3 * C) {                // [W_hi ; W_lo ; W_hi] against [x_hi | x_hi | x_lo]
+                            const int ch = k % C;
                             __half hi, lo;
                             split(gs * h[o_w1 + (size_t)ch * 2 * G1 + dir * G1 + kc], hi, lo);
-                            v = k < C ? hi : lo;
-                        } else if (k == 2 * C || k == 2 * C + 1) {
+                            v = k >= C && k < 2 * C ? lo : hi;
+                        } else if (k == 3 * C || k == 3 * C + 1) {
                             __half hi, lo;
                             split(gs * h[o_b1 + dir * G1 + kc], hi, lo);
-                            v = k == 2 * C ? hi : lo;
+                            v = k == 3 * C ? hi : lo;
                         } else if (k >= KX) {
                             v = __float2half(gs * h[o_u1 + (size_t)dir * U1 * G1 + (size_t)(k - KX) * G1 + kc]);
                         }
@@ -740,7 +754,7 @@ inline int tc_ensure(TcNet& t, int tiles, std::string* err) {
     t.abuf = nullptr;
     const size_t n_h1 = (size_t)tiles * NT * 4 * TC_IMG, n_h2 = (size_t)tiles * NT * 5 * TC_IMG;
     const size_t n_l4 = (size_t)tiles * 128 * DENSE;
-    const size_t n_xop = (size_t)tiles * NT * 64 * TC_TILE;
+    const size_t n_xop = (size_t)tiles * NT * LSTM1_KX_MAX * TC_TILE;
     t.abytes = (n_h1 + n_h2) * 2 * 2 + n_xop * 2 + n_l4 * (1 + L4_KSPLIT) * 4 + n_l4 * 2 * 2 + n_l4 * 2 * 4 + 1024;
     cudaError_t e = cudaMalloc(&t.abuf, t.abytes);
     if (e != cudaSuccess) { *err = std::string("activation scratch: ") + cudaGetErrorString(e); t.cap_tiles = 0; return -1; }
@@ -912,12 +926,11 @@ inline int tc_forward(TcNet& t, const NetF32& net, const int32_t* tensor, int64_
         t.h1_cur = h1buf;
         TCK(cudaStreamWaitEvent(st, P.h1_free2[hb], 0), "wait");   // LSTM2 of the pass before the previous one has read this buffer
         if (!xop_ready) TCK(cudaStreamWaitEvent(st, P.xop_free, 0), "wait");   // LSTM1 of the previous pass has read the shared image
-        const int kx_ = t.C == 18 ? 48 : 64;
         const __half* xop_in = t.xop;
-        if (xop_ready) xop_in = xop_ready + (size_t)(o / TC_TILE) * NT * (size_t)(kx_ * TC_TILE);
+        if (xop_ready) xop_in = xop_ready + (size_t)(o / TC_TILE) * NT * (size_t)(t.KX * TC_TILE);
         else {
-            if (t.C == 18) k_xop<18, 48><<<tiles * NT, TC_TILE, 0, st>>>(tensor + o * NT * t.C, t.xop, m);
-            else k_xop<30, 64><<<tiles * NT, TC_TILE, 0, st>>>(tensor + o * NT * t.C, t.xop, m);
+            if (t.C == 18) k_xop<18, lstm1_kx(18)><<<tiles * NT, TC_TILE, 0, st>>>(tensor + o * NT * t.C, t.xop, m);
+            else k_xop<30, lstm1_kx(30)><<<tiles * NT, TC_TILE, 0, st>>>(tensor + o * NT * t.C, t.xop, m);
             ++launches;
         }
         // A = the tile pairs that fill whole rounds of the recurrent kernels, B = the rest
@@ -931,11 +944,10 @@ inline int tc_forward(TcNet& t, const NetF32& net, const int32_t* tensor, int64_
         B.t0 = A.nt; B.nt = tiles - A.nt; B.s0 = A.ns; B.ns = m - A.ns;
         auto lstm1 = [&](const TcSub& b, cudaStream_t s) -> cudaError_t {
             LstmArgs a1;
-            const int kx = t.C == 18 ? 48 : 64;
-            a1.Wimg = t.img1; a1.xop = xop_in + (size_t)b.t0 * NT * kx * TC_TILE;
+            a1.Wimg = t.img1; a1.xop = xop_in + (size_t)b.t0 * NT * t.KX * TC_TILE;
             a1.hout = h1buf + (size_t)b.t0 * NT * 4 * TC_IMG;
             a1.n_sites = b.ns; a1.n_tiles = b.nt; a1.err = t.err; a1.trace = b.t0 == 0 ? t.trace : nullptr;
-            return t.C == 18 ? launch_lstm<4, 48>(a1, t.sm_count, s) : launch_lstm<4, 64>(a1, t.sm_count, s);
+            return t.C == 18 ? launch_lstm<4, lstm1_kx(18)>(a1, t.sm_count, s) : launch_lstm<4, lstm1_kx(30)>(a1, t.sm_count, s);
         };
         // The last LSTM2 launch of the pass before this one (its remainder round, or its only round) leaves
         // sm_count - 4 x pairs SMs idle: while it is still ahead of us, LSTM1 of THIS pass goes in pieces that fit

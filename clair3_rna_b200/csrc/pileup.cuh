@@ -1438,8 +1438,8 @@ __global__ void k_window(Dev d, int apply_scale) {
     }
 }
 // K4 fused with the network's input stage: the window goes straight into LSTM1's fp16 operand images
-//   xop[tile][33][KX/8][128 rows][8 halfs]   (k < C: x, C <= k < 2C: x again - it meets W_lo -, k = 2C, 2C+1: 1 - they
-//   meet the bias rows -, rest 0; nn_tc.cuh)
+//   xop[tile][33][KX/8][128 rows][8 halfs]   (k < C: x_hi = fp16(x), C <= k < 2C: x_hi again - it meets W_lo -,
+//   2C <= k < 3C: x_lo = x - x_hi, k = 3C, 3C+1: 1 - they meet the bias rows -, rest 0; nn_tc.cuh, k_xop)
 // instead of int32 tensor[n][33][C] that k_xop would read back: no 2.4 KB per site round trip through HBM.  Used
 // when nobody asks for the tensor itself (keep_tensor) and no padding pass has to patch it.
 // Block = (tile of 128 sites, window row t), thread = site: a thread reads the C counts of ITS row (72 / 120 contiguous
@@ -1447,6 +1447,7 @@ __global__ void k_window(Dev d, int apply_scale) {
 // every store instruction of a warp is 512 contiguous bytes.  Sites beyond n (the tile pair's padding) are zero rows.
 template <int C, int KX>
 __global__ void __launch_bounds__(128) k_window_xop(Dev d, __half* __restrict__ xop) {
+    static_assert(KX >= 3 * C + 2 && KX % 16 == 0, "x_hi | x_hi | x_lo | 1 | 1 must fit the input part");
     const int64_t n = *d.n_cand < d.cand_cap ? *d.n_cand : d.cand_cap;
     const int64_t n_tiles = ((n + 255) / 256) * 2;             // tiles come in pairs
     const int r = threadIdx.x;
@@ -1479,19 +1480,22 @@ __global__ void __launch_bounds__(128) k_window_xop(Dev d, __half* __restrict__ 
                 for (int c = 0; c < C; ++c) x[c] = (float)v[c];
             }
         }
+        __half xh[C], xl[C];                                   // x = xh + xl exactly (|x| <= 8000)
+#pragma unroll
+        for (int c = 0; c < C; ++c) {
+            xh[c] = __float2half(x[c]);
+            xl[c] = __float2half(x[c] - __half2float(xh[c]));
+        }
         __half* base = xop + ((size_t)tile * WIN + t) * (size_t)(KX * 128) + r * 8;
 #pragma unroll
         for (int k8 = 0; k8 < KX / 8; ++k8) {
-            __align__(16) __half2 hv[4];
+            __align__(16) __half hv[8];
 #pragma unroll
-            for (int j = 0; j < 4; ++j) {
-                float f[2];
-#pragma unroll
-                for (int e = 0; e < 2; ++e) {
-                    const int k = k8 * 8 + 2 * j + e;          // compile-time after unrolling
-                    f[e] = k < C ? x[k < C ? k : 0] : k < 2 * C ? x[k < 2 * C && k >= C ? k - C : 0] : k < 2 * C + 2 ? 1.0f : 0.0f;
-                }
-                hv[j] = __floats2half2_rn(f[0], f[1]);
+            for (int j = 0; j < 8; ++j) {
+                const int k = k8 * 8 + j;                      // compile-time after unrolling
+                hv[j] = k < C ? xh[k < C ? k : 0] : k < 2 * C ? xh[k < 2 * C && k >= C ? k - C : 0]
+                      : k < 3 * C ? xl[k < 3 * C && k >= 2 * C ? k - 2 * C : 0]
+                      : __float2half(k < 3 * C + 2 ? 1.0f : 0.0f);
             }
             *(uint4*)(base + (size_t)k8 * (128 * 8)) = *(const uint4*)hv;
         }
