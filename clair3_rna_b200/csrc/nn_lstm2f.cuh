@@ -396,7 +396,7 @@ inline void lstm2f_pack(std::vector<uint8_t>& out, const float* h, size_t o_w2, 
 }
 
 template <int NP, bool PROF>
-inline cudaError_t launch_lstm2f_np(const Lstm2fArgs& a, int sm_count, cudaStream_t st) {
+inline cudaError_t launch_lstm2f_np(const Lstm2fArgs& a, int sm_count, int max_clusters, cudaStream_t st) {
     static bool attr = false;
     if (!attr) {
         cudaError_t e = cudaFuncSetAttribute(k_lstm2_fused<NP, PROF>, cudaFuncAttributeMaxDynamicSharedMemorySize, L2F_SMEM);
@@ -420,6 +420,7 @@ inline cudaError_t launch_lstm2f_np(const Lstm2fArgs& a, int sm_count, cudaStrea
         if (cudaOccupancyMaxActiveClusters(&n_cl, k_lstm2_fused<NP, PROF>, &q) == cudaSuccess && n_cl > 0 && n_cl / 2 < max_per_dir)
             max_per_dir = n_cl / 2;
     }
+    if (max_per_dir > max_clusters) max_per_dir = max_clusters;
     if (max_per_dir < 1) max_per_dir = 1;
     if (per_dir > max_per_dir) per_dir = max_per_dir;
     if (per_dir < 1) per_dir = 1;
@@ -446,12 +447,13 @@ inline int lstm2f_np() {
     return v;
 }
 
-inline cudaError_t launch_lstm2f(const Lstm2fArgs& a, int sm_count, cudaStream_t st) {
-    if (a.prof) return launch_lstm2f_np<1, true>(a, sm_count, st);       // C3R_TRACE: the instrumented build
+// max_clusters: at most this many clusters per direction (a smaller grid takes more rounds of its persistent loop)
+inline cudaError_t launch_lstm2f(const Lstm2fArgs& a, int sm_count, int max_clusters, cudaStream_t st) {
+    if (a.prof) return launch_lstm2f_np<1, true>(a, sm_count, max_clusters, st);       // C3R_TRACE: the instrumented build
     switch (lstm2f_np()) {
-        case 2: return launch_lstm2f_np<2, false>(a, sm_count, st);
-        case 4: return launch_lstm2f_np<4, false>(a, sm_count, st);
-        default: return launch_lstm2f_np<1, false>(a, sm_count, st);
+        case 2: return launch_lstm2f_np<2, false>(a, sm_count, max_clusters, st);
+        case 4: return launch_lstm2f_np<4, false>(a, sm_count, max_clusters, st);
+        default: return launch_lstm2f_np<1, false>(a, sm_count, max_clusters, st);
     }
 }
 

@@ -22,11 +22,13 @@
 #pragma once
 #include <cstdint>
 #include <cstdlib>
+#include <cstring>
 #include <string>
 #include <vector>
 #include <cuda_runtime.h>
 #include <cuda_fp16.h>
 #include "nn_fp32.cuh"
+#include "nn_sched.h"
 #include "tc_ptx.cuh"
 
 namespace c3r {
@@ -779,7 +781,8 @@ inline int tc_ensure(TcNet& t, int tiles, std::string* err) {
 constexpr int TC_SUB_TILES = 320;
 
 template <int CH, int KX>
-inline cudaError_t launch_lstm(const LstmArgs& a, int sm_count, cudaStream_t st) {
+// max_cpairs: at most this many (forward, backward) cluster pairs (a smaller grid takes more rounds of its persistent loop)
+inline cudaError_t launch_lstm(const LstmArgs& a, int sm_count, int max_cpairs, cudaStream_t st) {
     typedef LstmCfg<CH, KX> Cfg;
     static bool attr = false;
     if (!attr) {
@@ -789,6 +792,7 @@ inline cudaError_t launch_lstm(const LstmArgs& a, int sm_count, cudaStream_t st)
     }
     int cpairs = a.n_tiles / 2;              // (forward, backward) cluster pairs, one per tile pair at most
     if (cpairs > sm_count / 4) cpairs = sm_count / 4;
+    if (cpairs > max_cpairs) cpairs = max_cpairs;
     if (cpairs < 1) cpairs = 1;
     k_lstm_tc<CH, KX><<<cpairs * 4, LSTM_THREADS, Cfg::SMEM, st>>>(a);
     return cudaGetLastError();
@@ -823,21 +827,25 @@ inline cudaError_t launch_gemm(const GemmArgs& g, int sm_count, cudaStream_t st)
 //
 // Work items of the recurrent kernels are (256-site tile pair, direction) on one CTA pair each, so a pass whose
 // item count is not a multiple of the 74 CTA pairs leaves SMs idle in its last round (116 items at 14.6 k sites:
-// the second round is 57 % full).  LSTM2 is therefore launched as A (the full rounds) and B (the rest), and the
-// L4 GEMM + heads of A run on a second stream while B is in flight: they are one-tile-per-CTA kernels, so they
-// simply take the SMs B leaves idle (measured: 2.205 -> 2.174 ms per forward at 14.6 k sites).
+// the second round is 57 % full).  A pass follows a plan of nn_sched.h: either rounds (LSTM1; LSTM2 as A, the full
+// rounds, and B, the rest, with the L4 GEMM + heads of A on a second stream beside B: one-tile-per-CTA kernels
+// that take the SMs B leaves idle) or two groups of SMs on the two streams, where LSTM1 waves of one group run
+// beside LSTM2 of the other.
 struct TcPipe {
     cudaStream_t s2 = nullptr;
-    cudaEvent_t ev[2] = {};
+    cudaEvent_t ev[8] = {};              // ev[i]: launch i of the pass's plan has ended
+    cudaEvent_t fork = nullptr;          // the second stream starts after the buffer waits of the caller's stream
     // Passes of different tickets run on different streams but share the scratch buffers.  A pass may write h2 / l4
     // once the previous pass has ended (pass_done).  (An event that was never recorded does not block.)
     cudaEvent_t pass_done = nullptr;
     // h1 is double-buffered (TcNet::h1[2]), so LSTM1 of the NEXT pass can run on the SMs the last LSTM2 launch of
     // this pass leaves idle (its remainder round: 84 of 148 SMs at config 2).
     // h1_free2[b]: LSTM2 has read buffer b;  xop_free: LSTM1 has read the shared operand image;
-    // last_ready / last_done: the last LSTM2 launch of the previous pass may start / has ended;  last_pairs: its tile pairs.
+    // last_ready: every LSTM2 launch of the previous pass but the one that ends last has ended;  last_done: all have;
+    // last_pairs: the cluster pairs of the one that ends last;  last_split: the previous pass ran in two groups.
     cudaEvent_t h1_free2[2] = {}, xop_free = nullptr, last_ready = nullptr, last_done = nullptr;
     int last_pairs = 0, parity = 0;
+    bool last_split = false;
     long n_pass = 0, n_overlap = 0;      // passes queued / passes whose LSTM1 went in pieces beside the previous pass (C3R_TIMING)
     bool ok = false;
 };
@@ -847,7 +855,8 @@ inline int tc_pipe_init(TcPipe& p, std::string* err) {
     cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);
     // the second stream (L4 + heads of the full rounds, beside LSTM2's remainder round) is high priority as well
     cudaError_t e = cudaStreamCreateWithPriority(&p.s2, cudaStreamNonBlocking, getenv("C3R_FLAT_PRIORITY") ? prio_lo : prio_hi);
-    for (int i = 0; i < 2 && e == cudaSuccess; ++i) e = cudaEventCreateWithFlags(&p.ev[i], cudaEventDisableTiming);
+    for (int i = 0; i < 8 && e == cudaSuccess; ++i) e = cudaEventCreateWithFlags(&p.ev[i], cudaEventDisableTiming);
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&p.fork, cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&p.pass_done, cudaEventDisableTiming);
     for (cudaEvent_t* ev : {&p.h1_free2[0], &p.h1_free2[1], &p.xop_free, &p.last_ready, &p.last_done})
         if (e == cudaSuccess) e = cudaEventCreateWithFlags(ev, cudaEventDisableTiming);
@@ -858,6 +867,7 @@ inline int tc_pipe_init(TcPipe& p, std::string* err) {
 inline void tc_pipe_release(TcPipe* p) {
     if (p->s2) cudaStreamDestroy(p->s2);
     for (cudaEvent_t e : p->ev) if (e) cudaEventDestroy(e);
+    if (p->fork) cudaEventDestroy(p->fork);
     if (p->pass_done) cudaEventDestroy(p->pass_done);
     for (cudaEvent_t ev : {p->h1_free2[0], p->h1_free2[1], p->xop_free, p->last_ready, p->last_done}) if (ev) cudaEventDestroy(ev);
     delete p;
@@ -866,14 +876,14 @@ inline void tc_pipe_release(TcPipe* p) {
 // tiles [t0, t0 + nt) of the pass, sites [s0, s0 + ns)
 struct TcSub { int t0, nt; int64_t s0, ns; };
 
-inline cudaError_t tc_lstm2(TcNet& t, const TcSub& b, cudaStream_t st, const __half* h1buf) {
+inline cudaError_t tc_lstm2(TcNet& t, const TcSub& b, int max_pairs, cudaStream_t st, const __half* h1buf) {
     Lstm2fArgs f;
     f.wstream = t.wstream2; f.h1 = h1buf + (size_t)b.t0 * NT * 4 * TC_IMG;
     f.hout = t.h2 + (size_t)b.t0 * NT * 5 * TC_IMG;
     f.hout_lo = (l4_terms() & 2) ? t.h2_lo + (size_t)b.t0 * NT * 5 * TC_IMG : nullptr;
     f.n_tiles = b.nt; f.err = t.err;
     f.prof = (t.trace && b.t0 == 0) ? t.trace + 2 * NT * 8 * 8 : nullptr;   // C3R_TRACE: wait-time totals of cluster 0 (LSTM2's part of the trace buffer)
-    return launch_lstm2f(f, t.sm_count, st);
+    return launch_lstm2f(f, t.sm_count, max_pairs / lstm2f_np(), st);
 }
 inline cudaError_t tc_l4_heads(TcNet& t, const NetF32& net, const TcSub& b, float* probs, cudaStream_t st) {
     GemmArgs g4;
@@ -933,28 +943,26 @@ inline int tc_forward(TcNet& t, const NetF32& net, const int32_t* tensor, int64_
             else k_xop<30, lstm1_kx(30)><<<tiles * NT, TC_TILE, 0, st>>>(tensor + o * NT * t.C, t.xop, m);
             ++launches;
         }
-        // A = the tile pairs that fill whole rounds of the recurrent kernels, B = the rest
-        // tile pairs one round of the LSTM2 kernel takes (clusters of 2*NP CTAs, half of them per direction)
         const int pairs = tiles / 2;
+        const int slots = t.sm_count / 4 > 0 ? t.sm_count / 4 : 1;          // tile pairs the recurrent kernels hold at once
+        // tile pairs one round of the LSTM2 kernel takes (clusters of 2*NP CTAs, half of them per direction)
         const int per_round = (t.sm_count / (2 * lstm2f_np()) / 2) * lstm2f_np();
-        int pa = pairs;
-        if (pairs > per_round && pairs % per_round != 0) pa = (pairs / per_round) * per_round;
-        TcSub A, B;
-        A.t0 = 0; A.nt = 2 * pa; A.s0 = 0; A.ns = m < (int64_t)A.nt * TC_TILE ? m : (int64_t)A.nt * TC_TILE;
-        B.t0 = A.nt; B.nt = tiles - A.nt; B.s0 = A.ns; B.ns = m - A.ns;
-        auto lstm1 = [&](const TcSub& b, cudaStream_t s) -> cudaError_t {
+        auto lstm1 = [&](const TcSub& b, int cap, cudaStream_t s) -> cudaError_t {
             LstmArgs a1;
             a1.Wimg = t.img1; a1.xop = xop_in + (size_t)b.t0 * NT * t.KX * TC_TILE;
             a1.hout = h1buf + (size_t)b.t0 * NT * 4 * TC_IMG;
             a1.n_sites = b.ns; a1.n_tiles = b.nt; a1.err = t.err; a1.trace = b.t0 == 0 ? t.trace : nullptr;
-            return t.C == 18 ? launch_lstm<4, lstm1_kx(18)>(a1, t.sm_count, s) : launch_lstm<4, lstm1_kx(30)>(a1, t.sm_count, s);
+            return t.C == 18 ? launch_lstm<4, lstm1_kx(18)>(a1, t.sm_count, cap, s) : launch_lstm<4, lstm1_kx(30)>(a1, t.sm_count, cap, s);
         };
-        // The last LSTM2 launch of the pass before this one (its remainder round, or its only round) leaves
-        // sm_count - 4 x pairs SMs idle: while it is still ahead of us, LSTM1 of THIS pass goes in pieces that fit
-        // beside it - two pieces (an LSTM1 round takes less than half an LSTM2 round), then the rest once it has
-        // ended.  At config 2 (37 + 21 tile pairs): 16 + 16 pairs of LSTM1 run under the previous pass's
-        // remainder round and the remaining 26 are ONE round instead of two; a 5 Mb chunk of config 5 (20 pairs,
-        // one partly filled round) puts all of its LSTM1 beside the previous chunk's LSTM2.
+        // The last LSTM2 launch of the pass before this one leaves sm_count - 4 x last_pairs SMs idle: while it is
+        // still ahead of us, LSTM1 of THIS pass goes beside it.  After a pass of rounds (its remainder round, or its
+        // only round) LSTM1 goes in pieces that fit - two pieces (an LSTM1 round takes less than half an LSTM2
+        // round), then the rest once it has ended.  At config 2 (37 + 21 tile pairs): 16 + 16 pairs of LSTM1 run
+        // under the previous pass's remainder round and the remaining 26 are ONE round instead of two; a 5 Mb chunk
+        // of config 5 (20 pairs, one partly filled round) puts all of its LSTM1 beside the previous chunk's LSTM2.
+        // After a pass in two groups, the last LSTM2 launch ends soon after the other group's: LSTM1 goes as one
+        // launch that starts on the SMs that group released and takes the rest as the last launch ends.
+        // Such a pass runs its LSTM2 in rounds.
         const int ip = (t.sm_count - 4 * P.last_pairs) / 4;         // tile pairs (both directions) that fit beside it
         bool overlap = o == 0 && P.last_pairs > 0 && ip >= 8 && getenv("C3R_NO_LSTM1_OVERLAP") == nullptr;
         if (overlap) {
@@ -967,52 +975,84 @@ inline int tc_forward(TcNet& t, const NetF32& net, const int32_t* tensor, int64_
             b.ns = left < 0 ? 0 : left < (int64_t)b.nt * TC_TILE ? left : (int64_t)b.nt * TC_TILE;
             return b;
         };
+        // C3R_PASS_SCHEDULE=rounds: every pass in rounds
+        const char* ps = getenv("C3R_PASS_SCHEDULE");
+        const SchedPlan plan = overlap || (ps && strcmp(ps, "rounds") == 0) ? sched_rounds(pairs, slots, per_round)
+                                                                            : sched_plan(pairs, slots, per_round, lstm2f_np());
         ++P.n_pass;
+        int first = 0;                                                  // plan launches already issued
         if (overlap) {
             ++P.n_overlap;
             TCK(cudaStreamWaitEvent(st, P.last_ready, 0), "wait");
-            int done = 0;
-            for (int c = 0; c < 2 && done < pairs; ++c) {
-                const int np = pairs - done < ip ? pairs - done : ip;
-                TCK(lstm1(piece(done, np), st), "lstm1");
-                done += np; ++launches;
+            if (P.last_split) {
+                TCK(lstm1(piece(0, pairs), slots, st), "lstm1");
+            } else {
+                int done = 0;
+                for (int c = 0; c < 2 && done < pairs; ++c) {
+                    const int np = pairs - done < ip ? pairs - done : ip;
+                    TCK(lstm1(piece(done, np), slots, st), "lstm1");
+                    done += np; ++launches;
+                }
+                if (done < pairs) {
+                    TCK(cudaStreamWaitEvent(st, P.last_done, 0), "wait");
+                    TCK(lstm1(piece(done, pairs - done), slots, st), "lstm1");
+                } else --launches;                                      // (counted with the plan's launch below)
             }
-            if (done < pairs) {
-                TCK(cudaStreamWaitEvent(st, P.last_done, 0), "wait");
-                TCK(lstm1(piece(done, pairs - done), st), "lstm1");
-            } else --launches;                                          // (the common count below adds one)
-        } else {
-            TcSub all; all.t0 = 0; all.nt = tiles; all.s0 = 0; all.ns = m;
-            TCK(lstm1(all, st), "lstm1");
+            TCK(cudaEventRecord(P.ev[0], st), "event");
+            first = 1;                                                  // in place of the plan's LSTM1 (launch 0)
+            ++launches;
         }
-        TCK(cudaEventRecord(P.xop_free, st), "event");
-        TCK(cudaStreamWaitEvent(st, P.pass_done, 0), "wait");       // the previous pass no longer reads h2 / l4
-        ++launches;
+        cudaStream_t ss[2] = {st, P.s2};
+        TCK(cudaEventRecord(P.fork, st), "event");
+        TCK(cudaStreamWaitEvent(P.s2, P.fork, 0), "wait");
+        // the last launch of `kind` on stream `s` listed before launch i, or -1
+        auto last_of = [&](int kind, int s, int i) {
+            int r = -1;
+            for (int j = 0; j < i; ++j) if (plan.l[j].kind == kind && plan.l[j].stream == s) r = j;
+            return r;
+        };
+        int l1_last = -1, l2_last = -1, l2_prev = -1, s2_last = -1;
+        for (int i = 0; i < plan.n; ++i) {
+            if (plan.l[i].kind == SCHED_LSTM1) l1_last = i;
+            if (plan.l[i].kind == SCHED_LSTM2) { l2_prev = l2_last; l2_last = i; }
+            if (plan.l[i].stream == 1) s2_last = i;
+        }
+        bool h2_free[2] = {false, false};                               // stream waited for pass_done
         float* pr = probs + o * 24;
-        if (B.nt == 0) TCK(cudaEventRecord(P.last_ready, st), "event");
-        TCK(tc_lstm2(t, A, st, h1buf), "lstm2");
-        ++launches;
-        if (B.nt == 0) {
-            TCK(cudaEventRecord(P.last_done, st), "event");
-            TCK(cudaEventRecord(P.h1_free2[hb], st), "event");
-            P.last_pairs = pa;
-            TCK(tc_l4_heads(t, net, A, pr, st), "l4/heads");
-            launches += 4;
-            TCK(cudaEventRecord(P.pass_done, st), "event");
-            continue;
+        for (int i = 0; i < plan.n; ++i) {
+            const SchedLaunch& L = plan.l[i];
+            cudaStream_t s = ss[L.stream];
+            const int other = L.stream ^ 1;
+            if (L.wait >= 0) TCK(cudaStreamWaitEvent(s, P.ev[L.wait], 0), "wait");
+            if (L.kind == SCHED_LSTM2 && !h2_free[L.stream]) {
+                TCK(cudaStreamWaitEvent(s, P.pass_done, 0), "wait");   // the previous pass no longer reads h2 / l4
+                h2_free[L.stream] = true;
+            }
+            if (i == l2_last && l2_prev < 0) TCK(cudaEventRecord(P.last_ready, s), "event");
+            if (i >= first) {
+                if (L.kind == SCHED_LSTM1) TCK(lstm1(piece(L.p0, L.np), L.cap, s), "lstm1");
+                else if (L.kind == SCHED_LSTM2) TCK(tc_lstm2(t, piece(L.p0, L.np), L.cap, s, h1buf), "lstm2");
+                else { TCK(tc_l4_heads(t, net, piece(L.p0, L.np), pr, s), "l4/heads"); launches += 3; }
+                ++launches;
+                TCK(cudaEventRecord(P.ev[i], s), "event");
+            }
+            // the shared operand image is free once every LSTM1 launch has read it; LSTM2 of the pass has read h1
+            // (and its last launch has ended) once every LSTM2 launch has ended
+            const int kind_last = i == l1_last ? SCHED_LSTM1 : i == l2_last || i == l2_prev ? SCHED_LSTM2 : -1;
+            if (kind_last >= 0) {
+                const int j = last_of(kind_last, other, i);
+                if (j >= 0) TCK(cudaStreamWaitEvent(s, P.ev[j], 0), "wait");
+            }
+            if (i == l1_last) TCK(cudaEventRecord(P.xop_free, s), "event");
+            if (i == l2_prev) TCK(cudaEventRecord(P.last_ready, s), "event");
+            if (i == l2_last) {
+                TCK(cudaEventRecord(P.last_done, s), "event");
+                TCK(cudaEventRecord(P.h1_free2[hb], s), "event");
+                P.last_pairs = L.np < L.cap ? L.np : L.cap;
+                P.last_split = plan.split != 0;
+            }
         }
-        TCK(cudaEventRecord(P.ev[0], st), "event");
-        TCK(cudaEventRecord(P.last_ready, st), "event");
-        TCK(tc_lstm2(t, B, st, h1buf), "lstm2");
-        TCK(cudaEventRecord(P.last_done, st), "event");
-        TCK(cudaEventRecord(P.h1_free2[hb], st), "event");
-        P.last_pairs = B.nt / 2;
-        TCK(cudaStreamWaitEvent(P.s2, P.ev[0], 0), "wait");
-        TCK(tc_l4_heads(t, net, A, pr, P.s2), "l4/heads");
-        TCK(cudaEventRecord(P.ev[1], P.s2), "event");
-        TCK(tc_l4_heads(t, net, B, pr, st), "l4/heads");
-        TCK(cudaStreamWaitEvent(st, P.ev[1], 0), "wait");       // the caller's stream ends after everything
-        launches += 9;
+        if (s2_last >= 0) TCK(cudaStreamWaitEvent(st, P.ev[s2_last], 0), "wait");   // the caller's stream ends after everything
         TCK(cudaEventRecord(P.pass_done, st), "event");
     }
 #undef TCK
