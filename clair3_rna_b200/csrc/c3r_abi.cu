@@ -21,6 +21,7 @@
 #include "pileup.cuh"
 #include "nn_fp32.cuh"
 #include "nn_tc.cuh"
+#include "call.cuh"
 
 using namespace c3r;
 
@@ -45,6 +46,8 @@ struct Slot {
     cudaStream_t st_a = nullptr;      // H2D copies and stage A (low priority: they fill the SMs the network passes leave idle)
     cudaEvent_t ev[N_EV] = {};
     cudaEvent_t ev_alt = nullptr;
+    cudaEvent_t ev_call[2] = {};      // around k_call
+    bool calls = false;               // call records for this ticket (c3r_enable_calls when it was submitted)
     // inputs
     Buf pos, flag, mapq, hp, cigar_off, cigar, seq_off, seq, ref;
     // per read/op
@@ -56,6 +59,7 @@ struct Slot {
     Buf binc, bin_cur, events, raw, cov, cov_tile, refnib;
     Buf pbed, cbed, known, covP;   // site filters of the chunk; printed columns (covA inside the pileup BED)
     Buf cand_row, cand_pos, cand_depth, tensor, alt_off, alt_n, alt, cur_ref, deleted, probs;
+    Buf d_calls;          // call records (k_call)
     Buf xop;              // LSTM1 operand images written by k_window_xop (fused K4 -> K5 path)
     bool fused_window = false;
     Buf scalars;          // [0] n_rows (i64) [1] n_cand (i64) [2] alt_total (i64) [3] err (i32) [4] tail columns (2 x i32) [5] raw row events (i64)
@@ -73,7 +77,7 @@ struct Slot {
     int deferred_rc = 0;              // error of the deferred part, reported by c3r_wait
     std::string deferred_err;
     // pinned results
-    Pin h_scalars, h_pos, h_depth, h_probs, h_alt_off, h_alt_n, h_alt, h_tensor, h_row_pos, h_counts, h_row_depth;
+    Pin h_scalars, h_pos, h_depth, h_probs, h_alt_off, h_alt_n, h_alt, h_tensor, h_row_pos, h_counts, h_row_depth, h_calls;
     Dev d;
     int64_t n_rows = 0, n_cand = 0, alt_total = 0;
     int launches = 0;
@@ -106,6 +110,7 @@ struct c3r_ctx {
     int64_t ref_res_start0 = 0, ref_res_len = 0;
     double t_phase[8] = {};   // C3R_TIMING: host seconds of submit's phases (printed by c3r_destroy)
     int64_t n_submit = 0;
+    bool calls = false;       // c3r_enable_calls: tickets submitted from now on make call records
     Buf fwd_in, fwd_out;      // c3r_forward staging
     cudaStream_t fwd_stream = nullptr;
 };
@@ -156,6 +161,25 @@ void release(Pin& b) { if (b.p) cudaFreeHost(b.p); b.p = nullptr; b.cap = 0; }
 template <class T> T* P(Buf& b) { return (T*)b.p; }
 
 // ------------------------------------------------------------ device stages
+// The call record of every candidate (csrc/call.cuh): a thread per candidate, reading the allele table, the
+// probabilities, the reference window and the reads' sequence pool where stage B left them.
+__global__ void __launch_bounds__(128) k_call(const Dev d, const float* __restrict__ probs, int64_t n, c3r_call* __restrict__ out) {
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        c3rcall::CallIn c;
+        c.e = reinterpret_cast<const c3r_alt_entry*>(d.alt) + d.alt_off[i];
+        c.n = d.alt_n[i];
+        c.probs = probs + 24 * i;
+        c.ref = d.ref;
+        c.ref_len = d.ref_len;
+        c.p0 = (int64_t)d.cand_pos[i] - (d.ref_start0 + 1);
+        c.seq = d.seq;
+        c3r_call r;
+        c3rcall::decide_call(c, r);
+        out[i] = r;
+    }
+}
+static_assert(sizeof(AltEntry) == sizeof(c3r_alt_entry), "AltEntry mirrors c3r_alt_entry");
+
 // Stage A: everything up to the candidate list.  Needs only the resident inputs.
 int run_stage_a(c3r_ctx* ctx, Slot& s) {
     Dev& d = s.d;
@@ -254,6 +278,7 @@ int ensure_stage_b(c3r_ctx* ctx, Slot& s) {
     d.alt_cap = 4 * n + d.events_ub + 8;
     if (ensure(ctx, s.alt, (size_t)d.alt_cap * sizeof(AltEntry))) return C3R_ERR_CUDA;
     if (ensure(ctx, s.probs, (size_t)n * 24 * 4)) return C3R_ERR_CUDA;
+    if (s.calls && ensure(ctx, s.d_calls, (size_t)n * sizeof(c3r_call))) return C3R_ERR_CUDA;
     d.tensor = P<int32_t>(s.tensor);
     d.alt_off = P<int64_t>(s.alt_off);
     d.alt_n = P<int32_t>(s.alt_n);
@@ -295,6 +320,15 @@ int run_stage_b(c3r_ctx* ctx, Slot& s) {
         L += nl;
     }
     CK(cudaEventRecord(s.ev[7], st));
+    if (s.calls) {
+        CK(cudaEventRecord(s.ev_call[0], st));
+        if (n > 0) {
+            const int64_t blocks = (n + 127) / 128;
+            k_call<<<(unsigned)(blocks < ctx->sm_count * 16 ? blocks : ctx->sm_count * 16), 128, 0, st>>>(d, P<float>(s.probs), n, P<c3r_call>(s.d_calls));
+            ++L;
+        }
+        CK(cudaEventRecord(s.ev_call[1], st));
+    }
     CK(cudaGetLastError());
     return 0;
 }
@@ -314,6 +348,10 @@ int queue_d2h(c3r_ctx* ctx, Slot& s) {
         CK(cudaMemcpyAsync(s.h_probs.p, s.probs.p, n * 96, cudaMemcpyDeviceToHost, st));
         CK(cudaMemcpyAsync(s.h_alt_off.p, s.alt_off.p, n * 8, cudaMemcpyDeviceToHost, st));
         CK(cudaMemcpyAsync(s.h_alt_n.p, s.alt_n.p, n * 4, cudaMemcpyDeviceToHost, st));
+        if (s.calls) {
+            if (ensure_pin(ctx, s.h_calls, (size_t)n * sizeof(c3r_call))) return C3R_ERR_CUDA;
+            CK(cudaMemcpyAsync(s.h_calls.p, s.d_calls.p, (size_t)n * sizeof(c3r_call), cudaMemcpyDeviceToHost, st));
+        }
         if (ctx->prm.keep_tensor) {
             if (ensure_pin(ctx, s.h_tensor, (size_t)n * per * 4)) return C3R_ERR_CUDA;
             CK(cudaMemcpyAsync(s.h_tensor.p, s.tensor.p, (size_t)n * per * 4, cudaMemcpyDeviceToHost, st));
@@ -402,6 +440,7 @@ int c3r_create(c3r_ctx** out, int device_ordinal, const c3r_params* params) {
         CK(cudaStreamCreateWithPriority(&s.st_a, cudaStreamNonBlocking, prio_lo));
         for (int k = 0; k < N_EV; ++k) CK(cudaEventCreate(&s.ev[k]));
         CK(cudaEventCreateWithFlags(&s.ev_alt, cudaEventDisableTiming));
+        for (int k = 0; k < 2; ++k) CK(cudaEventCreate(&s.ev_call[k]));
         // spin-wait by default: a blocking-sync event wakes the waiting thread ~0.3 ms late (measured), which delays
         // stage B by as much; C3R_BLOCKING_COUNTS trades that for an idle core while waiting
         CK(cudaEventCreateWithFlags(&s.ev_cnt, cudaEventDisableTiming | (getenv("C3R_BLOCKING_COUNTS") ? cudaEventBlockingSync : 0)));
@@ -435,13 +474,14 @@ void c3r_destroy(c3r_ctx* ctx) {
                      &s.word_base, &s.row_pos, &s.counts, &s.row_depth, &s.row_flag, &s.head_cnt, &s.tail_cnt,
                      &s.skipdiff, &s.max_skip, &s.row_ins, &s.row_del, &s.binc, &s.bin_cur, &s.events, &s.raw, &s.cov, &s.cov_tile, &s.refnib,
                      &s.cand_row, &s.cand_pos, &s.cand_depth, &s.tensor, &s.alt_off, &s.alt_n, &s.alt, &s.cur_ref,
-                     &s.deleted, &s.probs, &s.scalars, &s.scan_scratch, &s.pbed, &s.cbed, &s.known, &s.covP, &s.xop};
+                     &s.deleted, &s.probs, &s.scalars, &s.scan_scratch, &s.pbed, &s.cbed, &s.known, &s.covP, &s.xop, &s.d_calls};
         for (Buf* b : bs) release(*b);
         Pin* ps[] = {&s.h_scalars, &s.h_pos, &s.h_depth, &s.h_probs, &s.h_alt_off, &s.h_alt_n, &s.h_alt, &s.h_tensor,
-                     &s.h_row_pos, &s.h_counts, &s.h_row_depth};
+                     &s.h_row_pos, &s.h_counts, &s.h_row_depth, &s.h_calls};
         for (Pin* b : ps) release(*b);
         for (int k = 0; k < N_EV; ++k) if (s.ev[k]) cudaEventDestroy(s.ev[k]);
         if (s.ev_alt) cudaEventDestroy(s.ev_alt);
+        for (int k = 0; k < 2; ++k) if (s.ev_call[k]) cudaEventDestroy(s.ev_call[k]);
         if (s.ev_cnt) cudaEventDestroy(s.ev_cnt);
         if (s.st) cudaStreamDestroy(s.st);
         if (s.st_a) cudaStreamDestroy(s.st_a);
@@ -627,6 +667,7 @@ static int submit_once(c3r_ctx* ctx, const c3r_reads* rd, const uint8_t* ref, in
     Slot& s = ctx->slots[si];
     s.launches = 0;
     s.has_result = false;
+    s.calls = ctx->calls;
     Dev& d = s.d;
     memset(&d, 0, sizeof d);
     const c3r_params& pr = ctx->prm;
@@ -832,12 +873,32 @@ int c3r_wait(c3r_ctx* ctx, c3r_ticket ticket, c3r_result* res) {
     }
     for (int k = 0; k < 8; ++k) {
         float ms = 0.f;
-        cudaEventElapsedTime(&ms, s.ev[k], s.ev[k + 1]);
+        cudaEventElapsedTime(&ms, k == 7 && s.calls ? s.ev_call[1] : s.ev[k], s.ev[k + 1]);   // D2H: after k_call
         r.stage_ms[k] = ms;
     }
     r.kernel_launches = s.launches;
     *res = r;
     (void)d;
+    return C3R_OK;
+}
+
+int c3r_enable_calls(c3r_ctx* ctx, int on) {
+    if (!ctx) return C3R_ERR_ARG;
+    ctx->calls = on != 0;
+    return C3R_OK;
+}
+
+int c3r_wait_calls(c3r_ctx* ctx, c3r_ticket ticket, const c3r_call** calls, int64_t* n, float* device_ms) {
+    if (!ctx || !calls || !n || ticket < 0 || ticket >= N_SLOTS) return C3R_ERR_ARG;
+    Slot& s = ctx->slots[ticket];
+    if (!s.in_use || !s.has_result) return fail(ctx, C3R_ERR_STATE, "c3r_wait_calls needs a ticket c3r_wait has returned");
+    if (!s.calls) return fail(ctx, C3R_ERR_STATE, "call records were off when this ticket was submitted (c3r_enable_calls)");
+    *calls = s.n_cand > 0 ? (const c3r_call*)s.h_calls.p : nullptr;
+    *n = s.n_cand;
+    if (device_ms) {
+        CK(cudaSetDevice(ctx->device));
+        CK(cudaEventElapsedTime(device_ms, s.ev_call[0], s.ev_call[1]));
+    }
     return C3R_OK;
 }
 

@@ -24,6 +24,7 @@
 #include <vector>
 
 #include "../../include/c3r_b200.h"
+#include "call.cuh"
 
 namespace {
 
@@ -331,6 +332,48 @@ void dict_set(std::vector<std::pair<std::string, int>>& d, const std::string& k,
     d.emplace_back(k, v);
 }
 
+// output_with's row text from the decision: AF, QUAL, FILTER and the line (with '\n') appended to `out`.  Shared by
+// c3r_decode_vcf and c3r_format_vcf, so that both print the same bytes.
+void put_row(const char* contig, int pos, std::string& ref_base, std::string& alt_base, bool is_ref, const char* gt,
+             int depth, int ref_count, const long* counts, size_t n_counts, long support, float prob, double qual_cut,
+             std::string& out) {
+    double af = depth != 0 ? ((double)support + 0.0) / (double)depth : 0.0;
+    if (af > 1) af = 1;
+    const double p = (double)prob;
+    char qtxt[64];
+    const double qual = round2(PHRED_TRANS * std::log(((1.0 - p) + 1e-10) / (p + 1e-10)) + 10, qtxt, sizeof qtxt);
+    const char* filt = is_ref ? "RefCall" : ((qual_cut < 0 || qual >= qual_cut) ? "PASS" : "LowQual");
+    ref_base = iupac_to_n(ref_base);
+    alt_base = iupac_to_n(alt_base);
+    char buf[160];
+    char* b = buf;
+    out += contig;
+    *b++ = '\t'; b = put_int(b, pos); *b++ = '\t'; *b++ = '.'; *b++ = '\t';
+    out.append(buf, (size_t)(b - buf));
+    out += ref_base; out += '\t'; out += alt_base; out += '\t'; out += qtxt; out += '\t'; out += filt;
+    out += "\t.\tGT:GQ:DP:AD:AF\t";
+    out += gt;
+    b = buf;
+    *b++ = ':'; b = put_int(b, (long)(int)qual); *b++ = ':'; b = put_int(b, depth); *b++ = ':'; b = put_int(b, ref_count);
+    out.append(buf, (size_t)(b - buf));
+    for (size_t i = 0; i < n_counts; ++i) { b = buf; *b++ = ','; b = put_int(b, counts[i]); out.append(buf, (size_t)(b - buf)); }
+    out += ':';
+    if (n_counts <= 1) {
+        b = af >= 0 ? put_fixed(buf, af, 4) : buf + snprintf(buf, sizeof buf, "%.4f", af);
+        out.append(buf, (size_t)(b - buf));
+    } else {
+        for (size_t i = 0; i < n_counts; ++i) {
+            double a = 1.0 * (double)counts[i] / (double)depth;
+            if (a > 1.0) a = 1.0;
+            b = buf;
+            if (i) *b++ = ',';
+            b = (a >= 0) ? put_fixed(b, a, 4) : b + snprintf(b, 64, "%.4f", a);       // nan / negative: libc's text
+            out.append(buf, (size_t)(b - buf));
+        }
+    }
+    out += '\n';
+}
+
 // output_with: appends one VCF line (with '\n') to `out`; returns false when the reference prints nothing
 bool vcf_row(const char* contig, int pos, const std::string& ref33, int depth, const std::vector<Allele>& alt,
              const float* probs, double qual_cut, bool show_ref, std::string& out) {
@@ -420,97 +463,24 @@ bool vcf_row(const char* contig, int pos, const std::string& ref33, int depth, c
             support += c;
         }
     }
-    double af = depth != 0 ? ((double)support + 0.0) / (double)depth : 0.0;
-    if (af > 1) af = 1;
-    const double p = (double)D.prob;
-    char qtxt[64];
-    const double qual = round2(PHRED_TRANS * std::log(((1.0 - p) + 1e-10) / (p + 1e-10)) + 10, qtxt, sizeof qtxt);
-    const char* filt = is_ref ? "RefCall" : ((qual_cut < 0 || qual >= qual_cut) ? "PASS" : "LowQual");
-    ref_base = iupac_to_n(ref_base);
-    alt_base = iupac_to_n(alt_base);
-    char buf[160];
-    char* b = buf;
-    out += contig;
-    *b++ = '\t'; b = put_int(b, pos); *b++ = '\t'; *b++ = '.'; *b++ = '\t';
-    out.append(buf, (size_t)(b - buf));
-    out += ref_base; out += '\t'; out += alt_base; out += '\t'; out += qtxt; out += '\t'; out += filt;
-    out += "\t.\tGT:GQ:DP:AD:AF\t";
-    out += gt;
-    b = buf;
-    *b++ = ':'; b = put_int(b, (long)(int)qual); *b++ = ':'; b = put_int(b, depth); *b++ = ':'; b = put_int(b, ref_count);
-    out.append(buf, (size_t)(b - buf));
-    for (long c : counts) { b = buf; *b++ = ','; b = put_int(b, c); out.append(buf, (size_t)(b - buf)); }
-    out += ':';
-    if (counts.size() <= 1) {
-        b = af >= 0 ? put_fixed(buf, af, 4) : buf + snprintf(buf, sizeof buf, "%.4f", af);
-        out.append(buf, (size_t)(b - buf));
-    } else {
-        for (size_t i = 0; i < counts.size(); ++i) {
-            double a = 1.0 * (double)counts[i] / (double)depth;
-            if (a > 1.0) a = 1.0;
-            b = buf;
-            if (i) *b++ = ',';
-            b = (a >= 0) ? put_fixed(b, a, 4) : b + snprintf(b, 64, "%.4f", a);       // nan / negative: libc's text
-            out.append(buf, (size_t)(b - buf));
-        }
-    }
-    out += '\n';
+    put_row(contig, pos, ref_base, alt_base, is_ref, gt, depth, ref_count, counts.data(), counts.size(), support, D.prob,
+            qual_cut, out);
     return true;
 }
 
-}  // namespace
-
-extern "C" {
-
-// One VCF data line per candidate of `res`, in order, into a malloc'ed buffer (free with c3r_free_text).
-// reads: the records the result was computed from (inserted bases are read from reads->seq);
-// ref/ref_start1/ref_len: the reference window given to c3r_submit_chunk.  qual_cut < 0: no LowQual filter.
-int c3r_decode_vcf(const c3r_result* res, const c3r_reads* reads, const uint8_t* ref, int64_t ref_start1, int64_t ref_len,
-                   const char* contig, double qual_cut, int show_ref, int n_threads, char** text, int64_t* n_bytes, int64_t* n_rows) {
-    if (!res || !ref || !contig || !text || !n_bytes || !n_rows) return C3R_ERR_ARG;
-    const int64_t n = res->n_cand;
-    *text = nullptr; *n_bytes = 0; *n_rows = 0;
-    if (n > 0 && (!res->pos || !res->depth || !res->probs || !res->alt_off || !res->alt_n)) return C3R_ERR_ARG;
+// rows(i, out) appends the line of candidate i to `out` and says whether it printed one; candidates are split into
+// n_threads contiguous ranges whose texts are joined in order into one malloc'ed buffer
+template <class Rows>
+int rows_in_parallel(int64_t n, int n_threads, const Rows& rows, char** text, int64_t* n_bytes, int64_t* n_rows) {
     int nt = n_threads > 0 ? n_threads : (int)std::max(1u, std::thread::hardware_concurrency());
     if ((int64_t)nt > (n + 255) / 256) nt = (int)std::max<int64_t>(1, (n + 255) / 256);
     std::vector<std::string> parts(nt);
-    std::vector<int64_t> rows(nt, 0);
+    std::vector<int64_t> counted(nt, 0);
     auto work = [&](int t) {
         const int64_t a = n * t / nt, b = n * (t + 1) / nt;
         std::string& out = parts[t];
         out.reserve((size_t)(b - a) * 64);
-        std::vector<Allele> alt;
-        std::string ref33;
-        for (int64_t i = a; i < b; ++i) {
-            const int64_t p0 = (int64_t)res->pos[i] - ref_start1;            // offset of the candidate in ref
-            // 33-base context, padded with 'A' off the loaded reference (create_tensor_pileup.py:313-331)
-            ref33.assign(2 * FLANK + 1, 'A');
-            for (int k = -FLANK; k <= FLANK; ++k) {
-                const int64_t o = p0 + k;
-                if (o >= 0 && o < ref_len) ref33[k + FLANK] = (char)ref[o];
-            }
-            if (!base2acgt(ref33[FLANK])) continue;                          // clair3_rna/utils.py:113
-            alt.clear();
-            const c3r_alt_entry* e = res->alt + res->alt_off[i];
-            for (int32_t k = 0; k < res->alt_n[i]; ++k) {
-                Allele al;
-                al.kind = (char)e[k].kind;
-                al.count = e[k].count;
-                if (al.kind == 'X' || al.kind == 'R') al.key.assign(1, (char)e[k].base);
-                else if (al.kind == 'I') {
-                    al.key.assign(1, (char)e[k].base);
-                    if (reads && reads->seq)
-                        for (uint32_t q = e[k].seq_off; q < e[k].seq_off + e[k].len; ++q) {
-                            const uint8_t by = reads->seq[q >> 1];
-                            al.key.push_back(NT16[(q & 1) ? (by & 15) : (by >> 4)]);
-                        }
-                } else {
-                    for (int64_t o = p0 + 1; o < p0 + 1 + (int64_t)e[k].len && o < ref_len; ++o) if (o >= 0) al.key.push_back((char)ref[o]);
-                }
-                alt.push_back(std::move(al));
-            }
-            if (vcf_row(contig, res->pos[i], ref33, res->depth[i], alt, res->probs + 24 * i, qual_cut, show_ref != 0, out)) ++rows[t];
-        }
+        for (int64_t i = a; i < b; ++i) if (rows(i, out)) ++counted[t];
     };
     if (nt <= 1) work(0);
     else {
@@ -527,7 +497,139 @@ int c3r_decode_vcf(const c3r_result* res, const c3r_reads* reads, const uint8_t*
     buf[total] = 0;
     *text = buf;
     *n_bytes = (int64_t)total;
-    for (int64_t r : rows) *n_rows += r;
+    for (int64_t r : counted) *n_rows += r;
+    return C3R_OK;
+}
+
+c3rcall::CallIn call_input(const c3r_result* res, int64_t i, const c3r_reads* reads, const uint8_t* ref, int64_t ref_start1,
+                           int64_t ref_len) {
+    c3rcall::CallIn c;
+    c.e = res->alt + res->alt_off[i];
+    c.n = res->alt_n[i];
+    c.probs = res->probs + 24 * i;
+    c.ref = ref;
+    c.ref_len = ref_len;
+    c.p0 = (int64_t)res->pos[i] - ref_start1;
+    c.seq = reads ? reads->seq : nullptr;
+    return c;
+}
+
+// The text of one allele of a call record (see c3r_call_allele)
+void put_allele(std::string& s, const c3r_call_allele& a, const uint8_t* seq, const uint8_t* ref, int64_t del_start,
+                int ref_len) {
+    s += (char)a.first;
+    if (seq)
+        for (uint32_t q = a.ins_seq_off; q < a.ins_seq_off + a.ins_len; ++q) s += NT16[c3rcall::nib(seq, q)];
+    for (int k = a.suffix_from; k < ref_len; ++k) s += (char)ref[del_start + k - 1];
+}
+
+}  // namespace
+
+extern "C" {
+
+// One VCF data line per candidate of `res`, in order, into a malloc'ed buffer (free with c3r_free_text).
+// reads: the records the result was computed from (inserted bases are read from reads->seq);
+// ref/ref_start1/ref_len: the reference window given to c3r_submit_chunk.  qual_cut < 0: no LowQual filter.
+int c3r_decode_vcf(const c3r_result* res, const c3r_reads* reads, const uint8_t* ref, int64_t ref_start1, int64_t ref_len,
+                   const char* contig, double qual_cut, int show_ref, int n_threads, char** text, int64_t* n_bytes, int64_t* n_rows) {
+    if (!res || !ref || !contig || !text || !n_bytes || !n_rows) return C3R_ERR_ARG;
+    const int64_t n = res->n_cand;
+    *text = nullptr; *n_bytes = 0; *n_rows = 0;
+    if (n > 0 && (!res->pos || !res->depth || !res->probs || !res->alt_off || !res->alt_n)) return C3R_ERR_ARG;
+    auto rows = [&](int64_t i, std::string& out) {
+        static thread_local std::vector<Allele> alt;
+        static thread_local std::string ref33;
+        const int64_t p0 = (int64_t)res->pos[i] - ref_start1;            // offset of the candidate in ref
+        // 33-base context, padded with 'A' off the loaded reference (create_tensor_pileup.py:313-331)
+        ref33.assign(2 * FLANK + 1, 'A');
+        for (int k = -FLANK; k <= FLANK; ++k) {
+            const int64_t o = p0 + k;
+            if (o >= 0 && o < ref_len) ref33[k + FLANK] = (char)ref[o];
+        }
+        if (!base2acgt(ref33[FLANK])) return false;                      // clair3_rna/utils.py:113
+        alt.clear();
+        const c3r_alt_entry* e = res->alt + res->alt_off[i];
+        for (int32_t k = 0; k < res->alt_n[i]; ++k) {
+            Allele al;
+            al.kind = (char)e[k].kind;
+            al.count = e[k].count;
+            if (al.kind == 'X' || al.kind == 'R') al.key.assign(1, (char)e[k].base);
+            else if (al.kind == 'I') {
+                al.key.assign(1, (char)e[k].base);
+                if (reads && reads->seq)
+                    for (uint32_t q = e[k].seq_off; q < e[k].seq_off + e[k].len; ++q) {
+                        const uint8_t by = reads->seq[q >> 1];
+                        al.key.push_back(NT16[(q & 1) ? (by & 15) : (by >> 4)]);
+                    }
+            } else {
+                for (int64_t o = p0 + 1; o < p0 + 1 + (int64_t)e[k].len && o < ref_len; ++o) if (o >= 0) al.key.push_back((char)ref[o]);
+            }
+            alt.push_back(std::move(al));
+        }
+        return vcf_row(contig, res->pos[i], ref33, res->depth[i], alt, res->probs + 24 * i, qual_cut, show_ref != 0, out);
+    };
+    return rows_in_parallel(n, n_threads, rows, text, n_bytes, n_rows);
+}
+
+// c3r_decode_vcf's lines from call records: what is left of output_with once the decision is made
+int c3r_format_vcf(const c3r_result* res, const c3r_call* calls, const c3r_reads* reads, const uint8_t* ref,
+                   int64_t ref_start1, int64_t ref_len, const char* contig, double qual_cut, int show_ref, int n_threads,
+                   char** text, int64_t* n_bytes, int64_t* n_rows) {
+    if (!res || !ref || !contig || !text || !n_bytes || !n_rows) return C3R_ERR_ARG;
+    const int64_t n = res->n_cand;
+    *text = nullptr; *n_bytes = 0; *n_rows = 0;
+    if (n > 0 && (!res->pos || !res->depth || !calls)) return C3R_ERR_ARG;
+    static const char* const GT_TEXT[5] = {"0/0", "1/1", "0/1", "1/2", "None"};
+    const uint8_t* seq = reads ? reads->seq : nullptr;
+    const int64_t n_bases = seq ? 2 * reads->n_seq_bytes : 0;
+    // A record that cannot be printed - malformed, or made over another window or read pool than the one given -
+    // fails the call instead of losing its row.  REF letters 1.. are reference bases after the candidate; a
+    // candidate off the window (its context padded with 'A') has REF = ref_first alone and reads none.
+    for (int64_t i = 0; i < n; ++i) {
+        const c3r_call& c = calls[i];
+        if (c.family == C3R_CALL_NO_ROW) continue;
+        if (c.family > 9 || c.gt > 4 || c.n_alt > 2 || c.n_ad > 2 || c.ref_len < 1) return C3R_ERR_ARG;
+        const int64_t p0 = (int64_t)res->pos[i] - ref_start1;
+        const int64_t ds = p0 + 1 < 0 ? 0 : p0 + 1;
+        if (c.ref_len > 1 && ds + c.ref_len - 1 > ref_len) return C3R_ERR_ARG;
+        for (int a = 0; a < c.n_alt; ++a) {
+            const c3r_call_allele& al = c.alt[a];
+            if (al.suffix_from < 1 || al.suffix_from > c.ref_len) return C3R_ERR_ARG;
+            if (seq && (int64_t)al.ins_seq_off + al.ins_len > n_bases) return C3R_ERR_ARG;
+        }
+    }
+    auto rows = [&](int64_t i, std::string& out) {
+        const c3r_call& c = calls[i];
+        if (c.family == C3R_CALL_NO_ROW) return false;
+        const bool is_ref = c.family == 0;
+        if (!show_ref && is_ref) return false;
+        static thread_local std::string ref_base, alt_base;
+        const int64_t p0 = (int64_t)res->pos[i] - ref_start1;
+        const int64_t ds = p0 + 1 < 0 ? 0 : p0 + 1;
+        ref_base.assign(1, (char)c.ref_first);
+        for (int k = 1; k < c.ref_len; ++k) ref_base += (char)ref[ds + k - 1];
+        if (c.n_alt == 0) alt_base.assign(1, '.');
+        else {
+            alt_base.clear();
+            for (int a = 0; a < c.n_alt; ++a) {
+                if (a) alt_base += ',';
+                put_allele(alt_base, c.alt[a], seq, ref, ds, c.ref_len);
+            }
+        }
+        const long counts[2] = {c.ad[0], c.ad[1]};
+        put_row(contig, res->pos[i], ref_base, alt_base, is_ref, GT_TEXT[c.gt], res->depth[i], c.ref_count, counts,
+                c.n_ad, c.support, c.prob, qual_cut, out);
+        return true;
+    };
+    return rows_in_parallel(n, n_threads, rows, text, n_bytes, n_rows);
+}
+
+int c3r_debug_decide_calls(const c3r_result* res, const c3r_reads* reads, const uint8_t* ref, int64_t ref_start1,
+                           int64_t ref_len, c3r_call* out) {
+    if (!res || !ref) return C3R_ERR_ARG;
+    const int64_t n = res->n_cand;
+    if (n > 0 && (!out || !res->pos || !res->probs || !res->alt_off || !res->alt_n)) return C3R_ERR_ARG;
+    for (int64_t i = 0; i < n; ++i) c3rcall::decide_call(call_input(res, i, reads, ref, ref_start1, ref_len), out[i]);
     return C3R_OK;
 }
 

@@ -36,6 +36,8 @@ class ChunkResult:
     row_depth: np.ndarray | None
     stage_ms: list = field(default_factory=list)
     launches: int = 0
+    calls: np.ndarray | None = None   # lib.CALL_DTYPE [n]: call records (Engine(device_calls=True)), else None
+    call_ms: float = 0.0              # device time of k_call
 
     @property
     def n_cand(self) -> int:
@@ -59,7 +61,8 @@ def _view(ptr, n, dtype, copy=True):
 class Engine:
     def __init__(self, device: int = 0, channels: int = 18, *, snp_min_af=P.SNP_MIN_AF, indel_min_af=P.INDEL_MIN_AF,
                  min_coverage=P.MIN_COVERAGE, min_mq=P.MIN_MQ, enable_padding=False, nn_impl=1,
-                 keep_tensor=False, keep_rows=False, enable_head_tail=False):
+                 keep_tensor=False, keep_rows=False, enable_head_tail=False, device_calls=False):
+        """device_calls: also decide each candidate's genotype on the GPU (ChunkResult.calls, format_vcf_rows)"""
         self.lib = L.load()
         if self.lib.c3r_abi_version() != 2:
             raise C3RError("ABI version mismatch")
@@ -86,6 +89,9 @@ class Engine:
                 self.ctx = C.c_void_p()
             raise C3RError("c3r_create: %s (rc=%d)" % (msg, rc))
         self._keep = {}
+        self._calls_of = {}                          # ticket -> records on when it was submitted
+        self.device_calls = False
+        self.set_device_calls(device_calls)
 
     # ------------------------------------------------------------------
     def _check(self, rc, what):
@@ -103,6 +109,11 @@ class Engine:
             self.close()
         except Exception:
             pass
+
+    def set_device_calls(self, on: bool):
+        """call records for the tickets submitted from now on (c3r_enable_calls)"""
+        self._check(self.lib.c3r_enable_calls(self.ctx, int(bool(on))), "c3r_enable_calls")
+        self.device_calls = bool(on)
 
     def set_weights(self, weights: dict):
         arrs = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in weights.items()}
@@ -142,6 +153,7 @@ class Engine:
             self._check(self.lib.c3r_submit_chunk(self.ctx, C.byref(rd), rp, ref_start1, rn,
                                                   region_start1, region_end1, C.byref(t)), "c3r_submit_chunk")
             self._keep[int(t.value)] = (arrs, ref)       # the call only queues the copies: inputs live until wait()
+            self._calls_of[int(t.value)] = self.device_calls
             return int(t.value)
         f = L.SiteFilter()
         keep = []
@@ -157,6 +169,7 @@ class Engine:
         self._check(self.lib.c3r_submit_chunk_filtered(self.ctx, C.byref(rd), rp, ref_start1, rn, region_start1,
                                                        region_end1, C.byref(f), C.byref(t)), "c3r_submit_chunk_filtered")
         self._keep[int(t.value)] = (arrs, ref, keep)
+        self._calls_of[int(t.value)] = self.device_calls
         return int(t.value)
 
     def wait(self, ticket: int, release: bool = True, copy: bool = True) -> ChunkResult:
@@ -165,10 +178,16 @@ class Engine:
         faults (copying 3-4 MB into fresh memory costs ~1.5 ms per chunk, more than half a device pass) - which
         stay valid until release(ticket); the ticket is then NOT released here."""
         r = L.Result()
+        calls_on = self._calls_of.pop(ticket, False)
         try:
             self._check(self.lib.c3r_wait(self.ctx, ticket, C.byref(r)), "c3r_wait")
         finally:
             self._keep.pop(ticket, None)
+        calls, call_ms = None, 0.0
+        if calls_on:
+            cp, cn, ms = C.c_void_p(), C.c_int64(0), C.c_float(0)
+            self._check(self.lib.c3r_wait_calls(self.ctx, ticket, C.byref(cp), C.byref(cn), C.byref(ms)), "c3r_wait_calls")
+            calls, call_ms = _view(cp.value, cn.value, L.CALL_DTYPE, copy), float(ms.value)
         n, Ct = int(r.n_cand), self.channels
         v = lambda ptr, cnt, dt: _view(ptr, cnt, dt, copy)
         alt_off = v(r.alt_off, n, np.int64)
@@ -182,13 +201,14 @@ class Engine:
             row_pos=v(r.row_pos, r.n_rows, np.int32) if r.row_pos else None,
             row_counts=v(r.row_counts, r.n_rows * Ct, np.int32).reshape(-1, Ct) if r.row_counts else None,
             row_depth=v(r.row_depth, r.n_rows, np.int32) if r.row_depth else None,
-            stage_ms=[float(x) for x in r.stage_ms], launches=int(r.kernel_launches))
+            stage_ms=[float(x) for x in r.stage_ms], launches=int(r.kernel_launches), calls=calls, call_ms=call_ms)
         if release and copy:
             self.lib.c3r_release(self.ctx, ticket)
         return out
 
     def release(self, ticket: int):
         self._keep.pop(ticket, None)
+        self._calls_of.pop(ticket, None)
         self.lib.c3r_release(self.ctx, ticket)
 
     def call_chunk(self, batch, ref, ref_start1, region_start1, region_end1, site_filter=None) -> ChunkResult:
@@ -267,28 +287,22 @@ class PinnedPool:
 
 
 # ---------------------------------------------------------------------- native decode
-def decode_vcf_rows(res: ChunkResult, batch: ReadBatch, ref: np.ndarray, ref_start1: int, contig: str,
-                    qual=P.QUAL_CUT_OFF, show_ref: bool = True, threads: int = 0) -> list:
-    """VCF data lines of every candidate through c3r_decode_vcf (csrc/decode.cpp): the native, multi-threaded
-    form of decoder.vcf_row over alt_info_strings / flank_strings."""
-    from .bam import reads_struct
-    lib = L.load()
-    keep = []
+def _result_struct(res: ChunkResult, keep: list):
+    """c3r_result over the arrays of res (kept alive in `keep`)"""
     r = L.Result()
     arrs = dict(pos=np.ascontiguousarray(res.pos, np.int32), depth=np.ascontiguousarray(res.depth, np.int32),
                 probs=np.ascontiguousarray(res.probs, np.float32), alt_off=np.ascontiguousarray(res.alt_off, np.int64),
                 alt_n=np.ascontiguousarray(res.alt_n, np.int32), alt=np.ascontiguousarray(res.alt))
+    keep.append(arrs)
     r.n_rows, r.n_cand = res.n_rows, res.n_cand
     for k, a in arrs.items():
         setattr(r, k, a.ctypes.data if a.size else None)
-    rd = reads_struct(batch, keep)
-    ref = np.ascontiguousarray(ref, np.uint8)
-    text, nb, nr = C.c_void_p(), C.c_int64(0), C.c_int64(0)
-    rc = lib.c3r_decode_vcf(C.byref(r), C.byref(rd), ref.ctypes.data, int(ref_start1), int(ref.size), contig.encode(),
-                            -1.0 if qual is None else float(qual), int(show_ref), threads,
-                            C.byref(text), C.byref(nb), C.byref(nr))
+    return r
+
+
+def _rows_of(lib, rc, text, nb, nr, what):
     if rc != 0:
-        raise C3RError("c3r_decode_vcf failed (rc=%d)" % rc)
+        raise C3RError("%s failed (rc=%d)" % (what, rc))
     try:
         s = C.string_at(text, nb.value).decode("ascii") if nb.value else ""
     finally:
@@ -296,6 +310,62 @@ def decode_vcf_rows(res: ChunkResult, batch: ReadBatch, ref: np.ndarray, ref_sta
     rows = s.split("\n")[:-1] if s else []
     assert len(rows) == nr.value
     return rows
+
+
+def decode_vcf_rows(res: ChunkResult, batch: ReadBatch, ref: np.ndarray, ref_start1: int, contig: str,
+                    qual=P.QUAL_CUT_OFF, show_ref: bool = True, threads: int = 0) -> list:
+    """VCF data lines of every candidate through c3r_decode_vcf (csrc/decode.cpp): the native, multi-threaded
+    form of decoder.vcf_row over alt_info_strings / flank_strings."""
+    from .bam import reads_struct
+    lib = L.load()
+    keep = []
+    r = _result_struct(res, keep)
+    rd = reads_struct(batch, keep)
+    ref = np.ascontiguousarray(ref, np.uint8)
+    text, nb, nr = C.c_void_p(), C.c_int64(0), C.c_int64(0)
+    rc = lib.c3r_decode_vcf(C.byref(r), C.byref(rd), ref.ctypes.data, int(ref_start1), int(ref.size), contig.encode(),
+                            -1.0 if qual is None else float(qual), int(show_ref), threads,
+                            C.byref(text), C.byref(nb), C.byref(nr))
+    return _rows_of(lib, rc, text, nb, nr, "c3r_decode_vcf")
+
+
+def format_vcf_rows(res: ChunkResult, batch: ReadBatch, ref: np.ndarray, ref_start1: int, contig: str,
+                    qual=P.QUAL_CUT_OFF, show_ref: bool = True, threads: int = 0, calls=None) -> list:
+    """decode_vcf_rows from call records (c3r_format_vcf): the same lines, with the genotype decision taken from
+    `calls` (default res.calls, made on the GPU by Engine(device_calls=True)) instead of made on the host."""
+    from .bam import reads_struct
+    calls = res.calls if calls is None else calls
+    if calls is None:
+        raise C3RError("format_vcf_rows needs call records: Engine(device_calls=True) or decide_calls()")
+    calls = np.ascontiguousarray(calls, L.CALL_DTYPE)
+    if calls.shape[0] != res.n_cand:
+        raise C3RError("%d call records for %d candidates" % (calls.shape[0], res.n_cand))
+    lib = L.load()
+    keep = []
+    r = _result_struct(res, keep)
+    rd = reads_struct(batch, keep)
+    ref = np.ascontiguousarray(ref, np.uint8)
+    text, nb, nr = C.c_void_p(), C.c_int64(0), C.c_int64(0)
+    rc = lib.c3r_format_vcf(C.byref(r), calls.ctypes.data if calls.size else None, C.byref(rd), ref.ctypes.data,
+                            int(ref_start1), int(ref.size), contig.encode(), -1.0 if qual is None else float(qual),
+                            int(show_ref), threads, C.byref(text), C.byref(nb), C.byref(nr))
+    return _rows_of(lib, rc, text, nb, nr, "c3r_format_vcf")
+
+
+def decide_calls(res: ChunkResult, batch: ReadBatch, ref: np.ndarray, ref_start1: int) -> np.ndarray:
+    """the call records k_call makes, by the same code on the host (c3r_debug_decide_calls; no GPU needed)"""
+    from .bam import reads_struct
+    lib = L.load()
+    keep = []
+    r = _result_struct(res, keep)
+    rd = reads_struct(batch, keep)
+    ref = np.ascontiguousarray(ref, np.uint8)
+    out = np.zeros(res.n_cand, L.CALL_DTYPE)
+    rc = lib.c3r_debug_decide_calls(C.byref(r), C.byref(rd), ref.ctypes.data, int(ref_start1), int(ref.size),
+                                    out.ctypes.data if out.size else None)
+    if rc != 0:
+        raise C3RError("c3r_debug_decide_calls failed (rc=%d)" % rc)
+    return out
 
 
 # ---------------------------------------------------------------------- host formatting

@@ -4,6 +4,8 @@ Fails loudly when the library is missing: there is no CPU or PyTorch fallback.""
 import ctypes as C
 import os
 
+import numpy as np
+
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("C3R_LIB") or os.path.join(HERE, "libc3r_b200.so")   # C3R_LIB: an experimental build
 
@@ -42,6 +44,31 @@ class Result(C.Structure):
                 ("row_depth", C.c_void_p), ("stage_ms", C.c_float * 8), ("kernel_launches", C.c_int32)]
 
 
+class CallAllele(C.Structure):
+    """c3r_call_allele (include/c3r_b200.h)"""
+    _fields_ = [("first", C.c_uint8), ("reserved", C.c_uint8), ("ins_len", C.c_uint16), ("ins_seq_off", C.c_uint32),
+                ("suffix_from", C.c_uint16), ("reserved2", C.c_uint16)]
+
+
+class Call(C.Structure):
+    """c3r_call (include/c3r_b200.h): the call record of one candidate"""
+    _fields_ = [("prob", C.c_float), ("ref_count", C.c_int32), ("support", C.c_int32), ("ad", C.c_int32 * 2),
+                ("family", C.c_uint8), ("gt", C.c_uint8), ("n_ad", C.c_uint8), ("n_alt", C.c_uint8),
+                ("ref_first", C.c_uint8), ("reserved", C.c_uint8), ("ref_len", C.c_uint16), ("retries", C.c_uint16),
+                ("flags", C.c_uint16), ("alt", CallAllele * 2)]
+
+
+CALL_ALLELE_DTYPE = np.dtype([("first", "u1"), ("reserved", "u1"), ("ins_len", "<u2"), ("ins_seq_off", "<u4"),
+                              ("suffix_from", "<u2"), ("reserved2", "<u2")])
+# numpy view of an array of c3r_call
+CALL_DTYPE = np.dtype([("prob", "<f4"), ("ref_count", "<i4"), ("support", "<i4"), ("ad", "<i4", (2,)),
+                       ("family", "u1"), ("gt", "u1"), ("n_ad", "u1"), ("n_alt", "u1"),
+                       ("ref_first", "u1"), ("reserved", "u1"), ("ref_len", "<u2"), ("retries", "<u2"),
+                       ("flags", "<u2"), ("alt", CALL_ALLELE_DTYPE, (2,))])
+CALL_NO_ROW = 0xFF
+GT_TEXT = ("0/0", "1/1", "0/1", "1/2", "None")
+
+
 class SiteFilter(C.Structure):
     """c3r_site_filter (include/c3r_b200.h)"""
     _fields_ = [("pileup_bed", C.c_void_p), ("n_pileup_bed", C.c_int64),
@@ -54,7 +81,8 @@ EXPORTS = ["c3r_abi_version", "c3r_default_params", "c3r_create", "c3r_destroy",
            "c3r_bam_open", "c3r_bam_close", "c3r_bam_error", "c3r_bam_n_ref", "c3r_bam_ref_name", "c3r_bam_ref_len",
            "c3r_bam_header_text", "c3r_bam_idxstats", "c3r_bam_fetch", "c3r_bam_write",
            "c3r_decode_vcf", "c3r_free_text", "c3r_debug_format_fixed", "c3r_vcf_write_bgzf",
-           "c3r_host_alloc", "c3r_host_free", "c3r_fasta_fetch"]
+           "c3r_host_alloc", "c3r_host_free", "c3r_fasta_fetch",
+           "c3r_enable_calls", "c3r_wait_calls", "c3r_format_vcf", "c3r_debug_decide_calls"]
 
 _lib = None
 
@@ -108,6 +136,14 @@ def load():
     lib.c3r_decode_vcf.argtypes = [C.POINTER(Result), C.POINTER(Reads), C.c_void_p, C.c_int64, C.c_int64, C.c_char_p,
                                    C.c_double, C.c_int, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_int64),
                                    C.POINTER(C.c_int64)]
+    lib.c3r_enable_calls.argtypes = [C.c_void_p, C.c_int]
+    lib.c3r_wait_calls.argtypes = [C.c_void_p, C.c_int64, C.POINTER(C.c_void_p), C.POINTER(C.c_int64),
+                                   C.POINTER(C.c_float)]
+    lib.c3r_format_vcf.argtypes = [C.POINTER(Result), C.c_void_p, C.POINTER(Reads), C.c_void_p, C.c_int64, C.c_int64,
+                                   C.c_char_p, C.c_double, C.c_int, C.c_int, C.POINTER(C.c_void_p),
+                                   C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
+    lib.c3r_debug_decide_calls.argtypes = [C.POINTER(Result), C.POINTER(Reads), C.c_void_p, C.c_int64, C.c_int64,
+                                           C.c_void_p]
     lib.c3r_host_alloc.argtypes = [C.POINTER(C.c_void_p), C.c_int64]
     lib.c3r_host_free.argtypes = [C.c_void_p]
     lib.c3r_host_free.restype = None

@@ -52,14 +52,17 @@ def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, wo
         snp_min_af=P.SNP_MIN_AF, indel_min_af=P.INDEL_MIN_AF, min_coverage=P.MIN_COVERAGE, min_mq=P.MIN_MQ,
         qual=P.QUAL_CUT_OFF, sample_name="SAMPLE", gather=None, stats=None, bed_fn=None, vcf_fn=None, head_tail=False,
         merge_qual=None, show_ref=True, rediportal_fn=None, rediportal_tags=None, output_no_tagging=None,
-        compress_vcf=False, engine=None, loader_threads=2, native_threads=0, merge=True, cmdline=None):
+        compress_vcf=False, engine=None, loader_threads=2, native_threads=0, merge=True, cmdline=None,
+        device_calls=False):
     """merge_qual / show_ref / rediportal_*: the options of the merge stage (sharder.sort_vcf = sort_vcf_from of the
     reference); the defaults keep every row as the chunks produced it.  engine: an Engine to reuse (its parameters and
     weights are then the caller's business); loader_threads: BAM / FASTA readers working ahead of the GPU;
     native_threads: threads of each BGZF inflate and of the row decoder (0 = all cores - give every rank its share
-    when several ranks run on one host)."""
+    when several ranks run on one host).  device_calls: decide the genotypes on the GPU (call records, k_call) and
+    leave only the formatting to the decoder threads (c3r_format_vcf); the rows are the same.  A caller's engine
+    gets its own device_calls setting back when the run ends."""
     from .bam import BamFile
-    from .engine import Engine, PinnedPool, decode_vcf_rows
+    from .engine import Engine, PinnedPool, decode_vcf_rows, format_vcf_rows
     fai = fasta.read_fai(ref_fn)
     bf = BamFile(bam_fn)
     idx = {n: m for n, _, m, _ in bf.idxstats()}
@@ -72,15 +75,19 @@ def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, wo
     mine = [i for i in range(len(shards)) if owner[i] == rank]
     C = P.CHANNEL_SIZE + (P.PHASED_CHANNEL_SIZE if phased else 0)
     eng = engine
+    calls_before = eng.device_calls if eng is not None else None
     if eng is None:
         eng = Engine(device, C, snp_min_af=snp_min_af, indel_min_af=indel_min_af, min_coverage=min_coverage,
-                     min_mq=min_mq, enable_padding=padding, enable_head_tail=head_tail)
+                     min_mq=min_mq, enable_padding=padding, enable_head_tail=head_tail, device_calls=device_calls)
         eng.set_weights(W.load(chkpnt_fn))
+    elif eng.device_calls != bool(device_calls):
+        eng.set_device_calls(device_calls)
     t0 = time.time()
     rows_of = {}
     n_cand = 0
     # host seconds per stage of this rank's loop (the GPU works under all of them but `wait`)
     tm = dict(fetch=0.0, ref=0.0, submit=0.0, wait=0.0, decode=0.0)
+    call_ms = 0.0                                    # device time of k_call (device_calls)
 
     import threading
     tls = threading.local()
@@ -143,7 +150,8 @@ def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, wo
 
     def decode(res, pbatch, pref, prs1, pname, pbuf):
         t = time.time()
-        rows = decode_vcf_rows(res, pbatch, pref, prs1, pname, qual=qual, threads=dec_threads)
+        rows = (format_vcf_rows if device_calls else decode_vcf_rows)(res, pbatch, pref, prs1, pname, qual=qual,
+                                                                      threads=dec_threads)
         tm["decode"] += time.time() - t
         pool.put(pbuf)                               # the reference window is free again
         return rows
@@ -186,6 +194,7 @@ def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, wo
             res = eng.wait(ticket, copy=False)       # arrays over the library's pinned buffers, no copies
             tm["wait"] += time.time() - t
             n_cand += res.n_cand
+            call_ms += res.call_ms
             decoding.append((j, ticket, dec.submit(decode, res, pbatch, pref, prs1, pname, ppbuf)))
         retire(False)
         pending = nxt
@@ -197,12 +206,14 @@ def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, wo
         pool.close()
         eng._ref_pool = None
         eng.close()
+    elif eng.device_calls != calls_before:
+        eng.set_device_calls(calls_before)
     bf.close()
     for r in readers:
         r.close()
     if stats is not None:
         stats.update(shards=len(mine), candidates=n_cand, seconds=time.time() - t0, host_seconds=tm, submit_ms=submit_ms,
-                     cost=sum(costs[i] for i in mine), total_shards=len(shards))
+                     cost=sum(costs[i] for i in mine), total_shards=len(shards), call_device_ms=call_ms)
     if not merge:                                    # the caller only wants this rank's loop (timing passes)
         return None
     if world > 1:
@@ -277,6 +288,8 @@ def main(argv=None):
     ap.add_argument("--enable_phasing_model", action="store_true")
     ap.add_argument("--enable_padding_in_splice_junction_regions", action="store_true")
     ap.add_argument("--enable_variant_calling_at_sequence_head_and_tail", action="store_true")
+    ap.add_argument("--device_calls", action="store_true",
+                    help="decide the genotypes on the GPU and only format the rows on the host (same output)")
     a = ap.parse_args(argv)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -300,7 +313,7 @@ def main(argv=None):
         compress_vcf=a.compress_vcf,
         cmdline=" ".join(sys.argv) if argv is None else " ".join(["run_chunks"] + list(argv)),
         sample_name=a.sampleName, stats=stats, bed_fn=a.bed_fn, vcf_fn=a.genotyping_mode_vcf_fn,
-        head_tail=a.enable_variant_calling_at_sequence_head_and_tail)
+        head_tail=a.enable_variant_calling_at_sequence_head_and_tail, device_calls=a.device_calls)
     print("[rank %d] %d shards, %d candidates in %.2f s" % (rank, stats["shards"], stats["candidates"], stats["seconds"]),
           file=sys.stderr)
     if world > 1:

@@ -221,6 +221,85 @@ void c3r_free_text(char* text);
 int c3r_debug_format_fixed(double x, int decimals, char* out);
 
 /* ------------------------------------------------------------------------------------------
+ * Call records: the genotype decision of c3r_decode_vcf (output_from and the allele counts of output_with) made
+ * on the GPU, one fixed-size record per candidate (csrc/call.cuh, kernel k_call).  Only QUAL (a log), AF (a
+ * division) and the text are left to the host: c3r_format_vcf turns records into the lines c3r_decode_vcf prints.
+ *
+ * An allele's text is `first`, then ins_len inserted bases from c3r_reads.seq (nt16, base offset ins_seq_off),
+ * then REF's letters [suffix_from, ref_len).  REF's letter 0 is ref_first (the centre base; for a reference call
+ * the A/C/G/T it stands for), letters 1.. are the reference bases after the candidate, ref[pos - ref_start1 + 1 ..].
+ * Every ALT the decision makes has this form: SNP bases, insertion keys, INSDEL's ins + REF[1:], HET_ACGT_DEL's
+ * b + REF[1:] and HET_DELDEL's REF[0] + REF[1+len:]. */
+typedef struct {
+    uint8_t first;
+    uint8_t reserved;
+    uint16_t ins_len;
+    uint32_t ins_seq_off;
+    uint16_t suffix_from;
+    uint16_t reserved2;
+} c3r_call_allele;
+
+#define C3R_CALL_NO_ROW 0xFF   /* c3r_call.family of a candidate that gives no VCF row */
+
+/* c3r_call.gt: 0 "0/0", 1 "1/1", 2 "0/1", 3 "1/2", 4 "None" */
+typedef struct {
+    float prob;                /* probability of the call, the float32 QUAL is computed from            */
+    int32_t ref_count;         /* AD's first number (reads of the reference allele)                     */
+    int32_t support;           /* AF's numerator                                                        */
+    int32_t ad[2];             /* AD's numbers after ref_count, n_ad of them                            */
+    uint8_t family;            /* outcome family the call came from (0 = reference call, 1 HOMO_SNP, 2 HET_SNP,
+                                  3 HOMO_INS, 4 HET_ACGT_INS, 5 HET_INSINS, 6 HOMO_DEL, 7 HET_ACGT_DEL,
+                                  8 HET_DELDEL, 9 INSDEL), C3R_CALL_NO_ROW: no row                        */
+    uint8_t gt;
+    uint8_t n_ad;
+    uint8_t n_alt;             /* ALT alleles, comma separated; 0: ALT is "."                           */
+    uint8_t ref_first;
+    uint8_t reserved;
+    uint16_t ref_len;
+    uint16_t retries;          /* diagnostics: bit C3R_RETRY_* of every retry branch the decision passed */
+    uint16_t flags;            /* diagnostics: bit f of every family flagged by the last pass (its best member ties
+                                  the call's probability); AD follows the first flagged family in output_with's order,
+                                  which may differ from `family`                                              */
+    c3r_call_allele alt[2];
+} c3r_call;
+
+/* c3r_call.retries: the branches of output_from's retry loop that zero a family member and try again */
+enum {
+    C3R_RETRY_HOMO_SNP_NO_X = 0,      /* no X allele                                        */
+    C3R_RETRY_HOMO_SNP_IS_REF,        /* the chosen base is the centre base                 */
+    C3R_RETRY_HET_SNP_LT2_X,          /* neither genotype base is the centre: < 2 X alleles */
+    C3R_RETRY_HET_SNP_NO_X,
+    C3R_RETRY_HET_SNP_IS_REF,
+    C3R_RETRY_HOMO_INS_NO_I,          /* no insertion key of 1..50 letters                  */
+    C3R_RETRY_HET_ACGT_INS_NO_I,
+    C3R_RETRY_HET_ACGT_INS_NO_X,
+    C3R_RETRY_HET_INSINS_LT2_I,
+    C3R_RETRY_HET_INSINS_SAME,        /* the two keys are equal (distinct dict keys: never)   */
+    C3R_RETRY_HOMO_DEL_NO_D,
+    C3R_RETRY_HET_ACGT_DEL_NO_D,
+    C3R_RETRY_HET_DELDEL_LT2_D,
+    C3R_RETRY_HET_DELDEL_SAME,        /* the two ALTs coincide (distinct lengths: never)    */
+    C3R_RETRY_INSDEL_NO_I_OR_D
+};
+
+/* Make call records for the tickets submitted after this call (on != 0) or stop (0; the default).  With records
+ * off nothing about a ticket changes: the same kernels, copies and results. */
+int c3r_enable_calls(c3r_ctx* ctx, int on);
+/* The records of a ticket submitted with records on, one per candidate of its c3r_result, in pinned library
+ * memory valid until c3r_release.  Call after c3r_wait.  device_ms (may be NULL): device time of k_call.
+ * C3R_ERR_STATE when records were off for the ticket or c3r_wait has not returned it. */
+int c3r_wait_calls(c3r_ctx* ctx, c3r_ticket ticket, const c3r_call** calls, int64_t* n, float* device_ms);
+/* c3r_decode_vcf from call records: the same arguments and the same text, with the decision read from
+ * calls[n_cand] instead of made.  C3R_ERR_ARG (and no text) when a record cannot be printed: malformed, or made
+ * over another reference window or read pool than the ones given. */
+int c3r_format_vcf(const c3r_result* res, const c3r_call* calls, const c3r_reads* reads, const uint8_t* ref,
+                   int64_t ref_start1, int64_t ref_len, const char* contig, double qual_cut, int show_ref,
+                   int n_threads, char** text, int64_t* n_bytes, int64_t* n_rows);
+/* test hook: the records k_call makes, by the same code on the host (no GPU needed), into out[res->n_cand] */
+int c3r_debug_decide_calls(const c3r_result* res, const c3r_reads* reads, const uint8_t* ref, int64_t ref_start1,
+                           int64_t ref_len, c3r_call* out);
+
+/* ------------------------------------------------------------------------------------------
  * BAM / BGZF / BAI input (host side, zlib; csrc/bam_io.cpp).  The reference reads the BAM only
  * through external samtools: `samtools mpileup BAM -r ctg:s-e ...` (src/create_tensor_pileup.py:
  * 436-451) and `samtools idxstats BAM` (run_clair3_rna:187).  c3r_bam_fetch is the index fetch
