@@ -1,10 +1,13 @@
 // The genotype decision of one candidate as a fixed-size call record (c3r_call, include/c3r_b200.h), in code that
-// compiles for the host (c3r_debug_decide_calls, csrc/decode.cpp) and for sm_100a (k_call, csrc/c3r_abi.cu).
+// compiles for the host (c3r_decode_vcf, c3r_debug_decide_calls, csrc/decode.cpp) and for sm_100a (k_call,
+// csrc/c3r_abi.cu).
 //
-// It restates decide() and the allele-count part of vcf_row() in csrc/decode.cpp statement by statement, quirks
-// included: a failed family zeroes its probability and retries without clearing REF / ALT, find_alt_base ranks the
-// X alleles by descending count (ties stable) and falls back when the wanted base trails by >= 9 reads, indel dicts
-// keep a repeated key at its first position with its last value, keys longer than MAX_INDEL are cut, SNP counts are
+// It is the library's one native genotype decision: c3r_decode_vcf and k_call both call decide_call.  It restates
+// decide() and the allele-count part of vcf_row() in clair3_rna_b200/decoder.py - output_from and output_with of
+// the reference's call_variants.py (:684-1020 and :1117-1392) - statement by statement, quirks included: a failed
+// family zeroes its probability and retries without clearing REF / ALT, find_alt_base ranks the X alleles by
+// descending count (ties stable) and falls back when the wanted base trails by >= 9 reads, indel dicts keep a
+// repeated key at its first position with its last value, keys longer than MAX_INDEL are cut, SNP counts are
 // cumulative, deletion counts are matched by length (first_len_match), and a candidate whose centre base is outside
 // the IUPAC table gives no row.
 //
@@ -12,11 +15,12 @@
 // keys are compared by content - insertion keys by their sequence nibbles, deletion keys by their length, because
 // every deletion key of a candidate is a prefix of the same reference bases (a key cut at the window end is shorter).
 // The only arithmetic is IEEE float32 products and comparisons, so the device's record equals the host's bit for bit.
-// Everything inexact (QUAL's log, AF's division) and all text stay in the host formatter (c3r_format_vcf).
+// Everything inexact (QUAL's log, AF's division) and all text stay in the host formatter (put_call, decode.cpp).
 //
-// Two facts the record relies on, both true of the library's inputs: reference bytes and allele letters are never
-// ',' (a ',' in the text is always the separator of two alleles), and allele counts are at most the 8000-read depth
-// cap, so sums of two of them fit int32.
+// Three facts the record relies on, all true of the library's inputs: reference bytes and allele letters are never
+// ',' (a ',' in the text is always the separator of two alleles), allele counts are at most the 8000-read depth
+// cap, so sums of two of them fit int32, and a candidate has at most one X allele per base (k_altinfo), so ranking
+// X entries is ranking decoder.py's dict of X keys.
 #pragma once
 #include <stdint.h>
 
@@ -51,7 +55,7 @@ struct CallIn {
     const uint8_t* ref;         // the reference window
     int64_t ref_len;
     int64_t p0;                 // candidate offset in the window (pos - ref_start1)
-    const uint8_t* seq;         // nt16 pool of the reads; NULL: an insertion key is its base alone (like decode.cpp)
+    const uint8_t* seq;         // nt16 pool of the reads; NULL: an insertion key is its base alone
 };
 
 C3R_HD char base2acgt(char c) {                     // shared/utils.py:41-44; 0 when the base is not in the table
@@ -207,7 +211,7 @@ C3R_HD bool al_eq_ins_key(const CallIn& c, const Dec& D, const Al& a, int len, c
     return true;
 }
 
-// ---- output_from (decode.cpp decide())
+// ---- output_from (call_variants.py:684-1020, decoder.py decide())
 C3R_HD int fam_index_of(const float* v, int f, float x) {
     for (int j = fam_off(f); j < fam_off(f + 1); ++j) if (v[j] == x) return j - fam_off(f);
     return -1;
@@ -361,7 +365,7 @@ C3R_HD void decide(const CallIn& c, char center, Dec& D) {
     D.prob = best;
 }
 
-// ---- vcf_row(): which row, its GT and its allele counts
+// ---- output_with (call_variants.py:1117-1392, decoder.py vcf_row()): which row, its GT and its allele counts
 C3R_HD int32_t snp_count(const CallIn& c, char b) {      // dict_get(snp, b): last X allele of that base
     int32_t v = 0;
     for (int k = 0; k < c.n; ++k) if (c.e[k].kind == 'X' && (char)c.e[k].base == b) v = c.e[k].count;

@@ -237,6 +237,12 @@ def _iupac_to_n(s: str) -> str:
 def vcf_row(contig: str, pos: int, ref33: str, alt_info: str, probs, qual_for_pass=P.QUAL_CUT_OFF, show_ref=True):
     """output_with: one VCF data line, or None when the reference prints nothing."""
     depth, alt = parse_alt_info(alt_info)
+    return vcf_row_from(contig, pos, ref33, depth, alt, probs, qual_for_pass, show_ref)
+
+
+def vcf_row_from(contig: str, pos: int, ref33: str, depth: int, alt: dict, probs, qual_for_pass=P.QUAL_CUT_OFF,
+                 show_ref=True):
+    """vcf_row on the parsed alt_info: depth and the {key: count} dict"""
     f, ref_base, alt_base, prob = decide(ref33, probs, alt)
     is_ref = f["ref"]
     if (not show_ref and is_ref) or (not is_ref and ref_base == alt_base):

@@ -369,34 +369,41 @@ def decide_calls(res: ChunkResult, batch: ReadBatch, ref: np.ndarray, ref_start1
 
 
 # ---------------------------------------------------------------------- host formatting
-def alt_info_strings(res: ChunkResult, batch: ReadBatch, ref: np.ndarray, ref_start1: int) -> list:
-    """alt_info text of each candidate exactly as the reference's producer prints it
-    (/root/reference/src/create_tensor_pileup.py:595-596): "<depth>-KEY n KEY n ..."."""
+def alt_items(res: ChunkResult, batch: ReadBatch, ref: np.ndarray, ref_start1: int) -> list:
+    """each candidate's alt_info as [(KEY, count)] in table order; a deletion key is the reference bases after the
+    candidate that lie in the window"""
     out = []
     seq = batch.seq
     refb = ref.tobytes() if isinstance(ref, np.ndarray) else bytes(ref)
+    alt = res.alt.tolist()                          # ALT_DTYPE rows as tuples
     for i in range(res.n_cand):
         a, n = int(res.alt_off[i]), int(res.alt_n[i])
         items = []
         p0 = int(res.pos[i]) - ref_start1           # offset of the candidate in ref
-        for e in res.alt[a:a + n]:
-            kind = chr(int(e["kind"]))
+        for kind, base, ln, count, q, _ in alt[a:a + n]:
+            kind = chr(kind)
             if kind == 'X' or kind == 'R':
-                key = kind + chr(int(e["base"]))
+                key = kind + chr(base)
             elif kind == 'I':
-                q, ln = int(e["seq_off"]), int(e["len"])
                 by = seq[q // 2: (q + ln + 1) // 2 + 1]
                 codes = np.empty(by.size * 2, np.uint8)
                 codes[0::2] = by >> 4
                 codes[1::2] = by & 15
                 s = codes[q & 1: (q & 1) + ln]
-                key = 'I' + chr(int(e["base"])) + "".join(NT16[c] for c in s)
+                key = 'I' + chr(base) + "".join(NT16[c] for c in s)
             else:
-                ln = int(e["len"])
-                key = 'D' + refb[p0 + 1: p0 + 1 + ln].decode("ascii")
-            items.append("%s %d" % (key, int(e["count"])))
-        out.append("%d-%s" % (int(res.depth[i]), " ".join(items)))
+                lo, hi = max(0, p0 + 1), min(len(refb), p0 + 1 + ln)
+                key = 'D' + refb[lo:max(lo, hi)].decode("ascii")
+            items.append((key, count))
+        out.append(items)
     return out
+
+
+def alt_info_strings(res: ChunkResult, batch: ReadBatch, ref: np.ndarray, ref_start1: int) -> list:
+    """alt_info text of each candidate exactly as the reference's producer prints it
+    (/root/reference/src/create_tensor_pileup.py:595-596): "<depth>-KEY n KEY n ..."."""
+    return ["%d-%s" % (int(d), " ".join("%s %d" % kv for kv in items))
+            for d, items in zip(res.depth, alt_items(res, batch, ref, ref_start1))]
 
 
 def flank_strings(res: ChunkResult, ref: np.ndarray, ref_start1: int) -> list:

@@ -205,7 +205,8 @@ int c3r_fasta_fetch(const char* path, int64_t contig_len, int64_t offset, int64_
 /* ------------------------------------------------------------------------------------------
  * Probabilities + allele table -> VCF data lines (host, multi-threaded; csrc/decode.cpp).  Replaces the
  * per-candidate Python of output_with / output_from (clair3_rna/call_variants.py:684-1392, options as
- * forwarded by call_var_bam.py:247-272: --pileup --showRef, add_indel_length False).  One line per
+ * forwarded by call_var_bam.py:247-272: --pileup --showRef, add_indel_length False): each candidate's call
+ * record is made on the host by the code k_call runs (csrc/call.cuh) and printed like c3r_format_vcf.  One line per
  * candidate of `res` in order ("CHROM POS . REF ALT QUAL FILTER . GT:GQ:DP:AD:AF ..."), candidates whose
  * centre reference base is outside the IUPAC table are skipped (clair3_rna/utils.py:113).
  *   reads: the records `res` was computed from (inserted bases are read from reads->seq)

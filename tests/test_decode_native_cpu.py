@@ -1,5 +1,6 @@
-"""c3r_decode_vcf (csrc/decode.cpp, native multi-threaded A7) against the Python decoder and against the
-rows the reference's own output_with printed (tests/golden/decoder_*.npz)."""
+"""c3r_decode_vcf (csrc/decode.cpp: the decision of csrc/call.cuh on the host and its row printer, native
+multi-threaded A7) against the Python decoder and against the rows the reference's own output_with printed
+(tests/golden/decoder_*.npz)."""
 import os
 
 import numpy as np
