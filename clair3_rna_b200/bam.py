@@ -79,16 +79,58 @@ class BamFile:
         rc = self.lib.c3r_bam_fetch(self.h, self._tid[contig], int(start1), int(end1), C.byref(r))
         if rc != 0:
             raise RuntimeError("c3r_bam_fetch: " + self.lib.c3r_bam_error(self.h).decode())
+        return reads_from(contig, r)
 
-        def arr(ptr, n, dt):
-            if n == 0 or not ptr:
-                return np.zeros(0, dt)
-            return np.ctypeslib.as_array(C.cast(ptr, C.POINTER(np.ctypeslib.as_ctypes_type(dt))), shape=(n,)).copy()
+    def fetch_raw(self, contig: str, start1: int, end1: int, buf=None) -> RawChunk:
+        """fetch() without the inflate and the record walk: the index query and the compressed blocks of the region
+        read into `buf` (a uint8 array, e.g. from engine.PinnedPool); a new array when buf is None or too small"""
+        if contig not in self._tid:
+            raise KeyError("contig %s not in the BAM header" % contig)
+        r = L.BamRaw()
+        tid = self._tid[contig]
+        cap = 0 if buf is None else int(buf.size)
+        rc = self.lib.c3r_bam_fetch_raw(self.h, tid, int(start1), int(end1), buf.ctypes.data if cap else None, cap, C.byref(r))
+        if rc == -4:                                 # C3R_ERR_CAPACITY: r.n_bytes is the size needed
+            buf = np.empty(max(1, int(r.n_bytes)), np.uint8)
+            rc = self.lib.c3r_bam_fetch_raw(self.h, tid, int(start1), int(end1), buf.ctypes.data, buf.size, C.byref(r))
+        if rc != 0:
+            raise RuntimeError("c3r_bam_fetch_raw: " + self.lib.c3r_bam_error(self.h).decode())
+        blocks = _table(r.blocks, int(r.n_blocks), L.BgzfBlock)
+        windows = _table(r.windows, int(r.n_windows), L.BamWindow)
+        r.blocks = C.addressof(blocks) if r.n_blocks else None
+        r.windows = C.addressof(windows) if r.n_windows else None
+        return RawChunk(contig, r, buf, blocks, windows)
 
-        R, O, S = int(r.n_reads), int(r.n_ops), int(r.n_seq_bytes)
-        return ReadBatch(contig, arr(r.pos, R, np.int32), arr(r.flag, R, np.uint16), arr(r.mapq, R, np.uint8),
-                         arr(r.hp, R, np.uint8), arr(r.cigar_off, R + 1, np.int32), arr(r.cigar, O, np.uint32),
-                         arr(r.seq_off, R + 1, np.int64), arr(r.seq, S, np.uint8))
+
+def reads_from(contig: str, r: L.Reads, copy: bool = True) -> ReadBatch:
+    """ReadBatch over a c3r_reads; copy=False aliases the memory behind it"""
+    def arr(ptr, n, dt):
+        if n == 0 or not ptr:
+            return np.zeros(0, dt)
+        a = np.ctypeslib.as_array(C.cast(ptr, C.POINTER(np.ctypeslib.as_ctypes_type(dt))), shape=(n,))
+        return a.copy() if copy else a
+
+    R, O, S = int(r.n_reads), int(r.n_ops), int(r.n_seq_bytes)
+    return ReadBatch(contig, arr(r.pos, R, np.int32), arr(r.flag, R, np.uint16), arr(r.mapq, R, np.uint8),
+                     arr(r.hp, R, np.uint8), arr(r.cigar_off, R + 1, np.int32), arr(r.cigar, O, np.uint32),
+                     arr(r.seq_off, R + 1, np.int64), arr(r.seq, S, np.uint8))
+
+
+class RawChunk:
+    """The compressed blocks of a region fetch and their tables (c3r_bam_fetch_raw), ready for Engine.submit_bam:
+    `data` holds the bytes (a caller's buffer, possibly page-locked), `blocks` / `windows` are private copies of the
+    handle's tables, `raw` the c3r_bam_raw over all three.  Keep it unchanged until the ticket is waited for."""
+
+    def __init__(self, contig, raw, data, blocks, windows):
+        self.contig, self.raw, self.data, self.blocks, self.windows = contig, raw, data, blocks, windows
+
+    @property
+    def n_bytes(self) -> int:
+        return int(self.raw.n_bytes)
+
+
+def _table(ptr, n, ctype):
+    return (ctype * n).from_buffer_copy((ctype * n).from_address(ptr)) if n > 0 and ptr else (ctype * max(n, 0))()
 
 
 def write_bam(path: str, contigs: list, batches: dict, level: int = -1, header_text: str | None = None) -> None:

@@ -22,11 +22,13 @@
 #include <zlib.h>
 
 #include "../../include/c3r_b200.h"
+#include "bam_rec.cuh"
+#include "bgzf.cuh"
 
 namespace {
 
-inline uint16_t rd16(const uint8_t* p) { return (uint16_t)(p[0] | (p[1] << 8)); }
-inline uint32_t rd32(const uint8_t* p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24); }
+using c3rbam::rd16;
+using c3rbam::rd32;
 inline uint64_t rd64(const uint8_t* p) { return (uint64_t)rd32(p) | ((uint64_t)rd32(p + 4) << 32); }
 inline void wr16(std::vector<uint8_t>& v, uint16_t x) { v.push_back(x & 0xff); v.push_back(x >> 8); }
 inline void wr32(std::vector<uint8_t>& v, uint32_t x) { for (int i = 0; i < 4; ++i) v.push_back((x >> (8 * i)) & 0xff); }
@@ -84,6 +86,9 @@ struct c3r_bam {
     std::vector<int64_t> seq_off;
     // scratch
     std::vector<uint8_t> cbuf, ubuf;
+    // tables of the last raw fetch (c3r_bam_fetch_raw)
+    std::vector<c3r_bgzf_block> raw_blocks;
+    std::vector<c3r_bam_window> raw_windows;
 };
 
 namespace {
@@ -124,40 +129,64 @@ uint32_t bgzf_block_size(const uint8_t* p, size_t avail) {
     return 0;
 }
 
-// read [coff, coff + n) of the file into h->cbuf
-bool read_range(c3r_bam* h, uint64_t coff, uint64_t n) {
-    h->cbuf.resize(n);
-    if (fseeko(h->fp, (off_t)coff, SEEK_SET) != 0) return false;
-    return fread(h->cbuf.data(), 1, n, h->fp) == n;
+// the messages of c3rbgzf::FetchErr
+std::string fetch_err_text(const c3r_bam* h, int code) {
+    switch (code) {
+        case c3rbgzf::FE_INFLATE: return "BGZF inflate/CRC failure in " + h->path;
+        case c3rbgzf::FE_HEADER: return "corrupt BGZF block header in " + h->path;
+        case c3rbgzf::FE_BIG_BLOCK: return "BGZF block larger than 64 KiB";
+        case c3rbgzf::FE_SHORT_READ: return "short read from " + h->path;
+        case c3rbgzf::FE_CROSS: return "record crosses the end of an index chunk";
+        case c3rbgzf::FE_MALFORMED: return "malformed BAM record";
+        default: return "malformed aux data in a BAM record";
+    }
 }
 
-// Inflate the blocks starting at compressed offset `cbeg` up to (and including) the block that
-// contains compressed offset `cend_block` (or to EOF when cend_block == UINT64_MAX).  Fills h->ubuf;
-// `blocks` gets the block table.
-int inflate_range(c3r_bam* h, uint64_t cbeg, uint64_t cend_block, std::vector<Block>& blocks) {
+// Bytes read for the blocks starting at compressed offset `cbeg` up to (and including) the block that contains
+// compressed offset `cend_block` (or to EOF when cend_block == UINT64_MAX): one block more than the range, so that
+// the last block is whole.  0 when cbeg is at or past the end of the file.
+uint64_t range_bytes(const c3r_bam* h, uint64_t cbeg, uint64_t cend_block) {
+    if (cbeg >= h->file_size) return 0;
+    const uint64_t last = cend_block == UINT64_MAX ? h->file_size : std::min<uint64_t>(h->file_size, cend_block + 0x10000);
+    return last - cbeg;
+}
+
+// Reads range_bytes(cbeg, cend_block) bytes of the file into `dst` and cuts them into the block table (`blocks`,
+// uoff relative to the range, `*ubytes` their inflated size).  Returns a c3rbgzf::FetchErr.  The one reading of a
+// fetch's blocks: the host fetch inflates what it returns, the raw fetch hands it to the device.
+int read_blocks(c3r_bam* h, uint64_t cbeg, uint64_t cend_block, uint8_t* dst, std::vector<Block>& blocks, uint64_t* ubytes) {
     blocks.clear();
-    uint64_t last = cend_block == UINT64_MAX ? h->file_size : std::min<uint64_t>(h->file_size, cend_block + 0x10000);
-    if (cbeg >= h->file_size) { h->ubuf.clear(); return 0; }
-    if (!read_range(h, cbeg, last - cbeg)) return bfail(h, C3R_ERR_ARG, "short read from " + h->path);
-    const uint8_t* base = h->cbuf.data();
-    const size_t n = h->cbuf.size();
+    *ubytes = 0;
+    const uint64_t n = range_bytes(h, cbeg, cend_block);
+    if (n == 0) return 0;
+    if (fseeko(h->fp, (off_t)cbeg, SEEK_SET) != 0 || fread(dst, 1, n, h->fp) != n) return c3rbgzf::FE_SHORT_READ;
     size_t o = 0;
     uint64_t uoff = 0;
     while (o < n) {
-        const uint32_t bs = bgzf_block_size(base + o, n - o);
+        const uint32_t bs = bgzf_block_size(dst + o, n - o);
         if (bs == 0 || o + bs > n) {
             if (cend_block != UINT64_MAX && cbeg + o > cend_block) break;      // partial block past the range: ignore
             if (o + 18 > n && cend_block != UINT64_MAX) break;
-            return bfail(h, C3R_ERR_ARG, "corrupt BGZF block header in " + h->path);
+            return c3rbgzf::FE_HEADER;
         }
         Block b;
-        b.coff = cbeg + o; b.csize = bs; b.usize = rd32(base + o + bs - 4); b.uoff = uoff;
-        if (b.usize > 0x10000) return bfail(h, C3R_ERR_ARG, "BGZF block larger than 64 KiB");
+        b.coff = cbeg + o; b.csize = bs; b.usize = rd32(dst + o + bs - 4); b.uoff = uoff;
+        if (b.usize > 0x10000) return c3rbgzf::FE_BIG_BLOCK;
         blocks.push_back(b);
         uoff += b.usize;
         o += bs;
         if (cend_block != UINT64_MAX && b.coff > cend_block) break;
     }
+    *ubytes = uoff;
+    return 0;
+}
+
+// Inflate the blocks of read_blocks(cbeg, cend_block) into h->ubuf; `blocks` gets the block table.
+int inflate_range(c3r_bam* h, uint64_t cbeg, uint64_t cend_block, std::vector<Block>& blocks) {
+    h->cbuf.resize(range_bytes(h, cbeg, cend_block));
+    uint64_t uoff = 0;
+    if (int e = read_blocks(h, cbeg, cend_block, h->cbuf.data(), blocks, &uoff)) return bfail(h, C3R_ERR_ARG, fetch_err_text(h, e));
+    const uint8_t* base = h->cbuf.data();
     h->ubuf.resize(uoff);
     std::atomic<size_t> next(0);
     std::atomic<int> bad(0);
@@ -177,7 +206,7 @@ int inflate_range(c3r_bam* h, uint64_t cbeg, uint64_t cend_block, std::vector<Bl
         for (int i = 0; i < nt; ++i) th.emplace_back(work);
         for (auto& t : th) t.join();
     }
-    if (bad.load()) return bfail(h, C3R_ERR_ARG, "BGZF inflate/CRC failure in " + h->path);
+    if (bad.load()) return bfail(h, C3R_ERR_ARG, fetch_err_text(h, c3rbgzf::FE_INFLATE));
     return 0;
 }
 
@@ -265,119 +294,23 @@ int load_index(c3r_bam* h, const std::string& ipath) {
     return 0;
 }
 
-// ------------------------------------------------------------------ record decoding
-struct RecView {
-    int32_t tid, pos;
-    uint16_t flag, n_cigar;
-    uint8_t mapq, l_name;
-    int32_t l_seq;
-    const uint8_t* cigar;      // n_cigar u32
-    const uint8_t* seq;
-    const uint8_t* aux;
-    const uint8_t* aux_end;
-};
-
-inline bool view_record(const uint8_t* p, uint32_t block_size, RecView& r) {
-    if (block_size < 32) return false;
-    r.tid = (int32_t)rd32(p);
-    r.pos = (int32_t)rd32(p + 4);
-    r.l_name = p[8];
-    r.mapq = p[9];
-    r.n_cigar = rd16(p + 12);
-    r.flag = rd16(p + 14);
-    r.l_seq = (int32_t)rd32(p + 16);
-    if (r.l_seq < 0) return false;
-    const uint64_t need = 32ull + r.l_name + 4ull * r.n_cigar + (uint64_t)(r.l_seq + 1) / 2 + (uint64_t)r.l_seq;
-    if (need > block_size) return false;
-    r.cigar = p + 32 + r.l_name;
-    r.seq = r.cigar + 4 * r.n_cigar;
-    r.aux = r.seq + (r.l_seq + 1) / 2 + r.l_seq;
-    r.aux_end = p + block_size;
-    return true;
-}
-
-// walks the aux fields; returns false on malformed data.  Finds HP (integer) and CG (B,I long CIGAR).
-bool scan_aux(const RecView& r, int64_t* hp, const uint8_t** cg, uint32_t* cg_n) {
-    const uint8_t* a = r.aux;
-    const uint8_t* e = r.aux_end;
-    *hp = -1; *cg = nullptr; *cg_n = 0;
-    while (a + 3 <= e) {
-        const uint8_t t0 = a[0], t1 = a[1], ty = a[2];
-        a += 3;
-        int64_t iv = 0;
-        bool is_int = false;
-        switch (ty) {
-            case 'A': case 'c': case 'C':
-                if (a + 1 > e) return false;
-                iv = ty == 'c' ? (int8_t)a[0] : a[0]; is_int = ty != 'A'; a += 1; break;
-            case 's': case 'S':
-                if (a + 2 > e) return false;
-                iv = ty == 's' ? (int16_t)rd16(a) : rd16(a); is_int = true; a += 2; break;
-            case 'i': case 'I':
-                if (a + 4 > e) return false;
-                iv = ty == 'i' ? (int64_t)(int32_t)rd32(a) : (int64_t)rd32(a); is_int = true; a += 4; break;
-            case 'f':
-                if (a + 4 > e) return false;
-                a += 4; break;
-            case 'Z': case 'H':
-                while (a < e && *a) ++a;
-                if (a >= e) return false;
-                ++a; break;
-            case 'B': {
-                if (a + 5 > e) return false;
-                const uint8_t sub = a[0];
-                const uint32_t cnt = rd32(a + 1);
-                const uint32_t sz = (sub == 'c' || sub == 'C') ? 1 : (sub == 's' || sub == 'S') ? 2 : (sub == 'i' || sub == 'I' || sub == 'f') ? 4 : 0;
-                if (!sz) return false;
-                a += 5;
-                if ((uint64_t)(e - a) < (uint64_t)cnt * sz) return false;
-                if (t0 == 'C' && t1 == 'G' && sub == 'I') { *cg = a; *cg_n = cnt; }
-                a += (size_t)cnt * sz;
-                break;
-            }
-            default:
-                return false;
-        }
-        if (is_int && t0 == 'H' && t1 == 'P') *hp = iv;
-    }
-    return a == e;
-}
-
-inline int64_t cigar_ref_len(const uint8_t* c, uint32_t n) {
-    int64_t l = 0;
-    for (uint32_t i = 0; i < n; ++i) {
-        const uint32_t v = rd32(c + 4 * i), op = v & 15;
-        if (op == 0 || op == 2 || op == 3 || op == 7 || op == 8) l += v >> 4;
-    }
-    return l;
-}
-inline int64_t cigar_qry_len(const uint8_t* c, uint32_t n) {
-    int64_t l = 0;
-    for (uint32_t i = 0; i < n; ++i) {
-        const uint32_t v = rd32(c + 4 * i), op = v & 15;
-        if (op == 0 || op == 1 || op == 4 || op == 7 || op == 8) l += v >> 4;
-    }
-    return l;
-}
-
-void append_record(c3r_bam* h, const RecView& r, const uint8_t* cig, uint32_t n_cig, int64_t hp) {
+// ------------------------------------------------------------------ record decoding (bam_rec.cuh)
+void append_record(c3r_bam* h, const c3rbam::RecInfo& x) {
+    const c3rbam::RecView& r = x.r;
     h->pos.push_back(r.pos);
     h->flag.push_back(r.flag);
     h->mapq.push_back(r.mapq);
-    h->hp.push_back(hp <= 0 ? 0 : (uint8_t)(hp > 255 ? 255 : hp));
+    h->hp.push_back(c3rbam::clamp_hp(x.hp));
     const size_t c0 = h->cigar.size();
-    h->cigar.resize(c0 + n_cig);
-    for (uint32_t i = 0; i < n_cig; ++i) h->cigar[c0 + i] = rd32(cig + 4 * i);
+    h->cigar.resize(c0 + x.n_cig);
+    for (uint32_t i = 0; i < x.n_cig; ++i) h->cigar[c0 + i] = rd32(x.cig + 4 * i);
     h->cigar_off.push_back((int32_t)h->cigar.size());
-    int64_t n_bases;
+    const int64_t n_bases = x.n_bases;
     const size_t s0 = h->seq.size();
     if (r.l_seq > 0) {
-        n_bases = r.l_seq;
         h->seq.insert(h->seq.end(), r.seq, r.seq + (r.l_seq + 1) / 2);
         if (r.l_seq & 1) h->seq.back() &= 0xf0;
     } else {
-        // SEQ '*': samtools prints 'N' for every query position (bam_plcmd.c pileup_seq)
-        n_bases = cigar_qry_len(cig, n_cig);
         h->seq.resize(s0 + (size_t)(n_bases + 1) / 2, 0xff);
         if ((n_bases & 1) && n_bases > 0) h->seq.back() = 0xf0;
     }
@@ -451,15 +384,16 @@ int c3r_bam_idxstats(c3r_bam* h, int tid, int64_t* n_mapped, int64_t* n_unmapped
     return ri.has_meta ? C3R_OK : C3R_ERR_STATE;
 }
 
-int c3r_bam_fetch(c3r_bam* h, int tid, int64_t start1, int64_t end1, c3r_reads* out) {
-    if (!h || !out) return C3R_ERR_ARG;
-    if (tid < 0 || tid >= (int)h->ref_names.size()) return bfail(h, C3R_ERR_ARG, "reference id out of range");
-    if (start1 < 1 || end1 < start1) return bfail(h, C3R_ERR_ARG, "bad region");
-    reset_out(h);
-    const int64_t beg = start1 - 1, end = std::min<int64_t>(end1, 1LL << 29);      // 0-based half open
-    if (tid >= (int)h->index.size() || beg >= end) { export_out(h, out); return C3R_OK; }
+}  // extern "C"
+
+namespace {
+
+// The index query of a fetch: the chunks of the bins overlapping [beg, end), cut by the linear index, sorted and
+// merged (beg <= previous end).  Each merged chunk is one window of the fetch.
+void query_chunks(const c3r_bam* h, int tid, int64_t beg, int64_t end, std::vector<Chunk>& merged) {
+    merged.clear();
+    if (tid >= (int)h->index.size() || beg >= end) return;
     const RefIndex& ri = h->index[tid];
-    // candidate chunks: bins overlapping the region, cut by the linear index
     uint64_t min_off = 0;
     if (!ri.linear.empty()) {
         const size_t w = (size_t)(beg >> 14);
@@ -474,50 +408,141 @@ int c3r_bam_fetch(c3r_bam* h, int tid, int64_t start1, int64_t end1, c3r_reads* 
         if (it == ri.bins.end() || it->first != (uint32_t)b) continue;
         for (const Chunk& c : it->second) if (c.end > min_off) chunks.push_back(c);
     }
-    if (chunks.empty()) { export_out(h, out); return C3R_OK; }
     std::sort(chunks.begin(), chunks.end(), [](const Chunk& a, const Chunk& c) { return a.beg < c.beg; });
-    std::vector<Chunk> merged;
     for (const Chunk& c : chunks) {
         if (!merged.empty() && c.beg <= merged.back().end) merged.back().end = std::max(merged.back().end, c.end);
         else merged.push_back(c);
     }
+}
+
+// compressed range of a window and the record walk bounds in its inflated bytes (usize of them)
+inline uint64_t window_cbeg(const Chunk& c) { return c.beg >> 16; }
+inline uint64_t window_cend(const Chunk& c) { return c.end >> 16; }
+void window_bounds(const Chunk& c, const std::vector<Block>& blocks, uint64_t usize, uint64_t* ubeg, uint64_t* uend) {
+    *ubeg = c.beg & 0xffff;
+    *uend = usize;
+    for (const Block& b : blocks) if (b.coff == window_cend(c)) { *uend = b.uoff + (c.end & 0xffff); break; }
+}
+
+int check_fetch_args(c3r_bam* h, int tid, int64_t start1, int64_t end1) {
+    if (tid < 0 || tid >= (int)h->ref_names.size()) return bfail(h, C3R_ERR_ARG, "reference id out of range");
+    if (start1 < 1 || end1 < start1) return bfail(h, C3R_ERR_ARG, "bad region");
+    return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int c3r_bam_fetch(c3r_bam* h, int tid, int64_t start1, int64_t end1, c3r_reads* out) {
+    if (!h || !out) return C3R_ERR_ARG;
+    if (int rc = check_fetch_args(h, tid, start1, end1)) return rc;
+    reset_out(h);
+    const int64_t beg = start1 - 1, end = std::min<int64_t>(end1, 1LL << 29);      // 0-based half open
+    std::vector<Chunk> merged;
+    query_chunks(h, tid, beg, end, merged);
     std::vector<Block> blocks;
     bool past_end = false;
     for (const Chunk& c : merged) {
         if (past_end) break;
-        const uint64_t cb = c.beg >> 16, ce = c.end >> 16;
-        if (int rc = inflate_range(h, cb, ce, blocks)) return rc;
+        if (int rc = inflate_range(h, window_cbeg(c), window_cend(c), blocks)) return rc;
         if (blocks.empty()) continue;
-        // uncompressed window of the chunk: [beg within first block, end within the block at `ce`)
-        uint64_t ubeg = (c.beg & 0xffff), uend = h->ubuf.size();
-        for (const Block& b : blocks) if (b.coff == ce) { uend = b.uoff + (c.end & 0xffff); break; }
+        uint64_t ubeg, uend;
+        window_bounds(c, blocks, h->ubuf.size(), &ubeg, &uend);
         const uint8_t* u = h->ubuf.data();
         uint64_t o = ubeg;
         while (o + 4 <= uend) {
             const uint32_t bs = rd32(u + o);
-            if (o + 4 + bs > h->ubuf.size()) return bfail(h, C3R_ERR_ARG, "record crosses the end of an index chunk");
-            RecView r;
-            if (!view_record(u + o + 4, bs, r)) return bfail(h, C3R_ERR_ARG, "malformed BAM record");
+            if (o + 4 + bs > h->ubuf.size()) return bfail(h, C3R_ERR_ARG, fetch_err_text(h, c3rbgzf::FE_CROSS));
+            c3rbam::RecInfo x;
+            const int cls = c3rbam::classify_record(u + o + 4, bs, tid, beg, end, x);
             o += 4 + bs;
-            if (r.tid != tid) { if (r.tid > tid || r.tid < 0) { past_end = true; break; } continue; }
-            if (r.pos >= end) { past_end = true; break; }
-            int64_t hp;
-            const uint8_t* cg;
-            uint32_t cg_n;
-            if (!scan_aux(r, &hp, &cg, &cg_n)) return bfail(h, C3R_ERR_ARG, "malformed aux data in a BAM record");
-            const uint8_t* cig = r.cigar;
-            uint32_t n_cig = r.n_cigar;
-            if (cg && n_cig == 2 && (rd32(cig) & 15) == 4 && (int64_t)(rd32(cig) >> 4) == r.l_seq && (rd32(cig + 4) & 15) == 3) {
-                cig = cg; n_cig = cg_n;                     // long CIGAR kept in the CG:B,I tag (SAMv1 §4.2.2)
-            }
-            const int64_t rlen = cigar_ref_len(cig, n_cig);
-            const int64_t rend = r.pos + (rlen > 0 ? rlen : 1);
-            if (rend <= beg) continue;
-            append_record(h, r, cig, n_cig, hp);
+            if (cls == c3rbam::REC_ERR_MALFORMED) return bfail(h, C3R_ERR_ARG, fetch_err_text(h, c3rbgzf::FE_MALFORMED));
+            if (cls == c3rbam::REC_ERR_AUX) return bfail(h, C3R_ERR_ARG, fetch_err_text(h, c3rbgzf::FE_AUX));
+            if (cls == c3rbam::REC_STOP) { past_end = true; break; }
+            if (cls == c3rbam::REC_KEEP) append_record(h, x);
         }
     }
     export_out(h, out);
     return C3R_OK;
+}
+
+int c3r_bam_fetch_raw(c3r_bam* h, int tid, int64_t start1, int64_t end1, uint8_t* buf, int64_t cap, c3r_bam_raw* out) {
+    if (!h || !out || cap < 0 || (cap > 0 && !buf)) return C3R_ERR_ARG;
+    if (int rc = check_fetch_args(h, tid, start1, end1)) return rc;
+    memset(out, 0, sizeof *out);
+    h->raw_blocks.clear();
+    h->raw_windows.clear();
+    const int64_t beg = start1 - 1, end = std::min<int64_t>(end1, 1LL << 29);
+    out->tid = tid;
+    out->beg = beg;
+    out->end = end;
+    std::vector<Chunk> merged;
+    query_chunks(h, tid, beg, end, merged);
+    int64_t need = 0;
+    for (const Chunk& c : merged) need += (int64_t)range_bytes(h, window_cbeg(c), window_cend(c));
+    out->n_bytes = need;
+    if (need > cap) return bfail(h, C3R_ERR_CAPACITY, "buffer too small for the compressed blocks of the region");
+    std::vector<Block> blocks;
+    int64_t coff = 0, ubase = 0;
+    for (const Chunk& c : merged) {
+        c3r_bam_window w;
+        memset(&w, 0, sizeof w);
+        uint64_t usize = 0;
+        w.status = read_blocks(h, window_cbeg(c), window_cend(c), buf + coff, blocks, &usize);
+        w.first_block = (int32_t)h->raw_blocks.size();
+        if (!w.status) {
+            uint64_t ubeg, uend;
+            window_bounds(c, blocks, usize, &ubeg, &uend);
+            w.ubase = ubase; w.usize = (int64_t)usize; w.ubeg = (int64_t)ubeg; w.uend = (int64_t)uend;
+            w.n_blocks = (int32_t)blocks.size();
+            for (const Block& b : blocks) {
+                c3r_bgzf_block o;
+                o.coff = coff + (int64_t)(b.coff - window_cbeg(c));
+                o.uoff = ubase + (int64_t)b.uoff;
+                o.csize = (int32_t)b.csize; o.usize = (int32_t)b.usize;
+                o.window = (int32_t)h->raw_windows.size();
+                o.reserved = 0;
+                h->raw_blocks.push_back(o);
+            }
+            ubase += (int64_t)usize;
+        }
+        coff += (int64_t)range_bytes(h, window_cbeg(c), window_cend(c));
+        h->raw_windows.push_back(w);
+        if (w.status) break;                         // the host fetch returns here: nothing after it is read
+    }
+    out->n_windows = (int32_t)h->raw_windows.size();
+    out->n_blocks = (int64_t)h->raw_blocks.size();
+    out->n_ubytes = ubase;
+    out->data = buf;
+    out->blocks = h->raw_blocks.data();
+    out->windows = h->raw_windows.data();
+    return C3R_OK;
+}
+
+int c3r_debug_inflate(const uint8_t* block, int64_t n, uint8_t* out, int64_t cap, int64_t* n_out) {
+    if (!block || !n_out || n < 26 || n > 0x10000 || cap < 0 || (cap > 0 && !out)) return C3R_ERR_ARG;
+    const uint32_t bs = bgzf_block_size(block, (size_t)n);
+    if (bs != (uint32_t)n) return C3R_ERR_ARG;
+    const uint32_t usize = rd32(block + n - 4);
+    *n_out = usize;
+    if (usize > c3rbgzf::MAX_BLOCK || (int64_t)usize > cap) return C3R_ERR_ARG;
+    uint32_t off, len;
+    if (!c3rbgzf::bgzf_payload(block, (uint32_t)n, &off, &len)) return C3R_ERR_ARG;
+    c3rbgzf::HostSink sink;
+    sink.out = out; sink.cap = usize; sink.pos = 0;
+    c3rbgzf::Tables t;
+    if (c3rbgzf::inflate_core(block + off, len, sink, t) != c3rbgzf::IE_OK || sink.pos != usize) return C3R_ERR_ARG;
+    // the device's CRC: 32 segments combined
+    uint32_t tab[256];
+    for (uint32_t k = 0; k < 256; ++k) tab[k] = c3rbgzf::crc_table_entry(k);
+    const uint32_t seg = (usize + 31) / 32;
+    uint32_t acc = 0;
+    for (uint32_t a = 0; a < usize; a += seg) {
+        const uint32_t l = std::min(seg, usize - a);
+        acc = c3rbgzf::crc32_combine(acc, c3rbgzf::crc32_bytes(tab, out + a, l), l);
+    }
+    return acc == rd32(block + n - 8) ? C3R_OK : C3R_ERR_ARG;
 }
 
 // ---------------------------------------------------------------- writer (synthetic fixtures)

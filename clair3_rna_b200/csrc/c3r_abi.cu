@@ -22,6 +22,7 @@
 #include "nn_fp32.cuh"
 #include "nn_tc.cuh"
 #include "call.cuh"
+#include "bgzf.cuh"
 
 using namespace c3r;
 
@@ -82,6 +83,21 @@ struct Slot {
     int64_t n_rows = 0, n_cand = 0, alt_total = 0;
     int launches = 0;
     c3r_result res;
+    // device BAM reading (c3r_submit_bam_chunk): the records are parsed on the device before stage A
+    bool bam = false;
+    bool pending_parse = false;       // the parse counts have not been taken yet (advance())
+    cudaEvent_t ev_parse = nullptr;   // the parse counts are on the host
+    cudaEvent_t ev_bam[6] = {};       // [0, 1) inflate, [1, 2) record boundaries, [2, 3) parse + offsets, [4, 5) k_rec_write
+    c3rbgzf::Fetch fetch = {};
+    Buf b_cdata, b_blk, b_win, b_ubuf, b_nrec, b_soff, b_scls, b_skey, b_snops, b_snb, b_sdst, b_sc;
+    Pin h_fsc, h_rpos, h_rflag, h_rmapq, h_rhp, h_rcoff, h_rcig, h_rsoff, h_rseq;
+    c3r_reads h_reads = {};           // the parsed records in the pinned buffers above
+    // what c3r_submit_bam_chunk was given, for the part queued once the parse counts are in
+    const uint8_t* ref_host = nullptr;
+    int64_t ref_start1 = 0, ref_len = 0, region_start1 = 0, region_end1 = 0;
+    bool has_filter = false;
+    std::vector<int32_t> f_pbed, f_cbed, f_known;
+    c3r_site_filter flt = {};
 };
 
 }  // namespace
@@ -444,6 +460,8 @@ int c3r_create(c3r_ctx** out, int device_ordinal, const c3r_params* params) {
         // spin-wait by default: a blocking-sync event wakes the waiting thread ~0.3 ms late (measured), which delays
         // stage B by as much; C3R_BLOCKING_COUNTS trades that for an idle core while waiting
         CK(cudaEventCreateWithFlags(&s.ev_cnt, cudaEventDisableTiming | (getenv("C3R_BLOCKING_COUNTS") ? cudaEventBlockingSync : 0)));
+        CK(cudaEventCreateWithFlags(&s.ev_parse, cudaEventDisableTiming | (getenv("C3R_BLOCKING_COUNTS") ? cudaEventBlockingSync : 0)));
+        for (int k = 0; k < 6; ++k) CK(cudaEventCreate(&s.ev_bam[k]));
         if (ensure(ctx, s.scalars, 256)) return C3R_ERR_CUDA;
         if (ensure_pin(ctx, s.h_scalars, 256)) return C3R_ERR_CUDA;
     }
@@ -474,15 +492,20 @@ void c3r_destroy(c3r_ctx* ctx) {
                      &s.word_base, &s.row_pos, &s.counts, &s.row_depth, &s.row_flag, &s.head_cnt, &s.tail_cnt,
                      &s.skipdiff, &s.max_skip, &s.row_ins, &s.row_del, &s.binc, &s.bin_cur, &s.events, &s.raw, &s.cov, &s.cov_tile, &s.refnib,
                      &s.cand_row, &s.cand_pos, &s.cand_depth, &s.tensor, &s.alt_off, &s.alt_n, &s.alt, &s.cur_ref,
-                     &s.deleted, &s.probs, &s.scalars, &s.scan_scratch, &s.pbed, &s.cbed, &s.known, &s.covP, &s.xop, &s.d_calls};
+                     &s.deleted, &s.probs, &s.scalars, &s.scan_scratch, &s.pbed, &s.cbed, &s.known, &s.covP, &s.xop, &s.d_calls,
+                     &s.b_cdata, &s.b_blk, &s.b_win, &s.b_ubuf, &s.b_nrec, &s.b_soff, &s.b_scls, &s.b_skey, &s.b_snops, &s.b_snb,
+                     &s.b_sdst, &s.b_sc};
         for (Buf* b : bs) release(*b);
         Pin* ps[] = {&s.h_scalars, &s.h_pos, &s.h_depth, &s.h_probs, &s.h_alt_off, &s.h_alt_n, &s.h_alt, &s.h_tensor,
-                     &s.h_row_pos, &s.h_counts, &s.h_row_depth, &s.h_calls};
+                     &s.h_row_pos, &s.h_counts, &s.h_row_depth, &s.h_calls, &s.h_fsc, &s.h_rpos, &s.h_rflag, &s.h_rmapq,
+                     &s.h_rhp, &s.h_rcoff, &s.h_rcig, &s.h_rsoff, &s.h_rseq};
         for (Pin* b : ps) release(*b);
         for (int k = 0; k < N_EV; ++k) if (s.ev[k]) cudaEventDestroy(s.ev[k]);
         if (s.ev_alt) cudaEventDestroy(s.ev_alt);
         for (int k = 0; k < 2; ++k) if (s.ev_call[k]) cudaEventDestroy(s.ev_call[k]);
         if (s.ev_cnt) cudaEventDestroy(s.ev_cnt);
+        if (s.ev_parse) cudaEventDestroy(s.ev_parse);
+        for (int k = 0; k < 6; ++k) if (s.ev_bam[k]) cudaEventDestroy(s.ev_bam[k]);
         if (s.st) cudaStreamDestroy(s.st);
         if (s.st_a) cudaStreamDestroy(s.st_a);
     }
@@ -580,6 +603,29 @@ int c3r_submit_chunk_filtered(c3r_ctx* ctx, const c3r_reads* rd, const uint8_t* 
 // assumed not to outnumber the sequenced bases; row events - indel tokens + read bases that differ from the
 // reference - sized for one base in four); if a chunk breaks that, the device-side capacity checks fire and
 // advance() comes back here with the CIGARs for exact bounds (events then sized for every base).
+// The slot's scan state (scan.cuh), sized for scans of up to n elements.  Every scan of a slot uses the same layout
+// (aggregates of SCAN_ELEM bytes): the status words of one layout must never lie over the aggregates of another.
+constexpr size_t SCAN_ELEM = 32;
+static_assert(sizeof(ScanElem) <= SCAN_ELEM && sizeof(c3rbgzf::Slot3) <= SCAN_ELEM, "scan aggregates fit the layout");
+static int ensure_scan(c3r_ctx* ctx, Slot& s, int64_t n) {
+    const size_t elem = SCAN_ELEM;
+    // scan state: 256 B of counters, then per tile a status word, an aggregate and an inclusive prefix
+    const size_t tiles = (size_t)(n / SCAN_TILE + 2);
+    const size_t need = 256 + tiles * 4 + 2 * tiles * elem + 64;
+    if (s.scan_scratch.cap < need) {
+        if (ensure(ctx, s.scan_scratch, need)) return C3R_ERR_CUDA;
+        CK(cudaMemsetAsync(s.scan_scratch.p, 0, s.scan_scratch.cap, s.st_a));   // status words of epoch 0, ticket 0
+    }
+    uint8_t* sp = (uint8_t*)s.scan_scratch.p;
+    const size_t cap_tiles = (s.scan_scratch.cap - 256 - 64) / (4 + 2 * elem);
+    s.scan.ctrl = (unsigned int*)sp;
+    s.scan.status = (uint32_t*)(sp + 256);
+    s.scan.aggr = sp + 256 + ((cap_tiles * 4 + 15) / 16) * 16;
+    s.scan.incl = (uint8_t*)s.scan.aggr + cap_tiles * elem;
+    s.scan.err = P<int32_t>(s.scalars) + 6;
+    return 0;
+}
+
 static int size_rows(c3r_ctx* ctx, Slot& s, const uint32_t* cigar_host) {
     Dev& d = s.d;
     int64_t md_len = 0, n_skip = 0, ev_ub = 0;
@@ -616,20 +662,7 @@ static int size_rows(c3r_ctx* ctx, Slot& s, const uint32_t* cigar_host) {
     {
         int64_t mx = d.n_ops > d.NW ? d.n_ops : d.NW;
         if (L_ub + 4 > mx) mx = L_ub + 4;
-        // scan state: 256 B of counters, then per tile a status word, an aggregate and an inclusive prefix
-        const size_t tiles = (size_t)(mx / SCAN_TILE + 2);
-        const size_t need = 256 + tiles * 4 + 2 * tiles * sizeof(ScanElem) + 64;
-        if (s.scan_scratch.cap < need) {
-            EN(scan_scratch, need);
-            CK(cudaMemsetAsync(s.scan_scratch.p, 0, s.scan_scratch.cap, s.st_a));   // status words of epoch 0, ticket 0
-        }
-        uint8_t* sp = (uint8_t*)s.scan_scratch.p;
-        const size_t cap_tiles = (s.scan_scratch.cap - 256 - 64) / (4 + 2 * sizeof(ScanElem));
-        s.scan.ctrl = (unsigned int*)sp;
-        s.scan.status = (uint32_t*)(sp + 256);
-        s.scan.aggr = sp + 256 + ((cap_tiles * 4 + 15) / 16) * 16;
-        s.scan.incl = (uint8_t*)s.scan.aggr + cap_tiles * sizeof(ScanElem);
-        s.scan.err = P<int32_t>(s.scalars) + 6;
+        if (int rc = ensure_scan(ctx, s, mx)) return rc;
     }
 #undef EN
     d.row_pos = P<int32_t>(s.row_pos); d.counts = P<int32_t>(s.counts); d.row_depth = P<int32_t>(s.row_depth);
@@ -644,30 +677,40 @@ static int size_rows(c3r_ctx* ctx, Slot& s, const uint32_t* cigar_host) {
     return 0;
 }
 
-static int submit_once(c3r_ctx* ctx, const c3r_reads* rd, const uint8_t* ref, int64_t ref_start1, int64_t ref_len,
-                       int64_t region_start1, int64_t region_end1, c3r_ticket* ticket) {
+// checks of a submit that need no reads; fills in the resident reference window when ref == NULL
+static int check_submit(c3r_ctx* ctx, const uint8_t* ref, int64_t* ref_start1, int64_t* ref_len, int64_t region_start1,
+                        int64_t region_end1) {
     if (!ref) {
         if (!ctx->ref_res_len) return fail(ctx, C3R_ERR_STATE, "ref == NULL but c3r_set_reference was never called");
-        ref_start1 = ctx->ref_res_start0 + 1;
-        ref_len = ctx->ref_res_len;
+        *ref_start1 = ctx->ref_res_start0 + 1;
+        *ref_len = ctx->ref_res_len;
     }
     if (!ctx->have_weights) return fail(ctx, C3R_ERR_STATE, "c3r_set_weights must be called before c3r_submit_chunk");
     if (region_end1 < region_start1 || region_start1 < 1) return fail(ctx, C3R_ERR_ARG, "bad region");
     if (region_end1 > 0x7fff0000LL) return fail(ctx, C3R_ERR_CAPACITY, "positions must fit int32");
+    return 0;
+}
+
+static int free_slot(c3r_ctx* ctx) {
+    for (int i = 0; i < N_SLOTS; ++i) if (!ctx->slots[i].in_use) return i;
+    return fail(ctx, C3R_ERR_STATE, "all tickets in flight; c3r_release one first");
+}
+
+static int queue_rec_write(c3r_ctx* ctx, Slot& s);
+
+// Everything of a chunk from its reads onward: the slot's buffers sized from the read counts, the reads copied to
+// the device (host reads) or written there by k_rec_write (a device fetch, reads_on_device), the filters and the
+// reference, stage A and the copy of its counts.  The ticket is then pending_b.
+static int queue_chunk(c3r_ctx* ctx, Slot& s, const c3r_reads* rd, bool reads_on_device, const uint8_t* ref,
+                       int64_t ref_start1, int64_t ref_len, int64_t region_start1, int64_t region_end1,
+                       const c3r_site_filter* flt) {
     if (rd->n_seq_bytes * 2 >= 0xffffffffLL) return fail(ctx, C3R_ERR_CAPACITY, "more than 4G bases in one chunk");
     if (rd->n_reads >= (1LL << 28)) return fail(ctx, C3R_ERR_CAPACITY, "more than 2^28 reads in one chunk");
-    CK(cudaSetDevice(ctx->device));
     auto now = [] { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
     double tp = now();
     auto lap = [&](int k) { const double t = now(); ctx->t_phase[k] += t - tp; tp = t; };
-    ++ctx->n_submit;
-    int si = -1;
-    for (int i = 0; i < N_SLOTS; ++i) if (!ctx->slots[i].in_use) { si = i; break; }
-    if (si < 0) return fail(ctx, C3R_ERR_STATE, "all tickets in flight; c3r_release one first");
-    Slot& s = ctx->slots[si];
-    s.launches = 0;
+    if (!reads_on_device) s.launches = 0;          // a device fetch counts its parse kernels too
     s.has_result = false;
-    s.calls = ctx->calls;
     Dev& d = s.d;
     memset(&d, 0, sizeof d);
     const c3r_params& pr = ctx->prm;
@@ -681,7 +724,7 @@ static int submit_once(c3r_ctx* ctx, const c3r_reads* rd, const uint8_t* ref, in
     d.ref_start0 = ref_start1 - 1; d.ref_len = ref_len;
     d.thr_snp = (const uint16_t*)ctx->thr.p; d.thr_indel = (const uint16_t*)ctx->thr.p + THR_N;
     s.n_seq_bytes = rd->n_seq_bytes;
-    s.n_known_sites = (ctx->filter && ctx->filter->n_known_sites > 0) ? ctx->filter->n_known_sites : 0;
+    s.n_known_sites = (flt && flt->n_known_sites > 0) ? flt->n_known_sites : 0;
     s.exact_bounds = false;
     s.deferred_rc = 0;
     const int64_t R = rd->n_reads > 0 ? rd->n_reads : 1, O = rd->n_ops > 0 ? rd->n_ops : 1;
@@ -701,7 +744,6 @@ static int submit_once(c3r_ctx* ctx, const c3r_reads* rd, const uint8_t* ref, in
     s.zero_bytes = (size_t)pool_words * 4;
     EN(ptile, (NWp / PT_WORDS + 4) * 4);
     if (ref) { EN(refnib, ((ref_len + 7) / 8 + 1) * 4); }
-    const c3r_site_filter* flt = ctx->filter;
     d.n_pbed = d.n_cbed = d.n_known = -1;
     if (flt) {
         if (flt->n_pileup_bed >= 0) { EN(pbed, (flt->n_pileup_bed + 1) * 8); EN(covP, (d.NW + 4) * 4); d.n_pbed = (int32_t)flt->n_pileup_bed; }
@@ -735,20 +777,26 @@ static int submit_once(c3r_ctx* ctx, const c3r_reads* rd, const uint8_t* ref, in
 
     cudaStream_t st = s.st_a;
     lap(0);
-    CK(cudaEventRecord(s.ev[0], st));
-    if (rd->n_reads > 0) {
-        CK(cudaMemcpyAsync(s.pos.p, rd->pos, rd->n_reads * 4, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(s.flag.p, rd->flag, rd->n_reads * 2, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(s.mapq.p, rd->mapq, rd->n_reads, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(s.hp.p, rd->hp, rd->n_reads, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(s.cigar_off.p, rd->cigar_off, (rd->n_reads + 1) * 4, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(s.seq_off.p, rd->seq_off, (rd->n_reads + 1) * 8, cudaMemcpyHostToDevice, st));
+    if (reads_on_device) {
+        if (int rc = queue_rec_write(ctx, s)) return rc;
+    } else {
+        CK(cudaEventRecord(s.ev[0], st));
+        if (rd->n_reads > 0) {
+            CK(cudaMemcpyAsync(s.pos.p, rd->pos, rd->n_reads * 4, cudaMemcpyHostToDevice, st));
+            CK(cudaMemcpyAsync(s.flag.p, rd->flag, rd->n_reads * 2, cudaMemcpyHostToDevice, st));
+            CK(cudaMemcpyAsync(s.mapq.p, rd->mapq, rd->n_reads, cudaMemcpyHostToDevice, st));
+            CK(cudaMemcpyAsync(s.hp.p, rd->hp, rd->n_reads, cudaMemcpyHostToDevice, st));
+            CK(cudaMemcpyAsync(s.cigar_off.p, rd->cigar_off, (rd->n_reads + 1) * 4, cudaMemcpyHostToDevice, st));
+            CK(cudaMemcpyAsync(s.seq_off.p, rd->seq_off, (rd->n_reads + 1) * 8, cudaMemcpyHostToDevice, st));
+        }
     }
     if (d.n_pbed > 0) CK(cudaMemcpyAsync(s.pbed.p, flt->pileup_bed, (size_t)d.n_pbed * 8, cudaMemcpyHostToDevice, st));
     if (d.n_cbed > 0) CK(cudaMemcpyAsync(s.cbed.p, flt->confident_bed, (size_t)d.n_cbed * 8, cudaMemcpyHostToDevice, st));
     if (d.n_known > 0) CK(cudaMemcpyAsync(s.known.p, flt->known_sites, (size_t)d.n_known * 4, cudaMemcpyHostToDevice, st));
-    if (rd->n_ops > 0) CK(cudaMemcpyAsync(s.cigar.p, rd->cigar, rd->n_ops * 4, cudaMemcpyHostToDevice, st));
-    if (rd->n_seq_bytes > 0) CK(cudaMemcpyAsync(s.seq.p, rd->seq, rd->n_seq_bytes, cudaMemcpyHostToDevice, st));
+    if (!reads_on_device) {
+        if (rd->n_ops > 0) CK(cudaMemcpyAsync(s.cigar.p, rd->cigar, rd->n_ops * 4, cudaMemcpyHostToDevice, st));
+        if (rd->n_seq_bytes > 0) CK(cudaMemcpyAsync(s.seq.p, rd->seq, rd->n_seq_bytes, cudaMemcpyHostToDevice, st));
+    }
     if (ref && ref_len > 0) {
         CK(cudaMemcpyAsync(s.ref.p, ref, ref_len, cudaMemcpyHostToDevice, st));
         const int64_t nw = (ref_len + 7) / 8;
@@ -758,26 +806,264 @@ static int submit_once(c3r_ctx* ctx, const c3r_reads* rd, const uint8_t* ref, in
     // The copies above overlap the network pass of the ticket before this one, and so do the position / row stages:
     // the network's partly filled rounds and its tail leave SMs idle that these ~20 short kernels take (9.66 M sites/s
     // end to end against 8.73 M when they wait for the pass to end).
-    s.in_use = true;                                 // from here on every error path releases the slot (below)
     lap(1);
     int rc = run_stage_a(ctx, s);
     lap(2);
     // the counts of stage A travel to the host behind it; stage B is queued when they have arrived (advance)
     if (!rc) { cudaError_t e = cudaMemcpyAsync(s.h_scalars.p, s.scalars.p, 64, cudaMemcpyDeviceToHost, st); if (e != cudaSuccess) rc = fail(ctx, C3R_ERR_CUDA, cudaGetErrorString(e)); }
     if (!rc) { cudaError_t e = cudaEventRecord(s.ev_cnt, st); if (e != cudaSuccess) rc = fail(ctx, C3R_ERR_CUDA, cudaGetErrorString(e)); }
-    if (rc) { cudaStreamSynchronize(st); cudaStreamSynchronize(s.st); s.in_use = false; return rc; }
+    if (rc) return rc;
     s.pending_b = true;
+    return 0;
+}
+
+static int submit_once(c3r_ctx* ctx, const c3r_reads* rd, const uint8_t* ref, int64_t ref_start1, int64_t ref_len,
+                       int64_t region_start1, int64_t region_end1, c3r_ticket* ticket) {
+    if (int rc = check_submit(ctx, ref, &ref_start1, &ref_len, region_start1, region_end1)) return rc;
+    CK(cudaSetDevice(ctx->device));
+    ++ctx->n_submit;
+    const int si = free_slot(ctx);
+    if (si < 0) return si;
+    Slot& s = ctx->slots[si];
+    s.bam = false;
+    s.pending_parse = false;
+    s.calls = ctx->calls;
+    int rc = queue_chunk(ctx, s, rd, false, ref, ref_start1, ref_len, region_start1, region_end1, ctx->filter);
+    if (rc) { cudaStreamSynchronize(s.st_a); cudaStreamSynchronize(s.st); return rc; }
+    s.in_use = true;
     s.order = ++ctx->submit_seq;
     *ticket = si;
     // tickets submitted earlier whose counts are in by now get their stage B queued here (never blocks)
+    const auto t1 = std::chrono::steady_clock::now();
     advance_all(ctx, getenv("C3R_SYNC_SUBMIT") != nullptr);
-    lap(3);
+    ctx->t_phase[3] += std::chrono::duration<double>(std::chrono::steady_clock::now() - t1).count();
     return C3R_OK;
+}
+
+// ------------------------------------------------------------ device BAM reading (csrc/bgzf.cuh)
+static const char* fetch_err_text(int code) {
+    switch (code) {
+        case c3rbgzf::FE_INFLATE: return "BGZF inflate/CRC failure";
+        case c3rbgzf::FE_HEADER: return "corrupt BGZF block header";
+        case c3rbgzf::FE_BIG_BLOCK: return "BGZF block larger than 64 KiB";
+        case c3rbgzf::FE_SHORT_READ: return "short read from the BAM";
+        case c3rbgzf::FE_CROSS: return "record crosses the end of an index chunk";
+        case c3rbgzf::FE_MALFORMED: return "malformed BAM record";
+        default: return "malformed aux data in a BAM record";
+    }
+}
+
+// the tables of a raw fetch come from outside the library: every offset is checked before the kernels use it
+static int check_raw(c3r_ctx* ctx, const c3r_bam_raw* raw) {
+    if (raw->n_windows < 0 || raw->n_blocks < 0 || raw->n_bytes < 0 || raw->n_ubytes < 0 ||
+        (raw->n_bytes > 0 && !raw->data) || (raw->n_blocks > 0 && !raw->blocks) || (raw->n_windows > 0 && !raw->windows))
+        return fail(ctx, C3R_ERR_ARG, "raw fetch: bad counts or null tables");
+    if (raw->n_windows >= (1 << 20) || raw->n_ubytes >= (1LL << 40)) return fail(ctx, C3R_ERR_CAPACITY, "raw fetch too large");
+    if (raw->beg < 0 || raw->end > (1LL << 31) || raw->tid < 0) return fail(ctx, C3R_ERR_ARG, "raw fetch: bad region");
+    int64_t ub = 0, nb = 0;
+    for (int32_t w = 0; w < raw->n_windows; ++w) {
+        const c3r_bam_window& W = raw->windows[w];
+        if (W.status) {
+            if (W.status < c3rbgzf::FE_HEADER || W.status > c3rbgzf::FE_SHORT_READ || W.n_blocks != 0)
+                return fail(ctx, C3R_ERR_ARG, "raw fetch: bad window status");
+            continue;
+        }
+        if (W.ubase != ub || W.usize < 0 || W.ubeg < 0 || W.uend < 0 || W.first_block != nb || W.n_blocks < 0 ||
+            W.n_blocks > raw->n_blocks - nb)
+            return fail(ctx, C3R_ERR_ARG, "raw fetch: window table does not match its blocks");
+        int64_t uo = W.ubase;
+        for (int32_t k = 0; k < W.n_blocks; ++k) {
+            const c3r_bgzf_block& B = raw->blocks[nb + k];
+            if (B.window != w || B.uoff != uo || B.usize < 0 || B.usize > (int32_t)c3rbgzf::MAX_BLOCK || B.csize < 0 ||
+                B.coff < 0 || B.coff > raw->n_bytes - B.csize)
+                return fail(ctx, C3R_ERR_ARG, "raw fetch: block table out of bounds");
+            uo += B.usize;
+        }
+        if (uo != W.ubase + W.usize) return fail(ctx, C3R_ERR_ARG, "raw fetch: window size does not match its blocks");
+        ub += W.usize;
+        nb += W.n_blocks;
+    }
+    if (nb != raw->n_blocks || ub != raw->n_ubytes) return fail(ctx, C3R_ERR_ARG, "raw fetch: tables do not add up");
+    return 0;
+}
+
+int c3r_submit_bam_chunk(c3r_ctx* ctx, const c3r_bam_raw* raw, const uint8_t* ref, int64_t ref_start1, int64_t ref_len,
+                         int64_t region_start1, int64_t region_end1, const c3r_site_filter* filter, c3r_ticket* ticket) {
+    if (!ctx || !raw || !ticket) return C3R_ERR_ARG;
+    if (int rc = check_filter(ctx, filter)) return rc;
+    if (int rc = check_raw(ctx, raw)) return rc;
+    if (int rc = check_submit(ctx, ref, &ref_start1, &ref_len, region_start1, region_end1)) return rc;
+    CK(cudaSetDevice(ctx->device));
+    const int si = free_slot(ctx);
+    if (si < 0) return si;
+    Slot& s = ctx->slots[si];
+    s.bam = true;
+    s.calls = ctx->calls;
+    s.ref_host = ref; s.ref_start1 = ref_start1; s.ref_len = ref_len;
+    s.region_start1 = region_start1; s.region_end1 = region_end1;
+    // the filter is read during the call (as c3r_submit_chunk_filtered's): the slot keeps a copy for the deferred part
+    s.has_filter = filter != nullptr;
+    if (filter) {
+        s.f_pbed.assign(filter->pileup_bed, filter->pileup_bed + (filter->n_pileup_bed > 0 ? 2 * filter->n_pileup_bed : 0));
+        s.f_cbed.assign(filter->confident_bed, filter->confident_bed + (filter->n_confident_bed > 0 ? 2 * filter->n_confident_bed : 0));
+        s.f_known.assign(filter->known_sites, filter->known_sites + (filter->n_known_sites > 0 ? filter->n_known_sites : 0));
+        s.flt = *filter;
+        s.flt.pileup_bed = s.f_pbed.data(); s.flt.confident_bed = s.f_cbed.data(); s.flt.known_sites = s.f_known.data();
+    }
+    // device windows and the record slot capacity: window w holds at most usize / 36 + 1 records (a record is at least
+    // 36 bytes; the chain ends at a shorter one)
+    const int32_t nw = raw->n_windows;
+    std::vector<c3rbgzf::DevWindow> dw((size_t)(nw > 0 ? nw : 1));
+    int64_t n_slots = 0;
+    for (int32_t w = 0; w < nw; ++w) {
+        const c3r_bam_window& W = raw->windows[w];
+        c3rbgzf::DevWindow& x = dw[w];
+        x.ubase = W.ubase; x.usize = W.usize; x.ubeg = W.ubeg; x.uend = W.uend;
+        x.slot_base = n_slots; x.status = W.status; x.n_blocks = W.n_blocks;
+        n_slots += W.usize / 36 + 1;
+    }
+    const int64_t NB = raw->n_blocks, S = n_slots > 0 ? n_slots : 1;
+#define EN(b, bytes) if (ensure(ctx, s.b, (size_t)(bytes))) return C3R_ERR_CUDA
+    EN(b_cdata, raw->n_bytes + 16); EN(b_blk, (NB + 1) * 32); EN(b_win, (size_t)(nw + 1) * sizeof(c3rbgzf::DevWindow));
+    EN(b_ubuf, raw->n_ubytes + 64); EN(b_nrec, (nw + 1) * 4);
+    EN(b_soff, S * 8); EN(b_scls, S); EN(b_skey, S * 8); EN(b_snops, S * 4); EN(b_snb, S * 8);
+    EN(b_sdst, S * sizeof(c3rbgzf::Slot3)); EN(b_sc, sizeof(c3rbgzf::FetchSc));
+#undef EN
+    if (ensure_pin(ctx, s.h_fsc, sizeof(c3rbgzf::FetchSc))) return C3R_ERR_CUDA;
+    if (int rc = ensure_scan(ctx, s, S)) return rc;
+    // block table as columns
+    std::vector<int64_t> bcol((size_t)(2 * NB + 1));
+    std::vector<int32_t> icol((size_t)(3 * NB + 1));
+    for (int64_t k = 0; k < NB; ++k) {
+        const c3r_bgzf_block& B = raw->blocks[k];
+        bcol[k] = B.coff; bcol[NB + k] = B.uoff;
+        icol[k] = B.csize; icol[NB + k] = B.usize; icol[2 * NB + k] = B.window;
+    }
+    c3rbgzf::Fetch& f = s.fetch;
+    f = c3rbgzf::Fetch{};
+    f.tid = raw->tid; f.beg = raw->beg; f.end = raw->end; f.n_win = nw; f.n_slots = n_slots;
+    f.cdata = P<uint8_t>(s.b_cdata);
+    int64_t* b64 = P<int64_t>(s.b_blk);
+    int32_t* b32 = (int32_t*)(b64 + 2 * NB);
+    f.blk_coff = b64; f.blk_uoff = b64 + NB; f.blk_csize = b32; f.blk_usize = b32 + NB; f.blk_win = b32 + 2 * NB;
+    f.win = P<c3rbgzf::DevWindow>(s.b_win);
+    f.ubuf = P<uint8_t>(s.b_ubuf); f.n_rec = P<int32_t>(s.b_nrec);
+    f.slot_off = P<int64_t>(s.b_soff); f.slot_cls = P<uint8_t>(s.b_scls); f.slot_key = P<uint64_t>(s.b_skey);
+    f.slot_nops = P<int32_t>(s.b_snops); f.slot_nb = P<int64_t>(s.b_snb); f.slot_dst = P<c3rbgzf::Slot3>(s.b_sdst);
+    f.sc = P<c3rbgzf::FetchSc>(s.b_sc);
+    cudaStream_t st = s.st_a;
+    int launches = 0;
+    // the block tables are pageable host memory: the copies stage them before the call returns; the compressed bytes
+    // are read by DMA after it (page-locked) or staged likewise
+    if (raw->n_bytes > 0) CK(cudaMemcpyAsync(s.b_cdata.p, raw->data, raw->n_bytes, cudaMemcpyHostToDevice, st));
+    if (NB > 0) {
+        CK(cudaMemcpyAsync(b64, bcol.data(), (size_t)NB * 16, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(b32, icol.data(), (size_t)NB * 12, cudaMemcpyHostToDevice, st));
+    }
+    if (nw > 0) CK(cudaMemcpyAsync(s.b_win.p, dw.data(), (size_t)nw * sizeof(c3rbgzf::DevWindow), cudaMemcpyHostToDevice, st));
+    CK(cudaMemsetAsync(s.b_sc.p, 0xff, 16, st));                 // no error, no stop
+    CK(cudaMemsetAsync((uint8_t*)s.b_sc.p + 16, 0, sizeof(c3rbgzf::FetchSc) - 16, st));
+    CK(cudaEventRecord(s.ev_bam[0], st));
+    if (NB > 0) {
+        static bool smem_set = false;
+        if (!smem_set) {
+            CK(cudaFuncSetAttribute(c3rbgzf::k_inflate, cudaFuncAttributeMaxDynamicSharedMemorySize, c3rbgzf::INFLATE_SMEM));
+            smem_set = true;
+        }
+        c3rbgzf::k_inflate<<<(unsigned)NB, 32, c3rbgzf::INFLATE_SMEM, st>>>(f); ++launches;
+    }
+    CK(cudaEventRecord(s.ev_bam[1], st));
+    if (nw > 0) { c3rbgzf::k_rec_bounds<<<(unsigned)nw, c3rbgzf::BOUNDS_THREADS, 0, st>>>(f); ++launches; }
+    CK(cudaEventRecord(s.ev_bam[2], st));
+    if (n_slots > 0) {
+        const int64_t blocks = (n_slots + 255) / 256;
+        c3rbgzf::k_rec_parse<<<(unsigned)(blocks < ctx->sm_count * 16 ? blocks : ctx->sm_count * 16), 256, 0, st>>>(f); ++launches;
+        c3rbgzf::OpKeep op; op.f = f;
+        launches += device_scan(op, n_slots, s.scan, s.scan_epoch, (c3rbgzf::Slot3*)&f.sc->n_reads, st);
+    }
+    CK(cudaEventRecord(s.ev_bam[3], st));
+    CK(cudaMemcpyAsync(s.h_fsc.p, s.b_sc.p, sizeof(c3rbgzf::FetchSc), cudaMemcpyDeviceToHost, st));
+    CK(cudaEventRecord(s.ev_parse, st));
+    CK(cudaGetLastError());
+    s.launches = launches;
+    s.in_use = true;
+    s.has_result = false;
+    s.deferred_rc = 0;
+    s.pending_b = false;
+    s.pending_parse = true;
+    s.order = ++ctx->submit_seq;
+    ++ctx->n_submit;
+    *ticket = si;
+    advance_all(ctx, getenv("C3R_SYNC_SUBMIT") != nullptr);
+    return C3R_OK;
+}
+
+// k_rec_write into the read buffers queue_chunk sized, and the copy of the reads to the pinned host buffers
+static int queue_rec_write(c3r_ctx* ctx, Slot& s) {
+    cudaStream_t st = s.st_a;
+    c3rbgzf::Fetch& f = s.fetch;
+    c3r_reads& h = s.h_reads;
+    f.pos = P<int32_t>(s.pos); f.flag = P<uint16_t>(s.flag); f.mapq = P<uint8_t>(s.mapq); f.hp = P<uint8_t>(s.hp);
+    f.cigar_off = P<int32_t>(s.cigar_off); f.cigar = P<uint32_t>(s.cigar); f.seq_off = P<int64_t>(s.seq_off);
+    f.seq = P<uint8_t>(s.seq);
+    CK(cudaEventRecord(s.ev[0], st));
+    CK(cudaEventRecord(s.ev_bam[4], st));
+    CK(cudaMemsetAsync(s.cigar_off.p, 0, 4, st));
+    CK(cudaMemsetAsync(s.seq_off.p, 0, 8, st));
+    if (h.n_reads > 0) {
+        const int64_t blocks = (f.n_slots * 32 + 255) / 256;
+        c3rbgzf::k_rec_write<<<(unsigned)(blocks < ctx->sm_count * 16 ? blocks : ctx->sm_count * 16), 256, 0, st>>>(f);
+        ++s.launches;
+    }
+    CK(cudaEventRecord(s.ev_bam[5], st));
+    const int64_t R = h.n_reads;
+    if (ensure_pin(ctx, s.h_rpos, R * 4) || ensure_pin(ctx, s.h_rflag, R * 2) || ensure_pin(ctx, s.h_rmapq, R) ||
+        ensure_pin(ctx, s.h_rhp, R) || ensure_pin(ctx, s.h_rcoff, (R + 1) * 4) || ensure_pin(ctx, s.h_rcig, h.n_ops * 4) ||
+        ensure_pin(ctx, s.h_rsoff, (R + 1) * 8) || ensure_pin(ctx, s.h_rseq, h.n_seq_bytes)) return C3R_ERR_CUDA;
+    CK(cudaMemcpyAsync(s.h_rcoff.p, s.cigar_off.p, (R + 1) * 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(s.h_rsoff.p, s.seq_off.p, (R + 1) * 8, cudaMemcpyDeviceToHost, st));
+    if (R > 0) {
+        CK(cudaMemcpyAsync(s.h_rpos.p, s.pos.p, R * 4, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(s.h_rflag.p, s.flag.p, R * 2, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(s.h_rmapq.p, s.mapq.p, R, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(s.h_rhp.p, s.hp.p, R, cudaMemcpyDeviceToHost, st));
+    }
+    if (h.n_ops > 0) CK(cudaMemcpyAsync(s.h_rcig.p, s.cigar.p, h.n_ops * 4, cudaMemcpyDeviceToHost, st));
+    if (h.n_seq_bytes > 0) CK(cudaMemcpyAsync(s.h_rseq.p, s.seq.p, h.n_seq_bytes, cudaMemcpyDeviceToHost, st));
+    h.pos = (const int32_t*)s.h_rpos.p; h.flag = (const uint16_t*)s.h_rflag.p; h.mapq = (const uint8_t*)s.h_rmapq.p;
+    h.hp = (const uint8_t*)s.h_rhp.p; h.cigar_off = (const int32_t*)s.h_rcoff.p; h.cigar = (const uint32_t*)s.h_rcig.p;
+    h.seq_off = (const int64_t*)s.h_rsoff.p; h.seq = (const uint8_t*)s.h_rseq.p;
+    return 0;
+}
+
+// The parse counts of a device fetch are on the host: the first error before the first stop fails the ticket,
+// otherwise the read buffers are sized from the counts and the rest of the chunk is queued
+static int advance_parse(c3r_ctx* ctx, Slot& s) {
+    const c3rbgzf::FetchSc& sc = *(const c3rbgzf::FetchSc*)s.h_fsc.p;
+    if (sc.err_key < sc.stop_key) return fail(ctx, C3R_ERR_ARG, fetch_err_text((int)(sc.err_key & 7)));
+    memset(&s.h_reads, 0, sizeof s.h_reads);
+    s.h_reads.n_reads = sc.n_reads;
+    s.h_reads.n_ops = sc.n_ops;
+    s.h_reads.n_seq_bytes = sc.n_bases / 2;
+    if (sc.n_ops >= (1LL << 31)) return fail(ctx, C3R_ERR_CAPACITY, "more than 2^31 CIGAR operations in one chunk");
+    return queue_chunk(ctx, s, &s.h_reads, true, s.ref_host, s.ref_start1, s.ref_len, s.region_start1, s.region_end1,
+                       s.has_filter ? &s.flt : nullptr);
 }
 
 // Queue stage B of a ticket whose stage A counts have arrived (block: wait for them).  Errors of this deferred part
 // are kept in the slot and reported by c3r_wait(ticket).
 static int advance(c3r_ctx* ctx, Slot& s, bool block) {
+    if (s.in_use && s.pending_parse) {               // a device fetch: its parse counts first
+        if (!block && cudaEventQuery(s.ev_parse) == cudaErrorNotReady) return 0;
+        const auto t0 = std::chrono::steady_clock::now();
+        int rc = 0;
+        { cudaError_t e = cudaEventSynchronize(s.ev_parse); if (e != cudaSuccess) rc = fail(ctx, C3R_ERR_CUDA, cudaGetErrorString(e)); }
+        s.pending_parse = false;
+        if (!rc) rc = advance_parse(ctx, s);
+        if (rc) { cudaStreamSynchronize(s.st_a); cudaStreamSynchronize(s.st); s.pending_b = false; s.deferred_rc = rc; s.deferred_err = ctx->err; }
+        ctx->t_phase[4] += std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+        return 0;                                    // stage A is queued: its counts come later
+    }
     if (!s.in_use || !s.pending_b) return 0;
     if (!block) {
         const cudaError_t q = cudaEventQuery(s.ev_cnt);
@@ -816,11 +1102,13 @@ static void advance_all(c3r_ctx* ctx, bool block, uint64_t block_upto) {
         Slot* next = nullptr;
         for (int i = 0; i < N_SLOTS; ++i) {
             Slot& s = ctx->slots[i];
-            if (s.in_use && s.pending_b && (!next || s.order < next->order)) next = &s;
+            if (s.in_use && (s.pending_b || s.pending_parse) && (!next || s.order < next->order)) next = &s;
         }
         if (!next) return;
+        const bool parse = next->pending_parse;
         advance(ctx, *next, block && next->order <= block_upto);
-        if (next->pending_b) return;                 // not ready yet (non-blocking): the later ones wait their turn
+        if (parse && !next->pending_parse) continue;  // its stage A is queued now: take its counts in the next round
+        if (next->pending_b || next->pending_parse) return;   // not ready yet (non-blocking): the later ones wait their turn
     }
 }
 
@@ -902,12 +1190,44 @@ int c3r_wait_calls(c3r_ctx* ctx, c3r_ticket ticket, const c3r_call** calls, int6
     return C3R_OK;
 }
 
+int c3r_wait_reads(c3r_ctx* ctx, c3r_ticket ticket, c3r_reads* out, float* device_ms) {
+    if (!ctx || !out || ticket < 0 || ticket >= N_SLOTS) return C3R_ERR_ARG;
+    Slot& s = ctx->slots[ticket];
+    if (!s.in_use || !s.has_result) return fail(ctx, C3R_ERR_STATE, "c3r_wait_reads needs a ticket c3r_wait has returned");
+    if (!s.bam) return fail(ctx, C3R_ERR_STATE, "the ticket was submitted from host reads (c3r_submit_chunk)");
+    CK(cudaSetDevice(ctx->device));
+    CK(cudaStreamSynchronize(s.st_a));
+    *out = s.h_reads;
+    if (device_ms) {
+        float ms[3];
+        if (int rc = c3r_wait_reads_stages(ctx, ticket, ms)) return rc;
+        *device_ms = ms[0] + ms[1] + ms[2];
+    }
+    return C3R_OK;
+}
+
+int c3r_wait_reads_stages(c3r_ctx* ctx, c3r_ticket ticket, float stage_ms[3]) {
+    if (!ctx || !stage_ms || ticket < 0 || ticket >= N_SLOTS) return C3R_ERR_ARG;
+    Slot& s = ctx->slots[ticket];
+    if (!s.in_use || !s.has_result) return fail(ctx, C3R_ERR_STATE, "c3r_wait_reads_stages needs a ticket c3r_wait has returned");
+    if (!s.bam) return fail(ctx, C3R_ERR_STATE, "the ticket was submitted from host reads (c3r_submit_chunk)");
+    CK(cudaSetDevice(ctx->device));
+    float w = 0.f;
+    CK(cudaEventElapsedTime(&stage_ms[0], s.ev_bam[0], s.ev_bam[1]));
+    CK(cudaEventElapsedTime(&stage_ms[1], s.ev_bam[1], s.ev_bam[2]));
+    CK(cudaEventElapsedTime(&stage_ms[2], s.ev_bam[2], s.ev_bam[3]));
+    CK(cudaEventElapsedTime(&w, s.ev_bam[4], s.ev_bam[5]));
+    stage_ms[2] += w;
+    return C3R_OK;
+}
+
 int c3r_release(c3r_ctx* ctx, c3r_ticket ticket) {
     if (!ctx || ticket < 0 || ticket >= N_SLOTS) return C3R_ERR_ARG;
     Slot& s = ctx->slots[ticket];
     if (s.in_use) { cudaSetDevice(ctx->device); cudaStreamSynchronize(s.st_a); cudaStreamSynchronize(s.st); }
     s.in_use = false;
     s.pending_b = false;                             // released before its stage B was queued: nothing more to run
+    s.pending_parse = false;
     s.deferred_rc = 0;
     s.has_result = false;
     return C3R_OK;

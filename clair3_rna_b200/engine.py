@@ -38,6 +38,8 @@ class ChunkResult:
     launches: int = 0
     calls: np.ndarray | None = None   # lib.CALL_DTYPE [n]: call records (Engine(device_calls=True)), else None
     call_ms: float = 0.0              # device time of k_call
+    reads: ReadBatch | None = None    # the records parsed on the GPU (Engine.submit_bam), else None
+    bam_ms: float = 0.0               # device time of the parse stages (submit_bam)
 
     @property
     def n_cand(self) -> int:
@@ -90,6 +92,7 @@ class Engine:
             raise C3RError("c3r_create: %s (rc=%d)" % (msg, rc))
         self._keep = {}
         self._calls_of = {}                          # ticket -> records on when it was submitted
+        self._bam_of = {}                            # ticket -> contig of a submit_bam
         self.device_calls = False
         self.set_device_calls(device_calls)
 
@@ -155,21 +158,29 @@ class Engine:
             self._keep[int(t.value)] = (arrs, ref)       # the call only queues the copies: inputs live until wait()
             self._calls_of[int(t.value)] = self.device_calls
             return int(t.value)
-        f = L.SiteFilter()
-        keep = []
-        for key, field, width in (("pileup_bed", "pileup_bed", 2), ("confident", "confident_bed", 2), ("known", "known_sites", 1)):
-            a = site_filter.get(key)
-            if a is None:
-                setattr(f, "n_" + field, -1)
-                continue
-            a = np.ascontiguousarray(a, np.int32).reshape(-1, width)
-            keep.append(a)
-            setattr(f, field, a.ctypes.data if a.size else None)
-            setattr(f, "n_" + field, a.shape[0])
+        f, keep = _site_filter(site_filter)
         self._check(self.lib.c3r_submit_chunk_filtered(self.ctx, C.byref(rd), rp, ref_start1, rn, region_start1,
                                                        region_end1, C.byref(f), C.byref(t)), "c3r_submit_chunk_filtered")
         self._keep[int(t.value)] = (arrs, ref, keep)
         self._calls_of[int(t.value)] = self.device_calls
+        return int(t.value)
+
+    def submit_bam(self, raw, ref, ref_start1: int, region_start1: int, region_end1: int, site_filter=None) -> int:
+        """submit() of the records of a raw fetch (bam.BamFile.fetch_raw), inflated and parsed on the GPU; wait()
+        returns them as ChunkResult.reads.  `raw` and `ref` must stay unchanged until wait()."""
+        t = C.c_int64(-1)
+        if ref is None:
+            rp, rn = None, 0
+        else:
+            ref = np.ascontiguousarray(ref, np.uint8)
+            rp, rn = ref.ctypes.data, int(ref.size)
+        f, keep = _site_filter(site_filter) if site_filter is not None else (None, [])
+        self._check(self.lib.c3r_submit_bam_chunk(self.ctx, C.byref(raw.raw), rp, ref_start1, rn, region_start1,
+                                                  region_end1, C.byref(f) if f is not None else None, C.byref(t)),
+                    "c3r_submit_bam_chunk")
+        self._keep[int(t.value)] = (raw, ref, keep)
+        self._calls_of[int(t.value)] = self.device_calls
+        self._bam_of[int(t.value)] = raw.contig
         return int(t.value)
 
     def wait(self, ticket: int, release: bool = True, copy: bool = True) -> ChunkResult:
@@ -179,6 +190,7 @@ class Engine:
         stay valid until release(ticket); the ticket is then NOT released here."""
         r = L.Result()
         calls_on = self._calls_of.pop(ticket, False)
+        bam_contig = self._bam_of.pop(ticket, None)
         try:
             self._check(self.lib.c3r_wait(self.ctx, ticket, C.byref(r)), "c3r_wait")
         finally:
@@ -188,6 +200,12 @@ class Engine:
             cp, cn, ms = C.c_void_p(), C.c_int64(0), C.c_float(0)
             self._check(self.lib.c3r_wait_calls(self.ctx, ticket, C.byref(cp), C.byref(cn), C.byref(ms)), "c3r_wait_calls")
             calls, call_ms = _view(cp.value, cn.value, L.CALL_DTYPE, copy), float(ms.value)
+        reads, bam_ms = None, 0.0
+        if bam_contig is not None:
+            from .bam import reads_from
+            rd, ms = L.Reads(), C.c_float(0)
+            self._check(self.lib.c3r_wait_reads(self.ctx, ticket, C.byref(rd), C.byref(ms)), "c3r_wait_reads")
+            reads, bam_ms = reads_from(bam_contig, rd, copy), float(ms.value)
         n, Ct = int(r.n_cand), self.channels
         v = lambda ptr, cnt, dt: _view(ptr, cnt, dt, copy)
         alt_off = v(r.alt_off, n, np.int64)
@@ -201,13 +219,15 @@ class Engine:
             row_pos=v(r.row_pos, r.n_rows, np.int32) if r.row_pos else None,
             row_counts=v(r.row_counts, r.n_rows * Ct, np.int32).reshape(-1, Ct) if r.row_counts else None,
             row_depth=v(r.row_depth, r.n_rows, np.int32) if r.row_depth else None,
-            stage_ms=[float(x) for x in r.stage_ms], launches=int(r.kernel_launches), calls=calls, call_ms=call_ms)
+            stage_ms=[float(x) for x in r.stage_ms], launches=int(r.kernel_launches), calls=calls, call_ms=call_ms,
+            reads=reads, bam_ms=bam_ms)
         if release and copy:
             self.lib.c3r_release(self.ctx, ticket)
         return out
 
     def release(self, ticket: int):
         self._keep.pop(ticket, None)
+        self._bam_of.pop(ticket, None)
         self._calls_of.pop(ticket, None)
         self.lib.c3r_release(self.ctx, ticket)
 
@@ -246,6 +266,22 @@ class Engine:
             a = a.transpose(0, 4, 1, 2, 3, 5).reshape(tiles * 128, 33, kb * 64)
             return a[:n_sites].astype(np.float32)
         return buf.view(np.float32).reshape(tiles * 128, 128)[:n_sites]
+
+
+def _site_filter(site_filter):
+    """c3r_site_filter over a site_filter dict (Engine.submit) and the arrays it points at"""
+    f = L.SiteFilter()
+    keep = []
+    for key, field, width in (("pileup_bed", "pileup_bed", 2), ("confident", "confident_bed", 2), ("known", "known_sites", 1)):
+        a = site_filter.get(key)
+        if a is None:
+            setattr(f, "n_" + field, -1)
+            continue
+        a = np.ascontiguousarray(a, np.int32).reshape(-1, width)
+        keep.append(a)
+        setattr(f, field, a.ctypes.data if a.size else None)
+        setattr(f, "n_" + field, a.shape[0])
+    return f, keep
 
 
 class PinnedPool:

@@ -76,13 +76,33 @@ class SiteFilter(C.Structure):
                 ("known_sites", C.c_void_p), ("n_known_sites", C.c_int64)]
 
 
+class BgzfBlock(C.Structure):
+    """c3r_bgzf_block (include/c3r_b200.h)"""
+    _fields_ = [("coff", C.c_int64), ("uoff", C.c_int64), ("csize", C.c_int32), ("usize", C.c_int32),
+                ("window", C.c_int32), ("reserved", C.c_int32)]
+
+
+class BamWindow(C.Structure):
+    """c3r_bam_window (include/c3r_b200.h)"""
+    _fields_ = [("ubase", C.c_int64), ("usize", C.c_int64), ("ubeg", C.c_int64), ("uend", C.c_int64),
+                ("first_block", C.c_int32), ("n_blocks", C.c_int32), ("status", C.c_int32), ("reserved", C.c_int32)]
+
+
+class BamRaw(C.Structure):
+    """c3r_bam_raw (include/c3r_b200.h)"""
+    _fields_ = [("tid", C.c_int32), ("n_windows", C.c_int32), ("beg", C.c_int64), ("end", C.c_int64),
+                ("n_blocks", C.c_int64), ("n_bytes", C.c_int64), ("n_ubytes", C.c_int64), ("data", C.c_void_p),
+                ("blocks", C.c_void_p), ("windows", C.c_void_p)]
+
+
 EXPORTS = ["c3r_abi_version", "c3r_default_params", "c3r_create", "c3r_destroy", "c3r_last_error",
            "c3r_set_weights", "c3r_set_reference", "c3r_submit_chunk", "c3r_submit_chunk_filtered", "c3r_wait", "c3r_release", "c3r_rerun_resident", "c3r_forward", "c3r_debug_fetch",
            "c3r_bam_open", "c3r_bam_close", "c3r_bam_error", "c3r_bam_n_ref", "c3r_bam_ref_name", "c3r_bam_ref_len",
            "c3r_bam_header_text", "c3r_bam_idxstats", "c3r_bam_fetch", "c3r_bam_write",
            "c3r_decode_vcf", "c3r_free_text", "c3r_debug_format_fixed", "c3r_vcf_write_bgzf",
            "c3r_host_alloc", "c3r_host_free", "c3r_fasta_fetch",
-           "c3r_enable_calls", "c3r_wait_calls", "c3r_format_vcf", "c3r_debug_decide_calls"]
+           "c3r_enable_calls", "c3r_wait_calls", "c3r_format_vcf", "c3r_debug_decide_calls",
+           "c3r_bam_fetch_raw", "c3r_submit_bam_chunk", "c3r_wait_reads", "c3r_wait_reads_stages", "c3r_debug_inflate"]
 
 _lib = None
 
@@ -144,6 +164,13 @@ def load():
                                    C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
     lib.c3r_debug_decide_calls.argtypes = [C.POINTER(Result), C.POINTER(Reads), C.c_void_p, C.c_int64, C.c_int64,
                                            C.c_void_p]
+    lib.c3r_bam_fetch_raw.argtypes = [C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_void_p, C.c_int64,
+                                      C.POINTER(BamRaw)]
+    lib.c3r_submit_bam_chunk.argtypes = [C.c_void_p, C.POINTER(BamRaw), C.c_void_p, C.c_int64, C.c_int64, C.c_int64,
+                                         C.c_int64, C.POINTER(SiteFilter), C.POINTER(C.c_int64)]
+    lib.c3r_wait_reads.argtypes = [C.c_void_p, C.c_int64, C.POINTER(Reads), C.POINTER(C.c_float)]
+    lib.c3r_wait_reads_stages.argtypes = [C.c_void_p, C.c_int64, C.POINTER(C.c_float)]
+    lib.c3r_debug_inflate.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.POINTER(C.c_int64)]
     lib.c3r_host_alloc.argtypes = [C.POINTER(C.c_void_p), C.c_int64]
     lib.c3r_host_free.argtypes = [C.c_void_p]
     lib.c3r_host_free.restype = None

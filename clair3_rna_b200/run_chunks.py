@@ -48,19 +48,24 @@ def chunk_size_bytes():
     return P.CHUNK_SIZE + 2 * P.EXPAND_REFERENCE_REGION + 4 * P.NO_OF_POSITIONS + 64
 
 
+BAM_BUFFER_BYTES = 64 << 20                         # page-locked buffer of a chunk's compressed BAM bytes (device_bam)
+
+
 def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, world=1, phased=False, padding=False,
         snp_min_af=P.SNP_MIN_AF, indel_min_af=P.INDEL_MIN_AF, min_coverage=P.MIN_COVERAGE, min_mq=P.MIN_MQ,
         qual=P.QUAL_CUT_OFF, sample_name="SAMPLE", gather=None, stats=None, bed_fn=None, vcf_fn=None, head_tail=False,
         merge_qual=None, show_ref=True, rediportal_fn=None, rediportal_tags=None, output_no_tagging=None,
         compress_vcf=False, engine=None, loader_threads=2, native_threads=0, merge=True, cmdline=None,
-        device_calls=False):
+        device_calls=False, device_bam=False):
     """merge_qual / show_ref / rediportal_*: the options of the merge stage (sharder.sort_vcf = sort_vcf_from of the
     reference); the defaults keep every row as the chunks produced it.  engine: an Engine to reuse (its parameters and
     weights are then the caller's business); loader_threads: BAM / FASTA readers working ahead of the GPU;
     native_threads: threads of each BGZF inflate and of the row decoder (0 = all cores - give every rank its share
     when several ranks run on one host).  device_calls: decide the genotypes on the GPU (call records, k_call) and
     leave only the formatting to the decoder threads (c3r_format_vcf); the rows are the same.  A caller's engine
-    gets its own device_calls setting back when the run ends."""
+    gets its own device_calls setting back when the run ends.  device_bam: the loader threads only read the compressed
+    BAM blocks of a chunk (BamFile.fetch_raw, into page-locked buffers) and the GPU inflates and parses them
+    (Engine.submit_bam); the rows are the same."""
     from .bam import BamFile
     from .engine import Engine, PinnedPool, decode_vcf_rows, format_vcf_rows
     fai = fasta.read_fai(ref_fn)
@@ -88,6 +93,7 @@ def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, wo
     # host seconds per stage of this rank's loop (the GPU works under all of them but `wait`)
     tm = dict(fetch=0.0, ref=0.0, submit=0.0, wait=0.0, decode=0.0)
     call_ms = 0.0                                    # device time of k_call (device_calls)
+    bam_ms = 0.0                                     # device time of the BAM parse stages (device_bam)
 
     import threading
     tls = threading.local()
@@ -99,6 +105,15 @@ def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, wo
         if pool is not None:
             pool.close()
         pool = eng._ref_pool = PinnedPool(6 + 2 * max(1, loader_threads), chunk_size_bytes())
+    # compressed BAM bytes of a chunk (device_bam): tickets in flight (2) + loaded ahead; a larger chunk is read into
+    # ordinary memory
+    bam_pool = None
+    if device_bam:
+        bam_pool = getattr(eng, "_bam_pool", None)
+        if bam_pool is None or len(bam_pool.ptrs) < 4 + max(1, loader_threads):
+            if bam_pool is not None:
+                bam_pool.close()
+            bam_pool = eng._bam_pool = PinnedPool(4 + max(1, loader_threads), BAM_BUFFER_BYTES)
 
     def reader():
         # one BAM handle per loader thread (a handle serves one fetch at a time)
@@ -119,7 +134,15 @@ def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, wo
         if plan is None:
             return None
         t = time.time()
-        batch = reader().fetch(name, plan.start1, plan.end1)
+        bbuf = None
+        if device_bam:
+            bbuf = bam_pool.get(0)
+            batch = reader().fetch_raw(name, plan.start1, plan.end1, buf=bbuf)
+            if batch.data is not bbuf:               # larger than the pool's buffers: read into ordinary memory
+                bam_pool.put(bbuf)
+                bbuf = None
+        else:
+            batch = reader().fetch(name, plan.start1, plan.end1)
         tm["fetch"] += time.time() - t
         t = time.time()
         pbuf = pool.get(plan.ref_end1 - plan.ref_start1 + 1)
@@ -128,7 +151,7 @@ def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, wo
         else:
             ref = fasta.fetch(ref_fn, fai, name, plan.ref_start1, plan.ref_end1)
         tm["ref"] += time.time() - t
-        return name, batch, ref, plan, pbuf
+        return name, batch, ref, plan, (pbuf, bbuf)
 
     # Three host stages run side by side (the native calls release the GIL): a loader thread fetches + inflates the
     # BAM blocks and reads the reference of the shards ahead, this thread submits shard i+1 and waits for shard i,
@@ -153,7 +176,7 @@ def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, wo
         rows = (format_vcf_rows if device_calls else decode_vcf_rows)(res, pbatch, pref, prs1, pname, qual=qual,
                                                                       threads=dec_threads)
         tm["decode"] += time.time() - t
-        pool.put(pbuf)                               # the reference window is free again
+        pool.put(pbuf[0])                            # the reference window is free again
         return rows
 
     def retire(block):
@@ -184,7 +207,8 @@ def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, wo
                 name, batch, ref, plan, pbuf = got
                 retire(len(decoding) >= 2)           # keep a ticket free for this submit
                 t = time.time()
-                nxt = (i, eng.submit(batch, ref, plan.ref_start1, plan.start1, plan.end1, plan.site_filter()),
+                sub = eng.submit_bam if device_bam else eng.submit
+                nxt = (i, sub(batch, ref, plan.ref_start1, plan.start1, plan.end1, plan.site_filter()),
                        name, batch, ref, plan.ref_start1, pbuf)
                 tm["submit"] += time.time() - t
                 submit_ms.append(1e3 * (time.time() - t))
@@ -195,6 +219,10 @@ def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, wo
             tm["wait"] += time.time() - t
             n_cand += res.n_cand
             call_ms += res.call_ms
+            if device_bam:                           # the compressed bytes are on the device: the buffer is free
+                bam_ms += res.bam_ms
+                bam_pool.put(ppbuf[1])
+                pbatch = res.reads                   # the records the GPU parsed, valid until release
             decoding.append((j, ticket, dec.submit(decode, res, pbatch, pref, prs1, pname, ppbuf)))
         retire(False)
         pending = nxt
@@ -205,6 +233,9 @@ def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, wo
     if engine is None:
         pool.close()
         eng._ref_pool = None
+        if bam_pool is not None:
+            bam_pool.close()
+            eng._bam_pool = None
         eng.close()
     elif eng.device_calls != calls_before:
         eng.set_device_calls(calls_before)
@@ -213,7 +244,8 @@ def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, wo
         r.close()
     if stats is not None:
         stats.update(shards=len(mine), candidates=n_cand, seconds=time.time() - t0, host_seconds=tm, submit_ms=submit_ms,
-                     cost=sum(costs[i] for i in mine), total_shards=len(shards), call_device_ms=call_ms)
+                     cost=sum(costs[i] for i in mine), total_shards=len(shards), call_device_ms=call_ms,
+                     bam_device_ms=bam_ms)
     if not merge:                                    # the caller only wants this rank's loop (timing passes)
         return None
     if world > 1:
@@ -290,6 +322,8 @@ def main(argv=None):
     ap.add_argument("--enable_variant_calling_at_sequence_head_and_tail", action="store_true")
     ap.add_argument("--device_calls", action="store_true",
                     help="decide the genotypes on the GPU and only format the rows on the host (same output)")
+    ap.add_argument("--device_bam", action="store_true",
+                    help="inflate and parse the BAM blocks of each chunk on the GPU (same output)")
     a = ap.parse_args(argv)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -313,7 +347,8 @@ def main(argv=None):
         compress_vcf=a.compress_vcf,
         cmdline=" ".join(sys.argv) if argv is None else " ".join(["run_chunks"] + list(argv)),
         sample_name=a.sampleName, stats=stats, bed_fn=a.bed_fn, vcf_fn=a.genotyping_mode_vcf_fn,
-        head_tail=a.enable_variant_calling_at_sequence_head_and_tail, device_calls=a.device_calls)
+        head_tail=a.enable_variant_calling_at_sequence_head_and_tail, device_calls=a.device_calls,
+        device_bam=a.device_bam)
     print("[rank %d] %d shards, %d candidates in %.2f s" % (rank, stats["shards"], stats["candidates"], stats["seconds"]),
           file=sys.stderr)
     if world > 1:

@@ -323,6 +323,68 @@ const char* c3r_bam_header_text(c3r_bam* bam);
 int c3r_bam_idxstats(c3r_bam* bam, int tid, int64_t* n_mapped, int64_t* n_unmapped);
 int c3r_bam_fetch(c3r_bam* bam, int tid, int64_t start1, int64_t end1, c3r_reads* out);
 
+/* ------------------------------------------------------------------------------------------
+ * Device BAM reading: the host does c3r_bam_fetch's index query and reads the compressed bytes; the GPU inflates the
+ * BGZF blocks, finds and checks the records and writes the flat arrays c3r_bam_fetch would return, bit for bit, with
+ * the same status for every input the host fetch rejects (csrc/bgzf.cuh).
+ *
+ * A window is one merged index chunk: the BGZF blocks c3r_bam_fetch inflates for it, read back to back into the
+ * caller's buffer.  Its records start at ubeg of its inflated bytes and continue while a record's length field ends
+ * at or before uend; a block shared by two windows is read (and inflated) once for each. */
+typedef struct {
+    int64_t coff;              /* offset of the block in c3r_bam_raw.data                                  */
+    int64_t uoff;              /* offset of its inflated bytes in the fetch's inflated bytes (n_ubytes)     */
+    int32_t csize;             /* compressed size (BSIZE + 1)                                              */
+    int32_t usize;             /* ISIZE                                                                    */
+    int32_t window;            /* window of the block                                                      */
+    int32_t reserved;
+} c3r_bgzf_block;
+
+typedef struct {
+    int64_t ubase;             /* offset of the window's inflated bytes in the fetch's inflated bytes      */
+    int64_t usize;             /* inflated bytes of the window                                             */
+    int64_t ubeg, uend;        /* record walk bounds within the window                                     */
+    int32_t first_block, n_blocks;
+    int32_t status;            /* 0, or why the window could not be read (its blocks are then absent):
+                                  2 corrupt BGZF header, 3 block larger than 64 KiB, 4 short read; the error
+                                  is reported only if the fetch gets that far                               */
+    int32_t reserved;
+} c3r_bam_window;
+
+typedef struct {
+    int32_t tid;
+    int32_t n_windows;
+    int64_t beg, end;          /* 0-based half-open region of the fetch                                    */
+    int64_t n_blocks;
+    int64_t n_bytes;           /* compressed bytes in data                                                 */
+    int64_t n_ubytes;          /* inflated bytes of all windows                                            */
+    const uint8_t* data;
+    const c3r_bgzf_block* blocks;    /* [n_blocks], in window order                                        */
+    const c3r_bam_window* windows;   /* [n_windows]                                                        */
+} c3r_bam_raw;
+
+/* c3r_bam_fetch without the inflate and the record walk: the index query, and the compressed blocks of every
+ * window read into buf (cap bytes; page-locked memory from c3r_host_alloc makes the submit a pure DMA).  The block
+ * and window tables belong to the handle until its next fetch.  C3R_ERR_CAPACITY with the needed size in
+ * out->n_bytes when cap is too small. */
+int c3r_bam_fetch_raw(c3r_bam* bam, int tid, int64_t start1, int64_t end1, uint8_t* buf, int64_t cap, c3r_bam_raw* out);
+
+/* c3r_submit_chunk_filtered for the records of a raw fetch, parsed on the device.  raw->data and the tables must
+ * stay unchanged until c3r_wait returns.  The parse runs ahead of the chunk's stages: a later call into the library
+ * sizes the read buffers from its counts and queues the rest.  A corrupt BAM makes c3r_wait return C3R_ERR_ARG
+ * (the host fetch's message in c3r_last_error) and gives the ticket back. */
+int c3r_submit_bam_chunk(c3r_ctx* ctx, const c3r_bam_raw* raw, const uint8_t* ref, int64_t ref_start1, int64_t ref_len,
+                         int64_t region_start1, int64_t region_end1, const c3r_site_filter* filter, c3r_ticket* ticket);
+/* The device-parsed records of a ticket from c3r_submit_bam_chunk, in pinned library memory valid until
+ * c3r_release; call after c3r_wait.  device_ms (may be NULL): device time of the parse stages (inflate, record
+ * boundaries, parse, offsets, write).  C3R_ERR_STATE for a ticket submitted from host reads. */
+int c3r_wait_reads(c3r_ctx* ctx, c3r_ticket ticket, c3r_reads* out, float* device_ms);
+/* The same stages split: [0] inflate, [1] record boundaries, [2] parse + offsets + write (ms). */
+int c3r_wait_reads_stages(c3r_ctx* ctx, c3r_ticket ticket, float stage_ms[3]);
+/* test hook: the device's DEFLATE decoder and CRC check run on the host over one BGZF block of n bytes
+ * (header, payload, trailer) into out (cap bytes); *n_out receives ISIZE.  C3R_ERR_ARG on any failure.  No GPU. */
+int c3r_debug_inflate(const uint8_t* block, int64_t n, uint8_t* out, int64_t cap, int64_t* n_out);
+
 /* Writes a coordinate-sorted BAM and <path>.bai from flat records, batches[r] = records of
  * reference r (NULL = none): fixtures for the reader and for the drop-in entry point (there is
  * no samtools in the build image).  level: zlib level, -1 = default.  header_text NULL: minimal
