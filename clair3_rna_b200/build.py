@@ -7,7 +7,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libc3r_b200.so")
 SOURCES = ["c3r_abi.cu", "bam_io.cpp", "decode.cpp", "fasta_io.cpp"]
-HEADERS = ["scan.cuh", "pileup.cuh", "call.cuh", "bam_rec.cuh", "bgzf.cuh", "nn_fp32.cuh", "nn_tc.cuh", "nn_lstm2f.cuh", "nn_sched.h", "tc_ptx.cuh", os.path.join("..", "..", "include", "c3r_b200.h")]
+HEADERS = ["scan.cuh", "pileup.cuh", "call.cuh", "vcf_row.cuh", "bam_rec.cuh", "bgzf.cuh", "nn_fp32.cuh", "nn_tc.cuh", "nn_lstm2f.cuh", "nn_sched.h", "tc_ptx.cuh", os.path.join("..", "..", "include", "c3r_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared", "-lcuda", "-lz", "-lpthread"]
 

@@ -22,6 +22,7 @@
 #include "nn_fp32.cuh"
 #include "nn_tc.cuh"
 #include "call.cuh"
+#include "vcf_row.cuh"
 #include "bgzf.cuh"
 
 using namespace c3r;
@@ -49,6 +50,15 @@ struct Slot {
     cudaEvent_t ev_alt = nullptr;
     cudaEvent_t ev_call[2] = {};      // around k_call
     bool calls = false;               // call records for this ticket (c3r_enable_calls when it was submitted)
+    // VCF text for this ticket (c3r_set_vcf when it was submitted): k_vcf_len, the offsets scan and k_vcf_write after
+    // k_call; the totals (bytes, rows) land in the scalars [8], [9]
+    bool vcf = false;
+    int32_t vcf_show_ref = 1, vcf_q_min = 0;
+    std::string vcf_contig;
+    int64_t vcf_row_max = 0;
+    cudaEvent_t ev_vcf[2] = {};       // around the text kernels
+    Buf d_vlen, d_voff, d_text, d_contig;
+    Pin h_text;
     // inputs
     Buf pos, flag, mapq, hp, cigar_off, cigar, seq_off, seq, ref;
     // per read/op
@@ -127,6 +137,13 @@ struct c3r_ctx {
     double t_phase[8] = {};   // C3R_TIMING: host seconds of submit's phases (printed by c3r_destroy)
     int64_t n_submit = 0;
     bool calls = false;       // c3r_enable_calls: tickets submitted from now on make call records
+    // c3r_set_vcf: tickets submitted from now on print their VCF rows on the device
+    bool vcf = false;
+    int32_t vcf_show_ref = 1, vcf_q_min = 0;
+    std::string vcf_contig;
+    Buf vcf_qtab;             // QUAL thresholds (c3rvcf::qual_table), uploaded by the first c3r_set_vcf that turns text on
+    int32_t vcf_q_n = 0;
+    char nan_text[8] = {}, ninf_text[8] = {};
     Buf fwd_in, fwd_out;      // c3r_forward staging
     cudaStream_t fwd_stream = nullptr;
 };
@@ -294,7 +311,13 @@ int ensure_stage_b(c3r_ctx* ctx, Slot& s) {
     d.alt_cap = 4 * n + d.events_ub + 8;
     if (ensure(ctx, s.alt, (size_t)d.alt_cap * sizeof(AltEntry))) return C3R_ERR_CUDA;
     if (ensure(ctx, s.probs, (size_t)n * 24 * 4)) return C3R_ERR_CUDA;
-    if (s.calls && ensure(ctx, s.d_calls, (size_t)n * sizeof(c3r_call))) return C3R_ERR_CUDA;
+    if ((s.calls || s.vcf) && ensure(ctx, s.d_calls, (size_t)n * sizeof(c3r_call))) return C3R_ERR_CUDA;
+    if (s.vcf) {
+        s.vcf_row_max = c3rvcf::row_max((int64_t)s.vcf_contig.size());
+        if (ensure(ctx, s.d_vlen, (size_t)n * 4) || ensure(ctx, s.d_voff, (size_t)n * 8) ||
+            ensure(ctx, s.d_text, (size_t)n * s.vcf_row_max + 16) || ensure(ctx, s.d_contig, s.vcf_contig.size() + 1))
+            return C3R_ERR_CUDA;
+    }
     d.tensor = P<int32_t>(s.tensor);
     d.alt_off = P<int64_t>(s.alt_off);
     d.alt_n = P<int32_t>(s.alt_n);
@@ -336,7 +359,7 @@ int run_stage_b(c3r_ctx* ctx, Slot& s) {
         L += nl;
     }
     CK(cudaEventRecord(s.ev[7], st));
-    if (s.calls) {
+    if (s.calls || s.vcf) {
         CK(cudaEventRecord(s.ev_call[0], st));
         if (n > 0) {
             const int64_t blocks = (n + 127) / 128;
@@ -344,6 +367,41 @@ int run_stage_b(c3r_ctx* ctx, Slot& s) {
             ++L;
         }
         CK(cudaEventRecord(s.ev_call[1], st));
+    }
+    if (s.vcf) {
+        CK(cudaEventRecord(s.ev_vcf[0], st));
+        if (n > 0) {
+            CK(cudaMemcpyAsync(s.d_contig.p, s.vcf_contig.data(), s.vcf_contig.size(), cudaMemcpyHostToDevice, st));
+            c3rvcf::DevRows r;
+            r.f.contig = P<char>(s.d_contig);
+            r.f.contig_len = (int32_t)s.vcf_contig.size();
+            r.f.q_min = s.vcf_q_min;
+            r.f.ref = d.ref;
+            r.f.ref_start1 = d.ref_start0 + 1;
+            r.f.seq = d.seq;
+            r.f.show_ref = s.vcf_show_ref;
+            memcpy(r.f.nan_text, ctx->nan_text, 8);
+            memcpy(r.f.ninf_text, ctx->ninf_text, 8);
+            r.calls = P<c3r_call>(s.d_calls);
+            r.pos = d.cand_pos;
+            r.depth = d.cand_depth;
+            r.n = n;
+            r.qtab = P<float>(ctx->vcf_qtab);
+            r.q_n = ctx->vcf_q_n;
+            r.len = P<int32_t>(s.d_vlen);
+            r.off = P<long long>(s.d_voff);
+            r.out = P<char>(s.d_text);
+            const int64_t blocks = (n + 127) / 128;
+            c3rvcf::k_vcf_len<<<(unsigned)(blocks < ctx->sm_count * 16 ? blocks : ctx->sm_count * 16), 128, 0, st>>>(r);
+            c3rvcf::OpVcfOff op;
+            op.len = r.len; op.off = r.off; op.n = n;
+            L += 1 + device_scan(op, n, s.scan, s.scan_epoch, (c3rvcf::VcfTotals*)(P<long long>(s.scalars) + 8), st);
+            const int64_t tiles = (n + c3rvcf::VCF_TILE - 1) / c3rvcf::VCF_TILE;
+            c3rvcf::k_vcf_write<<<(unsigned)(tiles < ctx->sm_count * 32 ? tiles : ctx->sm_count * 32), c3rvcf::VCF_TILE,
+                                  c3rvcf::vcf_write_smem(s.vcf_row_max), st>>>(r, s.vcf_row_max);
+            ++L;
+        }
+        CK(cudaEventRecord(s.ev_vcf[1], st));
     }
     CK(cudaGetLastError());
     return 0;
@@ -354,8 +412,8 @@ int queue_d2h(c3r_ctx* ctx, Slot& s) {
     cudaStream_t st = s.st;
     const int64_t n = s.n_cand;
     const int per = WIN * d.C;
-    // alt total: a second tiny readback, taken before the network so it overlaps it
-    CK(cudaMemcpyAsync(s.h_scalars.p, s.scalars.p, 64, cudaMemcpyDeviceToHost, st));
+    // alt total (and the text totals): a second tiny readback, taken before the network so it overlaps it
+    CK(cudaMemcpyAsync(s.h_scalars.p, s.scalars.p, s.vcf ? 80 : 64, cudaMemcpyDeviceToHost, st));
     if (n > 0) {
         if (ensure_pin(ctx, s.h_pos, n * 4) || ensure_pin(ctx, s.h_depth, n * 4) || ensure_pin(ctx, s.h_probs, n * 96) ||
             ensure_pin(ctx, s.h_alt_off, n * 8) || ensure_pin(ctx, s.h_alt_n, n * 4)) return C3R_ERR_CUDA;
@@ -367,6 +425,11 @@ int queue_d2h(c3r_ctx* ctx, Slot& s) {
         if (s.calls) {
             if (ensure_pin(ctx, s.h_calls, (size_t)n * sizeof(c3r_call))) return C3R_ERR_CUDA;
             CK(cudaMemcpyAsync(s.h_calls.p, s.d_calls.p, (size_t)n * sizeof(c3r_call), cudaMemcpyDeviceToHost, st));
+        }
+        if (s.vcf) {                                 // the bound: the size of a copy is fixed when it is queued
+            const size_t bound = (size_t)n * s.vcf_row_max;
+            if (ensure_pin(ctx, s.h_text, bound)) return C3R_ERR_CUDA;
+            CK(cudaMemcpyAsync(s.h_text.p, s.d_text.p, bound, cudaMemcpyDeviceToHost, st));
         }
         if (ctx->prm.keep_tensor) {
             if (ensure_pin(ctx, s.h_tensor, (size_t)n * per * 4)) return C3R_ERR_CUDA;
@@ -457,6 +520,7 @@ int c3r_create(c3r_ctx** out, int device_ordinal, const c3r_params* params) {
         for (int k = 0; k < N_EV; ++k) CK(cudaEventCreate(&s.ev[k]));
         CK(cudaEventCreateWithFlags(&s.ev_alt, cudaEventDisableTiming));
         for (int k = 0; k < 2; ++k) CK(cudaEventCreate(&s.ev_call[k]));
+        for (int k = 0; k < 2; ++k) CK(cudaEventCreate(&s.ev_vcf[k]));
         // spin-wait by default: a blocking-sync event wakes the waiting thread ~0.3 ms late (measured), which delays
         // stage B by as much; C3R_BLOCKING_COUNTS trades that for an idle core while waiting
         CK(cudaEventCreateWithFlags(&s.ev_cnt, cudaEventDisableTiming | (getenv("C3R_BLOCKING_COUNTS") ? cudaEventBlockingSync : 0)));
@@ -494,15 +558,16 @@ void c3r_destroy(c3r_ctx* ctx) {
                      &s.cand_row, &s.cand_pos, &s.cand_depth, &s.tensor, &s.alt_off, &s.alt_n, &s.alt, &s.cur_ref,
                      &s.deleted, &s.probs, &s.scalars, &s.scan_scratch, &s.pbed, &s.cbed, &s.known, &s.covP, &s.xop, &s.d_calls,
                      &s.b_cdata, &s.b_blk, &s.b_win, &s.b_ubuf, &s.b_nrec, &s.b_soff, &s.b_scls, &s.b_skey, &s.b_snops, &s.b_snb,
-                     &s.b_sdst, &s.b_sc};
+                     &s.b_sdst, &s.b_sc, &s.d_vlen, &s.d_voff, &s.d_text, &s.d_contig};
         for (Buf* b : bs) release(*b);
         Pin* ps[] = {&s.h_scalars, &s.h_pos, &s.h_depth, &s.h_probs, &s.h_alt_off, &s.h_alt_n, &s.h_alt, &s.h_tensor,
                      &s.h_row_pos, &s.h_counts, &s.h_row_depth, &s.h_calls, &s.h_fsc, &s.h_rpos, &s.h_rflag, &s.h_rmapq,
-                     &s.h_rhp, &s.h_rcoff, &s.h_rcig, &s.h_rsoff, &s.h_rseq};
+                     &s.h_rhp, &s.h_rcoff, &s.h_rcig, &s.h_rsoff, &s.h_rseq, &s.h_text};
         for (Pin* b : ps) release(*b);
         for (int k = 0; k < N_EV; ++k) if (s.ev[k]) cudaEventDestroy(s.ev[k]);
         if (s.ev_alt) cudaEventDestroy(s.ev_alt);
         for (int k = 0; k < 2; ++k) if (s.ev_call[k]) cudaEventDestroy(s.ev_call[k]);
+        for (int k = 0; k < 2; ++k) if (s.ev_vcf[k]) cudaEventDestroy(s.ev_vcf[k]);
         if (s.ev_cnt) cudaEventDestroy(s.ev_cnt);
         if (s.ev_parse) cudaEventDestroy(s.ev_parse);
         for (int k = 0; k < 6; ++k) if (s.ev_bam[k]) cudaEventDestroy(s.ev_bam[k]);
@@ -515,6 +580,7 @@ void c3r_destroy(c3r_ctx* ctx) {
     release(ctx->ref_res);
     release(ctx->refnib_res);
     release(ctx->thr);
+    release(ctx->vcf_qtab);
     release(ctx->fwd_out);
     tc_release(ctx->tc);
     if (ctx->fwd_stream) cudaStreamDestroy(ctx->fwd_stream);
@@ -606,7 +672,8 @@ int c3r_submit_chunk_filtered(c3r_ctx* ctx, const c3r_reads* rd, const uint8_t* 
 // The slot's scan state (scan.cuh), sized for scans of up to n elements.  Every scan of a slot uses the same layout
 // (aggregates of SCAN_ELEM bytes): the status words of one layout must never lie over the aggregates of another.
 constexpr size_t SCAN_ELEM = 32;
-static_assert(sizeof(ScanElem) <= SCAN_ELEM && sizeof(c3rbgzf::Slot3) <= SCAN_ELEM, "scan aggregates fit the layout");
+static_assert(sizeof(ScanElem) <= SCAN_ELEM && sizeof(c3rbgzf::Slot3) <= SCAN_ELEM && sizeof(c3rvcf::VcfTotals) <= SCAN_ELEM,
+              "scan aggregates fit the layout");
 static int ensure_scan(c3r_ctx* ctx, Slot& s, int64_t n) {
     const size_t elem = SCAN_ELEM;
     // scan state: 256 B of counters, then per tile a status word, an aggregate and an inclusive prefix
@@ -689,6 +756,14 @@ static int check_submit(c3r_ctx* ctx, const uint8_t* ref, int64_t* ref_start1, i
     if (region_end1 < region_start1 || region_start1 < 1) return fail(ctx, C3R_ERR_ARG, "bad region");
     if (region_end1 > 0x7fff0000LL) return fail(ctx, C3R_ERR_CAPACITY, "positions must fit int32");
     return 0;
+}
+
+// the text options of the context, as the ticket in slot s is submitted
+static void take_vcf(c3r_ctx* ctx, Slot& s) {
+    s.vcf = ctx->vcf;
+    s.vcf_show_ref = ctx->vcf_show_ref;
+    s.vcf_q_min = ctx->vcf_q_min;
+    s.vcf_contig = ctx->vcf_contig;
 }
 
 static int free_slot(c3r_ctx* ctx) {
@@ -828,6 +903,7 @@ static int submit_once(c3r_ctx* ctx, const c3r_reads* rd, const uint8_t* ref, in
     s.bam = false;
     s.pending_parse = false;
     s.calls = ctx->calls;
+    take_vcf(ctx, s);
     int rc = queue_chunk(ctx, s, rd, false, ref, ref_start1, ref_len, region_start1, region_end1, ctx->filter);
     if (rc) { cudaStreamSynchronize(s.st_a); cudaStreamSynchronize(s.st); return rc; }
     s.in_use = true;
@@ -899,6 +975,7 @@ int c3r_submit_bam_chunk(c3r_ctx* ctx, const c3r_bam_raw* raw, const uint8_t* re
     Slot& s = ctx->slots[si];
     s.bam = true;
     s.calls = ctx->calls;
+    take_vcf(ctx, s);
     s.ref_host = ref; s.ref_start1 = ref_start1; s.ref_len = ref_len;
     s.region_start1 = region_start1; s.region_end1 = region_end1;
     // the filter is read during the call (as c3r_submit_chunk_filtered's): the slot keeps a copy for the deferred part
@@ -1161,7 +1238,8 @@ int c3r_wait(c3r_ctx* ctx, c3r_ticket ticket, c3r_result* res) {
     }
     for (int k = 0; k < 8; ++k) {
         float ms = 0.f;
-        cudaEventElapsedTime(&ms, k == 7 && s.calls ? s.ev_call[1] : s.ev[k], s.ev[k + 1]);   // D2H: after k_call
+        // D2H: after k_call and the text kernels
+        cudaEventElapsedTime(&ms, k != 7 ? s.ev[k] : s.vcf ? s.ev_vcf[1] : s.calls ? s.ev_call[1] : s.ev[7], s.ev[k + 1]);
         r.stage_ms[k] = ms;
     }
     r.kernel_launches = s.launches;
@@ -1186,6 +1264,49 @@ int c3r_wait_calls(c3r_ctx* ctx, c3r_ticket ticket, const c3r_call** calls, int6
     if (device_ms) {
         CK(cudaSetDevice(ctx->device));
         CK(cudaEventElapsedTime(device_ms, s.ev_call[0], s.ev_call[1]));
+    }
+    return C3R_OK;
+}
+
+int c3r_set_vcf(c3r_ctx* ctx, const c3r_vcf_options* opts) {
+    if (!ctx || !opts) return C3R_ERR_ARG;
+    if (!opts->on) { ctx->vcf = false; return C3R_OK; }
+    if (!opts->contig) return fail(ctx, C3R_ERR_ARG, "c3r_set_vcf: no contig name");
+    const size_t len = strlen(opts->contig);
+    if (len > (size_t)c3rvcf::CONTIG_MAX) return fail(ctx, C3R_ERR_ARG, "c3r_set_vcf: contig name longer than 1024 bytes");
+    if (!ctx->vcf_q_n) {                             // once per context: the QUAL table, the texts, k_vcf_write's shared memory
+        CK(cudaSetDevice(ctx->device));
+        int32_t q_n = 0;
+        const float* t = c3rvcf::qual_table(&q_n);
+        if (ensure(ctx, ctx->vcf_qtab, (size_t)q_n * sizeof(float))) return C3R_ERR_CUDA;
+        CK(cudaMemcpy(ctx->vcf_qtab.p, t, (size_t)q_n * sizeof(float), cudaMemcpyHostToDevice));
+        c3rvcf::special_texts(ctx->nan_text, ctx->ninf_text);
+        CK(cudaFuncSetAttribute(c3rvcf::k_vcf_write, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                (int)c3rvcf::vcf_write_smem(c3rvcf::row_max(c3rvcf::CONTIG_MAX))));
+        ctx->vcf_q_n = q_n;
+    }
+    ctx->vcf = true;
+    ctx->vcf_show_ref = opts->show_ref != 0;
+    ctx->vcf_q_min = c3rvcf::qual_q_min(opts->qual_cut);
+    ctx->vcf_contig.assign(opts->contig, len);
+    return C3R_OK;
+}
+
+int c3r_wait_vcf(c3r_ctx* ctx, c3r_ticket ticket, const char** text, int64_t* n_bytes, int64_t* n_rows, float* device_ms) {
+    if (!ctx || !text || !n_bytes || !n_rows || ticket < 0 || ticket >= N_SLOTS) return C3R_ERR_ARG;
+    Slot& s = ctx->slots[ticket];
+    if (!s.in_use || !s.has_result) return fail(ctx, C3R_ERR_STATE, "c3r_wait_vcf needs a ticket c3r_wait has returned");
+    if (!s.vcf) return fail(ctx, C3R_ERR_STATE, "VCF text was off when this ticket was submitted (c3r_set_vcf)");
+    const int64_t* hs = (const int64_t*)s.h_scalars.p;
+    const int64_t nb = s.n_cand > 0 ? hs[8] : 0, nr = s.n_cand > 0 ? hs[9] : 0;
+    if (nb < 0 || nb > s.n_cand * s.vcf_row_max || nr < 0 || nr > s.n_cand)
+        return fail(ctx, C3R_ERR_CUDA, "VCF text totals out of range");
+    *text = nb > 0 ? (const char*)s.h_text.p : "";
+    *n_bytes = nb;
+    *n_rows = nr;
+    if (device_ms) {
+        CK(cudaSetDevice(ctx->device));
+        CK(cudaEventElapsedTime(device_ms, s.ev_vcf[0], s.ev_vcf[1]));
     }
     return C3R_OK;
 }

@@ -40,6 +40,9 @@ class ChunkResult:
     call_ms: float = 0.0              # device time of k_call
     reads: ReadBatch | None = None    # the records parsed on the GPU (Engine.submit_bam), else None
     bam_ms: float = 0.0               # device time of the parse stages (submit_bam)
+    vcf_text: str | None = None       # the VCF data lines printed on the GPU (Engine(device_vcf=True)), else None
+    vcf_rows: int = 0                 # lines in vcf_text
+    vcf_ms: float = 0.0               # device time of the text kernels
 
     @property
     def n_cand(self) -> int:
@@ -63,8 +66,10 @@ def _view(ptr, n, dtype, copy=True):
 class Engine:
     def __init__(self, device: int = 0, channels: int = 18, *, snp_min_af=P.SNP_MIN_AF, indel_min_af=P.INDEL_MIN_AF,
                  min_coverage=P.MIN_COVERAGE, min_mq=P.MIN_MQ, enable_padding=False, nn_impl=1,
-                 keep_tensor=False, keep_rows=False, enable_head_tail=False, device_calls=False):
-        """device_calls: also decide each candidate's genotype on the GPU (ChunkResult.calls, format_vcf_rows)"""
+                 keep_tensor=False, keep_rows=False, enable_head_tail=False, device_calls=False, device_vcf=False):
+        """device_calls: also decide each candidate's genotype on the GPU (ChunkResult.calls, format_vcf_rows);
+        device_vcf: also print each candidate's VCF row on the GPU (ChunkResult.vcf_text, device_vcf_rows) with the
+        default QUAL cut-off and reference calls shown - set_device_vcf chooses them"""
         self.lib = L.load()
         if self.lib.c3r_abi_version() != 2:
             raise C3RError("ABI version mismatch")
@@ -93,8 +98,12 @@ class Engine:
         self._keep = {}
         self._calls_of = {}                          # ticket -> records on when it was submitted
         self._bam_of = {}                            # ticket -> contig of a submit_bam
+        self._vcf_of = {}                            # ticket -> VCF text on when it was submitted
         self.device_calls = False
         self.set_device_calls(device_calls)
+        self.device_vcf = False
+        self._vcf_opts = None                        # (qual, show_ref) while device_vcf is on
+        self.set_device_vcf(device_vcf)
 
     # ------------------------------------------------------------------
     def _check(self, rc, what):
@@ -117,6 +126,25 @@ class Engine:
         """call records for the tickets submitted from now on (c3r_enable_calls)"""
         self._check(self.lib.c3r_enable_calls(self.ctx, int(bool(on))), "c3r_enable_calls")
         self.device_calls = bool(on)
+
+    def set_device_vcf(self, on: bool, qual=P.QUAL_CUT_OFF, show_ref: bool = True):
+        """VCF rows printed on the GPU for the tickets submitted from now on (c3r_set_vcf), as format_vcf_rows would
+        print them with this qual (None: no LowQual filter) and show_ref; each submit names its own contig"""
+        self._vcf_opts = (qual, bool(show_ref)) if on else None
+        self._set_vcf("")
+        self.device_vcf = bool(on)
+
+    def _set_vcf(self, contig: str):
+        o = L.VcfOptions()
+        o.on = int(self._vcf_opts is not None)
+        if self._vcf_opts is not None:
+            qual, show_ref = self._vcf_opts
+            o.show_ref, o.qual_cut, o.contig = int(show_ref), -1.0 if qual is None else float(qual), contig.encode()
+        self._check(self.lib.c3r_set_vcf(self.ctx, C.byref(o)), "c3r_set_vcf")
+
+    def _submitted(self, ticket: int):
+        self._calls_of[ticket] = self.device_calls
+        self._vcf_of[ticket] = self.device_vcf
 
     def set_weights(self, weights: dict):
         arrs = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in weights.items()}
@@ -146,6 +174,8 @@ class Engine:
                     seq_off=np.ascontiguousarray(batch.seq_off, np.int64), seq=np.ascontiguousarray(batch.seq, np.uint8))
         for k, v in arrs.items():
             setattr(rd, k, v.ctypes.data)
+        if self.device_vcf:
+            self._set_vcf(batch.contig)
         t = C.c_int64(-1)
         if ref is None:
             rp, rn = None, 0
@@ -156,13 +186,13 @@ class Engine:
             self._check(self.lib.c3r_submit_chunk(self.ctx, C.byref(rd), rp, ref_start1, rn,
                                                   region_start1, region_end1, C.byref(t)), "c3r_submit_chunk")
             self._keep[int(t.value)] = (arrs, ref)       # the call only queues the copies: inputs live until wait()
-            self._calls_of[int(t.value)] = self.device_calls
+            self._submitted(int(t.value))
             return int(t.value)
         f, keep = _site_filter(site_filter)
         self._check(self.lib.c3r_submit_chunk_filtered(self.ctx, C.byref(rd), rp, ref_start1, rn, region_start1,
                                                        region_end1, C.byref(f), C.byref(t)), "c3r_submit_chunk_filtered")
         self._keep[int(t.value)] = (arrs, ref, keep)
-        self._calls_of[int(t.value)] = self.device_calls
+        self._submitted(int(t.value))
         return int(t.value)
 
     def submit_bam(self, raw, ref, ref_start1: int, region_start1: int, region_end1: int, site_filter=None) -> int:
@@ -175,11 +205,13 @@ class Engine:
             ref = np.ascontiguousarray(ref, np.uint8)
             rp, rn = ref.ctypes.data, int(ref.size)
         f, keep = _site_filter(site_filter) if site_filter is not None else (None, [])
+        if self.device_vcf:
+            self._set_vcf(raw.contig)
         self._check(self.lib.c3r_submit_bam_chunk(self.ctx, C.byref(raw.raw), rp, ref_start1, rn, region_start1,
                                                   region_end1, C.byref(f) if f is not None else None, C.byref(t)),
                     "c3r_submit_bam_chunk")
         self._keep[int(t.value)] = (raw, ref, keep)
-        self._calls_of[int(t.value)] = self.device_calls
+        self._submitted(int(t.value))
         self._bam_of[int(t.value)] = raw.contig
         return int(t.value)
 
@@ -190,6 +222,7 @@ class Engine:
         stay valid until release(ticket); the ticket is then NOT released here."""
         r = L.Result()
         calls_on = self._calls_of.pop(ticket, False)
+        vcf_on = self._vcf_of.pop(ticket, False)
         bam_contig = self._bam_of.pop(ticket, None)
         try:
             self._check(self.lib.c3r_wait(self.ctx, ticket, C.byref(r)), "c3r_wait")
@@ -200,6 +233,13 @@ class Engine:
             cp, cn, ms = C.c_void_p(), C.c_int64(0), C.c_float(0)
             self._check(self.lib.c3r_wait_calls(self.ctx, ticket, C.byref(cp), C.byref(cn), C.byref(ms)), "c3r_wait_calls")
             calls, call_ms = _view(cp.value, cn.value, L.CALL_DTYPE, copy), float(ms.value)
+        vcf_text, vcf_rows, vcf_ms = None, 0, 0.0
+        if vcf_on:
+            tp, nb, nr, ms = C.c_void_p(), C.c_int64(0), C.c_int64(0), C.c_float(0)
+            self._check(self.lib.c3r_wait_vcf(self.ctx, ticket, C.byref(tp), C.byref(nb), C.byref(nr), C.byref(ms)),
+                        "c3r_wait_vcf")
+            vcf_text = C.string_at(tp.value, nb.value).decode("ascii") if nb.value else ""
+            vcf_rows, vcf_ms = int(nr.value), float(ms.value)
         reads, bam_ms = None, 0.0
         if bam_contig is not None:
             from .bam import reads_from
@@ -220,7 +260,7 @@ class Engine:
             row_counts=v(r.row_counts, r.n_rows * Ct, np.int32).reshape(-1, Ct) if r.row_counts else None,
             row_depth=v(r.row_depth, r.n_rows, np.int32) if r.row_depth else None,
             stage_ms=[float(x) for x in r.stage_ms], launches=int(r.kernel_launches), calls=calls, call_ms=call_ms,
-            reads=reads, bam_ms=bam_ms)
+            reads=reads, bam_ms=bam_ms, vcf_text=vcf_text, vcf_rows=vcf_rows, vcf_ms=vcf_ms)
         if release and copy:
             self.lib.c3r_release(self.ctx, ticket)
         return out
@@ -229,6 +269,7 @@ class Engine:
         self._keep.pop(ticket, None)
         self._bam_of.pop(ticket, None)
         self._calls_of.pop(ticket, None)
+        self._vcf_of.pop(ticket, None)
         self.lib.c3r_release(self.ctx, ticket)
 
     def call_chunk(self, batch, ref, ref_start1, region_start1, region_end1, site_filter=None) -> ChunkResult:
@@ -386,6 +427,34 @@ def format_vcf_rows(res: ChunkResult, batch: ReadBatch, ref: np.ndarray, ref_sta
                             int(ref_start1), int(ref.size), contig.encode(), -1.0 if qual is None else float(qual),
                             int(show_ref), threads, C.byref(text), C.byref(nb), C.byref(nr))
     return _rows_of(lib, rc, text, nb, nr, "c3r_format_vcf")
+
+
+def device_vcf_rows(res: ChunkResult) -> list:
+    """the VCF data lines the GPU printed for a ticket (Engine(device_vcf=True)): format_vcf_rows' lines"""
+    if res.vcf_text is None:
+        raise C3RError("device_vcf_rows needs a ticket submitted with Engine.set_device_vcf(True)")
+    rows = res.vcf_text.split("\n")[:-1] if res.vcf_text else []
+    if len(rows) != res.vcf_rows:
+        raise C3RError("%d lines in the text of %d rows" % (len(rows), res.vcf_rows))
+    return rows
+
+
+def debug_vcf_rows(res: ChunkResult, batch: ReadBatch, ref: np.ndarray, ref_start1: int, contig: str,
+                   qual=P.QUAL_CUT_OFF, show_ref: bool = True, calls=None) -> list:
+    """format_vcf_rows the device's way, on the host (c3r_debug_vcf_rows): QUAL from the threshold table, each row's
+    length counted first and the row then written at its offset (no GPU needed)"""
+    from .bam import reads_struct
+    calls = np.ascontiguousarray(res.calls if calls is None else calls, L.CALL_DTYPE)
+    lib = L.load()
+    keep = []
+    r = _result_struct(res, keep)
+    rd = reads_struct(batch, keep)
+    ref = np.ascontiguousarray(ref, np.uint8)
+    text, nb, nr = C.c_void_p(), C.c_int64(0), C.c_int64(0)
+    rc = lib.c3r_debug_vcf_rows(C.byref(r), calls.ctypes.data if calls.size else None, C.byref(rd), ref.ctypes.data,
+                                int(ref_start1), int(ref.size), contig.encode(), -1.0 if qual is None else float(qual),
+                                int(show_ref), C.byref(text), C.byref(nb), C.byref(nr))
+    return _rows_of(lib, rc, text, nb, nr, "c3r_debug_vcf_rows")
 
 
 def decide_calls(res: ChunkResult, batch: ReadBatch, ref: np.ndarray, ref_start1: int) -> np.ndarray:

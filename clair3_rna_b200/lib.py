@@ -69,6 +69,11 @@ CALL_NO_ROW = 0xFF
 GT_TEXT = ("0/0", "1/1", "0/1", "1/2", "None")
 
 
+class VcfOptions(C.Structure):
+    """c3r_vcf_options (include/c3r_b200.h)"""
+    _fields_ = [("on", C.c_int32), ("show_ref", C.c_int32), ("qual_cut", C.c_double), ("contig", C.c_char_p)]
+
+
 class SiteFilter(C.Structure):
     """c3r_site_filter (include/c3r_b200.h)"""
     _fields_ = [("pileup_bed", C.c_void_p), ("n_pileup_bed", C.c_int64),
@@ -102,7 +107,9 @@ EXPORTS = ["c3r_abi_version", "c3r_default_params", "c3r_create", "c3r_destroy",
            "c3r_decode_vcf", "c3r_free_text", "c3r_debug_format_fixed", "c3r_vcf_write_bgzf",
            "c3r_host_alloc", "c3r_host_free", "c3r_fasta_fetch",
            "c3r_enable_calls", "c3r_wait_calls", "c3r_format_vcf", "c3r_debug_decide_calls",
-           "c3r_bam_fetch_raw", "c3r_submit_bam_chunk", "c3r_wait_reads", "c3r_wait_reads_stages", "c3r_debug_inflate"]
+           "c3r_bam_fetch_raw", "c3r_submit_bam_chunk", "c3r_wait_reads", "c3r_wait_reads_stages", "c3r_debug_inflate",
+           "c3r_set_vcf", "c3r_wait_vcf", "c3r_vcf_row_max", "c3r_debug_vcf_rows", "c3r_debug_vcf_qual_check",
+           "c3r_debug_vcf_q_min"]
 
 _lib = None
 
@@ -164,6 +171,16 @@ def load():
                                    C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
     lib.c3r_debug_decide_calls.argtypes = [C.POINTER(Result), C.POINTER(Reads), C.c_void_p, C.c_int64, C.c_int64,
                                            C.c_void_p]
+    lib.c3r_set_vcf.argtypes = [C.c_void_p, C.POINTER(VcfOptions)]
+    lib.c3r_wait_vcf.argtypes = [C.c_void_p, C.c_int64, C.POINTER(C.c_void_p), C.POINTER(C.c_int64),
+                                 C.POINTER(C.c_int64), C.POINTER(C.c_float)]
+    lib.c3r_vcf_row_max.argtypes = [C.c_int64]
+    lib.c3r_vcf_row_max.restype = C.c_int64
+    lib.c3r_debug_vcf_rows.argtypes = [C.POINTER(Result), C.c_void_p, C.POINTER(Reads), C.c_void_p, C.c_int64,
+                                       C.c_int64, C.c_char_p, C.c_double, C.c_int, C.POINTER(C.c_void_p),
+                                       C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
+    lib.c3r_debug_vcf_qual_check.argtypes = [C.c_int, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
+    lib.c3r_debug_vcf_q_min.argtypes = [C.c_double, C.POINTER(C.c_int32)]
     lib.c3r_bam_fetch_raw.argtypes = [C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_void_p, C.c_int64,
                                       C.POINTER(BamRaw)]
     lib.c3r_submit_bam_chunk.argtypes = [C.c_void_p, C.POINTER(BamRaw), C.c_void_p, C.c_int64, C.c_int64, C.c_int64,

@@ -56,7 +56,7 @@ def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, wo
         qual=P.QUAL_CUT_OFF, sample_name="SAMPLE", gather=None, stats=None, bed_fn=None, vcf_fn=None, head_tail=False,
         merge_qual=None, show_ref=True, rediportal_fn=None, rediportal_tags=None, output_no_tagging=None,
         compress_vcf=False, engine=None, loader_threads=2, native_threads=0, merge=True, cmdline=None,
-        device_calls=False, device_bam=False):
+        device_calls=False, device_bam=False, device_vcf=False):
     """merge_qual / show_ref / rediportal_*: the options of the merge stage (sharder.sort_vcf = sort_vcf_from of the
     reference); the defaults keep every row as the chunks produced it.  engine: an Engine to reuse (its parameters and
     weights are then the caller's business); loader_threads: BAM / FASTA readers working ahead of the GPU;
@@ -65,9 +65,11 @@ def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, wo
     leave only the formatting to the decoder threads (c3r_format_vcf); the rows are the same.  A caller's engine
     gets its own device_calls setting back when the run ends.  device_bam: the loader threads only read the compressed
     BAM blocks of a chunk (BamFile.fetch_raw, into page-locked buffers) and the GPU inflates and parses them
-    (Engine.submit_bam); the rows are the same."""
+    (Engine.submit_bam); the rows are the same.  device_vcf: the GPU also prints each chunk's rows (Engine.set_device_vcf,
+    which implies the decisions on the GPU) and the decoder threads only split its text; the rows are the same, and a
+    caller's engine gets its own setting back when the run ends."""
     from .bam import BamFile
-    from .engine import Engine, PinnedPool, decode_vcf_rows, format_vcf_rows
+    from .engine import Engine, PinnedPool, decode_vcf_rows, device_vcf_rows, format_vcf_rows
     fai = fasta.read_fai(ref_fn)
     bf = BamFile(bam_fn)
     idx = {n: m for n, _, m, _ in bf.idxstats()}
@@ -81,18 +83,23 @@ def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, wo
     C = P.CHANNEL_SIZE + (P.PHASED_CHANNEL_SIZE if phased else 0)
     eng = engine
     calls_before = eng.device_calls if eng is not None else None
+    vcf_before = eng._vcf_opts if eng is not None else None
     if eng is None:
         eng = Engine(device, C, snp_min_af=snp_min_af, indel_min_af=indel_min_af, min_coverage=min_coverage,
                      min_mq=min_mq, enable_padding=padding, enable_head_tail=head_tail, device_calls=device_calls)
         eng.set_weights(W.load(chkpnt_fn))
     elif eng.device_calls != bool(device_calls):
         eng.set_device_calls(device_calls)
+    if device_vcf or eng.device_vcf:
+        eng.set_device_vcf(device_vcf, qual=qual, show_ref=True)
     t0 = time.time()
     rows_of = {}
     n_cand = 0
     # host seconds per stage of this rank's loop (the GPU works under all of them but `wait`)
     tm = dict(fetch=0.0, ref=0.0, submit=0.0, wait=0.0, decode=0.0)
     call_ms = 0.0                                    # device time of k_call (device_calls)
+    vcf_ms = 0.0                                     # device time of the text kernels (device_vcf)
+    vcf_d2h = 0                                      # bytes of the text copies: each ticket's bound (device_vcf)
     bam_ms = 0.0                                     # device time of the BAM parse stages (device_bam)
 
     import threading
@@ -173,8 +180,11 @@ def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, wo
 
     def decode(res, pbatch, pref, prs1, pname, pbuf):
         t = time.time()
-        rows = (format_vcf_rows if device_calls else decode_vcf_rows)(res, pbatch, pref, prs1, pname, qual=qual,
-                                                                      threads=dec_threads)
+        if device_vcf:
+            rows = device_vcf_rows(res)
+        else:
+            rows = (format_vcf_rows if device_calls else decode_vcf_rows)(res, pbatch, pref, prs1, pname, qual=qual,
+                                                                          threads=dec_threads)
         tm["decode"] += time.time() - t
         pool.put(pbuf[0])                            # the reference window is free again
         return rows
@@ -219,6 +229,9 @@ def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, wo
             tm["wait"] += time.time() - t
             n_cand += res.n_cand
             call_ms += res.call_ms
+            vcf_ms += res.vcf_ms
+            if device_vcf:
+                vcf_d2h += res.n_cand * eng.lib.c3r_vcf_row_max(len(pname.encode()))
             if device_bam:                           # the compressed bytes are on the device: the buffer is free
                 bam_ms += res.bam_ms
                 bam_pool.put(ppbuf[1])
@@ -237,15 +250,18 @@ def run(bam_fn, ref_fn, chkpnt_fn, output, *, contigs=None, device=0, rank=0, wo
             bam_pool.close()
             eng._bam_pool = None
         eng.close()
-    elif eng.device_calls != calls_before:
-        eng.set_device_calls(calls_before)
+    else:
+        if eng.device_calls != calls_before:
+            eng.set_device_calls(calls_before)
+        if eng._vcf_opts != vcf_before:
+            eng.set_device_vcf(vcf_before is not None, *(vcf_before or ()))
     bf.close()
     for r in readers:
         r.close()
     if stats is not None:
         stats.update(shards=len(mine), candidates=n_cand, seconds=time.time() - t0, host_seconds=tm, submit_ms=submit_ms,
                      cost=sum(costs[i] for i in mine), total_shards=len(shards), call_device_ms=call_ms,
-                     bam_device_ms=bam_ms)
+                     bam_device_ms=bam_ms, vcf_device_ms=vcf_ms, vcf_d2h_bytes=vcf_d2h)
     if not merge:                                    # the caller only wants this rank's loop (timing passes)
         return None
     if world > 1:
@@ -324,6 +340,8 @@ def main(argv=None):
                     help="decide the genotypes on the GPU and only format the rows on the host (same output)")
     ap.add_argument("--device_bam", action="store_true",
                     help="inflate and parse the BAM blocks of each chunk on the GPU (same output)")
+    ap.add_argument("--device_vcf", action="store_true",
+                    help="decide the genotypes and print the VCF rows on the GPU (same output)")
     a = ap.parse_args(argv)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -348,7 +366,7 @@ def main(argv=None):
         cmdline=" ".join(sys.argv) if argv is None else " ".join(["run_chunks"] + list(argv)),
         sample_name=a.sampleName, stats=stats, bed_fn=a.bed_fn, vcf_fn=a.genotyping_mode_vcf_fn,
         head_tail=a.enable_variant_calling_at_sequence_head_and_tail, device_calls=a.device_calls,
-        device_bam=a.device_bam)
+        device_bam=a.device_bam, device_vcf=a.device_vcf)
     print("[rank %d] %d shards, %d candidates in %.2f s" % (rank, stats["shards"], stats["candidates"], stats["seconds"]),
           file=sys.stderr)
     if world > 1:

@@ -301,6 +301,41 @@ int c3r_debug_decide_calls(const c3r_result* res, const c3r_reads* reads, const 
                            int64_t ref_len, c3r_call* out);
 
 /* ------------------------------------------------------------------------------------------
+ * VCF text made on the GPU: after k_call, each candidate's row is printed on the device (csrc/vcf_row.cuh, the same
+ * printer c3r_decode_vcf and c3r_format_vcf use on the host) and a ticket returns its data lines as one block of text,
+ * byte for byte what c3r_format_vcf prints for the same contig, qual_cut and show_ref.
+ * QUAL on the device comes from a table of the host formula's thresholds (built once per process, uploaded once per
+ * context); the text of a NaN AF is the host printf's. */
+typedef struct {
+    int32_t on;
+    int32_t show_ref;
+    double qual_cut;           /* < 0: no LowQual filter                                                  */
+    const char* contig;        /* CHROM of the rows (copied; at most 1024 bytes)                          */
+} c3r_vcf_options;
+
+/* VCF text for the tickets submitted after this call (opts->on != 0) or not (the default).  The options are copied
+ * into a ticket when it is submitted, so a caller may set the contig before every submit.  Text on implies k_call;
+ * its records reach the host only if c3r_enable_calls is on too (else c3r_wait_calls keeps returning C3R_ERR_STATE).
+ * With text off nothing about a ticket changes: the same kernels, copies and results. */
+int c3r_set_vcf(c3r_ctx* ctx, const c3r_vcf_options* opts);
+/* The data lines of a ticket submitted with text on ('\n' after each, not NUL terminated), in pinned library memory
+ * valid until c3r_release; call after c3r_wait.  device_ms (may be NULL): device time of the text kernels (row lengths,
+ * offsets, rows).  C3R_ERR_STATE for a ticket submitted with text off or not returned by c3r_wait. */
+int c3r_wait_vcf(c3r_ctx* ctx, c3r_ticket ticket, const char** text, int64_t* n_bytes, int64_t* n_rows, float* device_ms);
+/* The most bytes one row can take with a contig name of contig_len bytes: the device sizes a ticket's text buffers
+ * as n_cand times this. */
+int64_t c3r_vcf_row_max(int64_t contig_len);
+/* test hooks (no GPU): the device's printing on the host - QUAL from the table, lengths counted first, rows written
+ * at their offsets, each checked to fill its counted length (else C3R_ERR_STATE) - with c3r_format_vcf's arguments
+ * and result (one thread; free with c3r_free_text); QUAL by table against QUAL by formula for all 2^32 float32 bit
+ * patterns (n_threads <= 0: all cores); FILTER's threshold q_min (hundredths) of a qual_cut. */
+int c3r_debug_vcf_rows(const c3r_result* res, const c3r_call* calls, const c3r_reads* reads, const uint8_t* ref,
+                       int64_t ref_start1, int64_t ref_len, const char* contig, double qual_cut, int show_ref,
+                       char** text, int64_t* n_bytes, int64_t* n_rows);
+int c3r_debug_vcf_qual_check(int n_threads, int64_t* n_checked, int64_t* n_mismatch);
+int c3r_debug_vcf_q_min(double qual_cut, int32_t* q_min);
+
+/* ------------------------------------------------------------------------------------------
  * BAM / BGZF / BAI input (host side, zlib; csrc/bam_io.cpp).  The reference reads the BAM only
  * through external samtools: `samtools mpileup BAM -r ctg:s-e ...` (src/create_tensor_pileup.py:
  * 436-451) and `samtools idxstats BAM` (run_clair3_rna:187).  c3r_bam_fetch is the index fetch
